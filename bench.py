@@ -2,11 +2,13 @@
 """Benchmark of the DCANet cost-volume hot path (feature maps -> disparity) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config kitti_384x1248]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is ONE stereo pair through the whole hot path at BASELINE.json's configs[1]
 (KITTI 384x1248, maxdisp 192, batch 1).  Pairs shard by rank with no collective (weak scaling).
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  The inputs and weights are seeded, so the same arguments give the same inputs on every
+run; --dump-outputs writes what rank 0's last timed step returned, to compare two builds output for output.
 """
 import argparse
 import gc
@@ -187,6 +189,24 @@ def cpu_reference_run(cfg, steps, warmup, budget_s=150.0):
     return 1.0 / t_pair, t_pair * 1e3, cores, sample
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT):
+    """Writes every array as out_dir/<name>.npy in float32.  When they exceed `limit` bytes in all, each one is replaced by
+    a fixed sample of its flattened elements (sorted indices drawn by numpy's default_rng(0)), sized in proportion, so that
+    two runs with the same arguments still compare element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {name: a.numpy().astype(np.float32, copy=False) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > limit:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, a.size * limit // total, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def halo_plan_bytes(H, W, maxdisp, B, planes=2):
     """Bytes ONE rank sends to ONE neighbour per forward in the H-sharded mode (the plan of hshard.hot_path_steps: only
     the one live row next to a cut travels).  1/4-res 32-ch plane rows: dres0.0/2, dres1.0/2, 3 x (fused, out), classif3.0
@@ -298,7 +318,12 @@ def main():
                     help="N > 1: skip the H-sharded Middlebury sub-record (configs[4]) appended to the line")
     ap.add_argument("--hshard-transport", default="p2p", choices=["nccl", "p2p"],
                     help="halo rows by NCCL send/recv or by peer-memory stores (csrc/halo_p2p.cu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write pred4 and prob_volume2 of rank 0's last timed step as DIR/<name>.npy "
+                         "(float32, pairs of the step concatenated; a fixed sample when over 64 MB in all)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.hshard or args.breakdown):
+        ap.error("--dump-outputs applies to the --impl ours throughput run (not --hshard or --breakdown)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -385,9 +410,11 @@ def main():
 
     # ---------------- device-resident throughput ----------------
     with torch.no_grad():
-        def step(i):
+        def step(i, keep=None):
             for j in range(ppr):
-                net.hot_path(*dev_sets[(i * ppr + j) % nsets])
+                res = net.hot_path(*dev_sets[(i * ppr + j) % nsets])
+                if keep is not None:
+                    keep.append(res)
 
         for i in range(Wm):
             step(i)
@@ -398,15 +425,20 @@ def main():
         if rank == 0 and sampler.interval > 0:
             sampler.start()
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(K + 1)]
+        last_step = [] if args.dump_outputs and rank == 0 else None
         barrier()
         ev[0].record()
         for i in range(K):
-            step(i)
+            step(i, last_step if i == K - 1 else None)
             ev[i + 1].record()
         barrier()
         launches = d._lib.LAUNCHES
         step_ms = [ev[i].elapsed_time(ev[i + 1]) for i in range(K)]
         total_ms = ev[0].elapsed_time(ev[K])
+        if last_step is not None:        # to the host before anything else runs; written at the end
+            outputs = {"pred4": torch.cat([p for p, _ in last_step]).float().cpu(),
+                       "prob_volume2": torch.cat([v for _, v in last_step]).float().cpu()}
+            del last_step
 
         # ---------------- roofline of the dominant kernel: conv3d k3 s1 32->32 at 1/4 res ----------------
         # (timed right after the headline loop: the long latency / graph / two-stream loops further down leave the GPU at its
@@ -696,6 +728,8 @@ def main():
             v, ms, cores, kind, sample = cpu_arm(args.config, 2, 1, 25.0)
             line["cpu_baseline"] = {"value": v, "unit": UNIT, "cores": cores, "kind": kind, "sample": sample,
                                     "ms_per_pair": ms}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()

@@ -48,6 +48,15 @@ def synthetic_pair(seed, H, W, shift):
     return left, right
 
 
+def save_split(stem, arrays, limit=256 * 1024):
+    """np.savez_compressed to `<stem>.npz`, except that every array over `limit` bytes goes to its own
+    `<stem>.<key>.npz`, so that no fixture file comes near 1 MB (tests/_util.load_e2e merges them)."""
+    big = {k: v for k, v in arrays.items() if v.nbytes > limit}
+    np.savez_compressed(stem + ".npz", **{k: v for k, v in arrays.items() if k not in big})
+    for k, v in big.items():
+        np.savez_compressed(f"{stem}.{k}.npz", **{k: v})
+
+
 def main():
     from oracle import dcanet_oracle as O
     ref_model, ref_sub = import_reference()
@@ -143,7 +152,7 @@ def main():
             out["bn:" + k] = msd[k].numpy()
     out["conv_weight_abs_sum"] = np.array(csum)
     # (front-end weights are NOT stored: 13 MB, out of scope; its outputs above are the inputs)
-    np.savez_compressed(os.path.join(HERE, "e2e_64x128_d48.npz"), **out)
+    save_split(os.path.join(HERE, "e2e_64x128_d48"), out)
     keys = sorted(msd.keys())
     with open(os.path.join(HERE, "state_dict_keys.txt"), "w") as f:
         for k in keys:
