@@ -1,7 +1,8 @@
 """B200-native DCANet cost-volume hot path (feature maps -> disparity) behind the reference's module API."""
-from . import _lib, engine, frontend, gwcnet, hshard, kitti_io, pipeline
+from . import _lib, engine, evaluation, frontend, gwcnet, hshard, kitti_io, pipeline
 from . import gwcnet_dca0_g, gwcnet_dca1_g, gwcnet_dca2_g, gwcnet_dca4_g
 from .cva import Multi_Aggregation, cva
+from .evaluation import DisparityMeter, evaluate_files, read_kitti_disparity, read_pfm
 from .gwcnet_dca_g import GwcNet, feature_extraction, hourglass
 from .pipeline import HotPathPipeline
 from .self_attention import SelfAttentionBlock
@@ -11,4 +12,5 @@ from .submodule import (PropgationNet_4x, build_concat_volume, build_cost_planes
 
 __all__ = ["GwcNet", "feature_extraction", "hourglass", "cva", "Multi_Aggregation", "SemanticLevelContext",
            "SelfAttentionBlock", "PropgationNet_4x", "build_gwc_volume", "build_concat_volume", "build_cost_planes",
-           "disparity_regression", "softmax_disparity_regression", "convbn", "convbn_3d", "engine", "hshard", "kitti_io", "HotPathPipeline"]
+           "disparity_regression", "softmax_disparity_regression", "convbn", "convbn_3d", "engine", "hshard", "kitti_io", "HotPathPipeline",
+           "evaluation", "DisparityMeter", "evaluate_files", "read_pfm", "read_kitti_disparity"]

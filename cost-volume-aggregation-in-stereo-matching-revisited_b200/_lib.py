@@ -80,6 +80,8 @@ SIGNATURES = {
     "dca_halo_wait_unpack": [_vp, _ll, _ll, _ll, _c_int, _c_int, _vp, _vp, _vp, _vp, ctypes.c_ulonglong, _vp, _vp],
     "dca_adaptive_avgpool3d_rows": [_vp, _vp] + [_c_int] * 8 + [_vp],
     "dca_fold_bn": [_vp, _vp, _vp, _vp, _f, _vp, _vp, _c_int, _c_int, _vp],
+    "dca_disparity_metrics": [_vp, _vp, _vp] + [_c_int] * 3 + [_f, _vp],
+    "dca_class_confusion": [_vp, _vp, _vp] + [_c_int] * 4 + [_f, _vp],
 }
 _RESTYPES = {"dca_pack_weights_tc_bytes": ctypes.c_longlong, "dca_pack_weights_tc2d_bytes": ctypes.c_longlong,
              "dca_pack_weights_tc_march_bytes": ctypes.c_longlong}

@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libdca_b200.so")
-SOURCES = ["volume.cu", "conv_direct.cu", "conv_tc.cu", "dca_ops.cu", "halo_p2p.cu", "abi_composites.cu"]
+SOURCES = ["volume.cu", "conv_direct.cu", "conv_tc.cu", "dca_ops.cu", "halo_p2p.cu", "abi_composites.cu", "metrics.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "--use_fast_math=false"]
@@ -30,6 +30,7 @@ def _stale(target, deps):
 
 def build(force=False, verbose=False):
     hdrs = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cuh", ".h"))]
+    hdrs.append(os.path.join(os.path.dirname(HERE), "include", "dca_b200.h"))     # metrics.cu includes the C ABI header
     objs = []
     for s in SOURCES:
         src = os.path.join(CSRC, s)

@@ -1,0 +1,365 @@
+"""Accuracy against ground-truth disparity: the reference's evaluation loop (main_dca.py `mytest` :143-232) on the GPU.
+
+  read_pfm, read_kitti_disparity   ground-truth readers (SceneFlow / Middlebury PFM, KITTI uint16 PNG)
+  DisparityMeter                   device-side accumulator: per-image counters of dca_disparity_metrics (EPE, >1/2/3 px,
+                                   D1, utils/metrics.py:45-63) and the DCA class-map confusion matrix of
+                                   dca_class_confusion (main_dca.py:66-120, 209-232); no host sync until read back
+  summarize                        counters -> EPE / bad-N / D1 under both conventions, pixel accuracy / mPA / mIoU
+  evaluate_files                   the `mytest` loop as a streaming pipeline (ImagePipeline plus a GT slot per pair)
+
+Per-rank meters of a distributed run combine by concatenating their `rows()` (and summing `confusion()`) before
+`summarize`.  There is no CPU path: the kernels need CUDA tensors.
+"""
+import warnings
+
+import numpy as np
+import torch
+
+from . import _lib
+from .engine import _require_cuda
+from .kitti_io import (ImagePipeline, crop_prediction, fit_gt_to_crop, load_pair, pad_gt_to_multiple, pad_to_multiple,
+                       save_disparity_png)
+
+# column order of the counter rows (DCA_METRIC_* of include/dca_b200.h)
+VALID, SUM_ABS, GT1, GT2, GT3, D1, PRED_NONFINITE = range(7)
+METRIC_COUNT = 7
+SUM_ABS_UNIT = 2.0 ** -20          # SUM_ABS is fixed point: px = SUM_ABS * 2^-20
+
+
+# ---- ground-truth readers (host) ---------------------------------------------------------------------------
+def read_pfm(path):
+    """Single-channel PFM ('Pf') -> float32 [H,W], top row first.  A negative scale means little-endian data, a
+    positive one big-endian; rows are stored bottom-up.  inf (Middlebury's 'no ground truth') is kept."""
+    with open(path, "rb") as f:
+        header = f.readline().strip()
+        if header == b"PF":
+            raise ValueError(f"{path}: 3-channel PFM ('PF'), expected a single-channel disparity map ('Pf')")
+        if header != b"Pf":
+            raise ValueError(f"{path}: not a PFM file (header {header[:8]!r})")
+        dims = f.readline().split()
+        while len(dims) < 2:
+            dims += f.readline().split()
+        w, h = int(dims[0]), int(dims[1])
+        scale = float(f.readline().strip())
+        data = np.frombuffer(f.read(), dtype="<f4" if scale < 0 else ">f4")
+    if data.size < w * h:
+        raise ValueError(f"{path}: {data.size} values for a {h}x{w} image")
+    return np.ascontiguousarray(data[:w * h].reshape(h, w)[::-1], dtype=np.float32)
+
+
+def read_kitti_disparity(path):
+    """KITTI disparity PNG (uint16, disp * 256) -> float32 [H,W] px; 0 = no ground truth."""
+    from PIL import Image
+    a = np.asarray(Image.open(path))
+    if a.ndim != 2:
+        raise ValueError(f"{path}: expected a single-channel 16-bit PNG")
+    return a.astype(np.float32) / np.float32(256.0)
+
+
+# ---- kernel calls ----------------------------------------------------------------------------------------
+def _disparity_metrics(pred, gt, rows, max_valid):
+    """rows int64 [B, METRIC_COUNT] += counters of pred / gt fp32 [B,H,W] (dca_disparity_metrics)."""
+    _require_cuda(pred, gt, rows)
+    B, H, W = pred.shape
+    _lib.call("dca_disparity_metrics", pred.data_ptr(), gt.data_ptr(), rows.data_ptr(), B, H, W, max_valid,
+              torch.cuda.current_stream(pred.device).cuda_stream)
+
+
+def _class_confusion(logits, gt, conf, max_valid):
+    """conf int64 [D8,D8] += confusion of logits [B,D8,H8,W8] against gt fp32 [B,8*H8,8*W8] (dca_class_confusion)."""
+    _require_cuda(logits, gt, conf)
+    B, D8, H8, W8 = logits.shape
+    _lib.call("dca_class_confusion", logits.data_ptr(), gt.data_ptr(), conf.data_ptr(), B, D8, H8, W8, max_valid,
+              torch.cuda.current_stream(logits.device).cuda_stream)
+
+
+def _as_bhw(t, what):
+    if t.dim() == 4 and t.shape[1] == 1:
+        t = t[:, 0]
+    if t.dim() != 3:
+        raise ValueError(f"{what}: expected [B,H,W] or [B,1,H,W], got {tuple(t.shape)}")
+    if t.dtype != torch.float32:
+        raise ValueError(f"{what}: expected float32, got {t.dtype}")
+    return t.contiguous()
+
+
+class DisparityMeter:
+    """Accumulates evaluation counters on the device.
+
+    maxdisp     the model's maxdisp; D8 = maxdisp // 8 disparity classes in the confusion matrix
+    max_valid   GT upper bound of the valid mask: None = maxdisp (the (gt > 0) & (gt < maxdisp) mask of the GwcNet /
+                PSMNet test loops), 0 = no upper bound (KITTI devkit)
+    device      where the counter tables live; None = the device of the first prediction
+
+    `update` launches the two kernels on the current stream and never synchronises; it allocates only when the row
+    table doubles.  `rows()` / `confusion()` / `summary()` are the read-back points."""
+
+    def __init__(self, maxdisp, max_valid=None, device=None, capacity=64):
+        self.maxdisp = int(maxdisp)
+        self.D8 = self.maxdisp // 8
+        self.max_valid = float(self.maxdisp if max_valid is None else max_valid)
+        self.device = None if device is None else torch.device(device)
+        if self.device is not None and self.device.type == "cuda" and self.device.index is None:
+            self.device = torch.device("cuda", torch.cuda.current_device())
+        self._cap = max(1, int(capacity))
+        self._rows = self._conf = None
+        self._n = 0
+        self._has_conf = False
+        if self.device is not None:
+            self._alloc()
+
+    def _alloc(self):
+        self._rows = torch.zeros((self._cap, METRIC_COUNT), dtype=torch.int64, device=self.device)
+        self._conf = torch.zeros((self.D8, self.D8), dtype=torch.int64, device=self.device)
+
+    def __len__(self):
+        return self._n
+
+    def update(self, pred4, disp_true, prob_volume=None):
+        """Score a batch: pred4 [B,1,H,W] (or [B,H,W]) against disp_true [B,H,W] (or [B,1,H,W]) in the same pixel
+        frame, both fp32 on the same device; prob_volume [B,D8,H/8,W/8] (the model's second output) adds to the
+        confusion matrix."""
+        pred, gt = _as_bhw(pred4, "pred4"), _as_bhw(disp_true, "disp_true")
+        if gt.shape != pred.shape:
+            raise ValueError(f"disp_true {tuple(gt.shape)} and pred4 {tuple(pred.shape)} differ")
+        if self.device is None:
+            self.device = pred.device
+            self._alloc()
+        if pred.device != self.device or gt.device != self.device:
+            raise ValueError(f"meter lives on {self.device}, tensors on {pred.device} / {gt.device}")
+        pv = None
+        if prob_volume is not None:
+            pv = prob_volume.contiguous()
+            B, H, W = pred.shape
+            if pv.dim() != 4 or tuple(pv.shape) != (B, self.D8, H // 8, W // 8) or H % 8 or W % 8 \
+                    or pv.dtype != torch.float32 or pv.device != self.device:
+                raise ValueError(f"prob_volume {tuple(pv.shape)} {pv.dtype}: expected float32 "
+                                 f"[{B}, {self.D8}, {H}/8, {W}/8] on {self.device}")
+        B = pred.shape[0]
+        if self._n + B > self._cap:
+            while self._n + B > self._cap:
+                self._cap *= 2
+            grown = torch.zeros((self._cap, METRIC_COUNT), dtype=torch.int64, device=self.device)
+            grown[:self._n].copy_(self._rows[:self._n])
+            self._rows = grown
+        _disparity_metrics(pred, gt, self._rows[self._n:self._n + B], self.max_valid)
+        if pv is not None:
+            _class_confusion(pv, gt, self._conf, self.max_valid)
+            self._has_conf = True
+        self._n += B
+
+    def _readback(self, t):
+        if t.is_cuda:
+            torch.cuda.synchronize(t.device)          # updates may have run on any stream of the device
+        return t.cpu().numpy().astype(np.uint64)
+
+    def rows(self):
+        """numpy uint64 [N, METRIC_COUNT]: one counter row per image, in update order."""
+        if self._rows is None:
+            return np.zeros((0, METRIC_COUNT), np.uint64)
+        return self._readback(self._rows[:self._n])
+
+    def confusion(self):
+        """numpy uint64 [D8, D8]: row = GT class, column = predicted class."""
+        if self._conf is None:
+            return np.zeros((self.D8, self.D8), np.uint64)
+        return self._readback(self._conf)
+
+    def summary(self):
+        return summarize(self.rows(), self.confusion() if self._has_conf else None)
+
+
+def _nanmean(a):
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore", RuntimeWarning)
+        return float(np.nanmean(a)) if a.size else float("nan")
+
+
+def summarize(rows, confusion=None):
+    """Counter rows [N, METRIC_COUNT] (+ confusion [D8,D8]) -> dict of metrics.
+
+    epe, bad1, bad2, bad3, d1            mean over images of the per-image values (GwcNet / PSMNet test loops); images
+                                         without valid pixels are skipped and counted in n_images_skipped
+    *_pooled                             the same over all valid pixels at once (KITTI devkit)
+    bad-N and D1 are fractions of the valid pixels; a non-finite prediction counts as an error of every kind and is
+    left out of the EPE sum (the EPE is over the valid pixels with a finite prediction; n_pred_nonfinite says how many
+    were not).  From the confusion matrix, the segmentation Evaluator's formulas (main_dca.py:66-120):
+    pixel_accuracy = trace / total, mpa = nanmean(diag / row sums), miou = nanmean(diag / (row + column sums - diag));
+    classes with neither GT nor predictions are nan and left out of the means."""
+    r = np.asarray(rows, dtype=np.uint64).reshape(-1, METRIC_COUNT).astype(np.float64)
+    valid, nonfinite = r[:, VALID], r[:, PRED_NONFINITE]
+    finite = valid - nonfinite
+    epe_sum = r[:, SUM_ABS] * SUM_ABS_UNIT
+    has = valid > 0
+    out = {"n_images": int(r.shape[0]), "n_images_skipped": int((~has).sum()), "n_valid": int(valid.sum()),
+           "n_pred_nonfinite": int(nonfinite.sum())}
+    with np.errstate(divide="ignore", invalid="ignore"):
+        per = {"epe": epe_sum[has] / finite[has]}
+        for name, col in (("bad1", GT1), ("bad2", GT2), ("bad3", GT3), ("d1", D1)):
+            per[name] = r[has, col] / valid[has]
+        for name, v in per.items():
+            out[name] = float(v.mean()) if v.size else float("nan")
+        n, nf = valid.sum(), finite.sum()
+        out["epe_pooled"] = float(epe_sum.sum() / nf) if nf else float("nan")
+        for name, col in (("bad1", GT1), ("bad2", GT2), ("bad3", GT3), ("d1", D1)):
+            out[name + "_pooled"] = float(r[:, col].sum() / n) if n else float("nan")
+        if confusion is not None:
+            cm = np.asarray(confusion, dtype=np.float64)
+            diag, gt_n, pred_n = np.diag(cm), cm.sum(axis=1), cm.sum(axis=0)
+            total = cm.sum()
+            out["pixel_accuracy"] = float(diag.sum() / total) if total else float("nan")
+            out["mpa"] = _nanmean(diag / gt_n)
+            out["miou"] = _nanmean(diag / (gt_n + pred_n - diag))
+            out["n_class_pixels"] = int(total)
+    return out
+
+
+# ---- the evaluation loop -----------------------------------------------------------------------------------
+class EvalPipeline(ImagePipeline):
+    """ImagePipeline with a ground-truth slot per pair and a `DisparityMeter.update` after every forward.
+
+      loader threads   decode + standardise + frame the pair AND its GT (same framing, padding = invalid)
+      slot ring        pinned image and GT buffers; both go to the device on the copy stream
+      compute stream   forward, then meter.update (pred4 and prob_volume2 against the framed GT), then the D2H of the
+                       prediction when a PNG is wanted
+      writer thread    crops the prediction back and writes the KITTI PNG, as ImagePipeline does
+
+    mode "fit": fit_to_crop / fit_gt_to_crop into crop_height x crop_width (my_img.py); "pad16": top/right zero padding
+    to multiples of 16 (main_dca.py:153-166), slot buffers follow each pair's padded size."""
+
+    def __init__(self, model, meter, mode="fit", crop_height=384, crop_width=1248, depth=3, workers=2):
+        if mode not in ("fit", "pad16"):
+            raise ValueError(f"mode must be 'fit' or 'pad16', got {mode!r}")
+        super().__init__(model, crop_height, crop_width, depth, workers)
+        self.meter, self.mode = meter, mode
+        self.gt_host = [self._host(crop_height, crop_width) for _ in range(self.depth)]
+        self.gt_dev = [torch.empty((crop_height, crop_width), dtype=torch.float32, device=self.dev)
+                       for _ in range(self.depth)] if self.cuda else self.gt_host
+
+    def _host(self, *shape):
+        t = torch.empty(shape, dtype=torch.float32)
+        return t.pin_memory() if self.cuda else t
+
+    def _ensure(self, slot, H, W):
+        """(Re)size a slot's buffers to an H x W frame (only pad16 mode changes sizes; the slot is idle here)."""
+        if tuple(self.gt_host[slot].shape) == (H, W):
+            return
+        self.in_host[slot], self.out_host[slot], self.gt_host[slot] = self._host(6, H, W), self._host(H, W), \
+            self._host(H, W)
+        if self.cuda:
+            self.in_dev[slot] = torch.empty((6, H, W), dtype=torch.float32, device=self.dev)
+            self.gt_dev[slot] = torch.empty((H, W), dtype=torch.float32, device=self.dev)
+        else:
+            self.in_dev[slot], self.gt_dev[slot] = self.in_host[slot], self.gt_host[slot]
+
+    def _load_eval(self, left, right, gt_path):
+        gt = read_pfm(gt_path) if str(gt_path).lower().endswith(".pfm") else read_kitti_disparity(gt_path)
+        if self.mode == "fit":
+            fitted, h, w = self._load(left, right)
+            if gt.shape != (h, w):
+                raise ValueError(f"{gt_path}: ground truth {gt.shape} does not match the images ({h}, {w})")
+            return fitted, fit_gt_to_crop(gt, self.ch, self.cw), h, w, 0
+        pair = load_pair(left, right)
+        _, h, w = pair.shape
+        if gt.shape != (h, w):
+            raise ValueError(f"{gt_path}: ground truth {gt.shape} does not match the images ({h}, {w})")
+        fitted, top, _ = pad_to_multiple(torch.from_numpy(pair)[None], 16)
+        return fitted[0].numpy(), pad_gt_to_multiple(gt, 16)[0], h, w, top
+
+    def _forward_eval(self, slot):
+        x = self.in_dev[slot]
+        out = self.model(x[None, 0:3], x[None, 3:6])
+        pred, pv = (out[0], out[1]) if isinstance(out, (tuple, list)) else (out, None)
+        self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None)
+        return pred.reshape(x.shape[1], x.shape[2])
+
+    def _crop_back(self, disp, h, w, top):
+        if self.mode == "fit":
+            return crop_prediction(disp, h, w, self.ch, self.cw)
+        return disp[top:top + h, :w]
+
+    def run(self, quads):
+        """quads: iterable of (leftname, rightname, gt_path, savename or None).  Scores every pair into the meter in
+        input order; writes the PNGs (cropped back to the image size) of the pairs with a savename."""
+        import queue
+        import threading
+        from concurrent.futures import ThreadPoolExecutor
+        quads = list(quads)
+        slot_sem = threading.Semaphore(self.depth)          # a slot is reusable once the writer is done with it
+        q = queue.Queue()
+        err = []
+
+        def writer():
+            while True:
+                item = q.get()
+                if item is None:
+                    return
+                slot, h, w, top, savename = item
+                try:
+                    if self.cuda:
+                        self.done[slot].synchronize()
+                    if savename is not None:
+                        save_disparity_png(savename, self._crop_back(self.out_host[slot].numpy(), h, w, top).copy())
+                except Exception as e:          # surfaced by run()
+                    err.append(e)
+                finally:
+                    slot_sem.release()
+
+        wt = threading.Thread(target=writer, daemon=True)
+        wt.start()
+        was_training = getattr(self.model, "training", False)
+        if hasattr(self.model, "eval"):
+            self.model.eval()
+        try:
+            with ThreadPoolExecutor(self.workers) as pool, torch.no_grad():
+                futs = [pool.submit(self._load_eval, l, r, g) for l, r, g, _ in quads]
+                for i, (fut, quad) in enumerate(zip(futs, quads)):
+                    fitted, gt, h, w, top = fut.result()
+                    slot_sem.acquire()
+                    slot = i % self.depth
+                    self._ensure(slot, fitted.shape[1], fitted.shape[2])
+                    np.copyto(self.in_host[slot].numpy(), fitted)
+                    np.copyto(self.gt_host[slot].numpy(), gt)
+                    savename = quad[3]
+                    if self.cuda:
+                        with torch.cuda.stream(self.copy_stream):
+                            if i >= self.depth:
+                                self.copy_stream.wait_event(self.free[slot])     # kernels of the slot's previous pair
+                            self.in_dev[slot].copy_(self.in_host[slot], non_blocking=True)
+                            self.gt_dev[slot].copy_(self.gt_host[slot], non_blocking=True)
+                            self.h2d[slot].record(self.copy_stream)
+                        with torch.cuda.stream(self.compute_stream):
+                            self.compute_stream.wait_event(self.h2d[slot])
+                            pred = self._forward_eval(slot)
+                            self.free[slot].record(self.compute_stream)
+                            if savename is not None:
+                                self.out_host[slot].copy_(pred, non_blocking=True)
+                            self.done[slot].record(self.compute_stream)
+                    else:
+                        pred = self._forward_eval(slot)
+                        if savename is not None:
+                            self.out_host[slot].copy_(pred)
+                    q.put((slot, h, w, top, savename))
+        finally:
+            q.put(None)
+            wt.join()
+            if was_training and hasattr(self.model, "train"):
+                self.model.train()
+        if err:
+            raise err[0]
+
+
+def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=2, maxdisp=None, max_valid=None):
+    """main_dca.py `mytest` over files: quads = (left, right, gt_path, savename or None); GT is a KITTI PNG or a PFM
+    (by extension).  maxdisp defaults to model.maxdisp, max_valid as in DisparityMeter.  Returns (summary dict,
+    per-image counter rows [N, METRIC_COUNT] in input order); synchronises once, at the end."""
+    if maxdisp is None:
+        maxdisp = getattr(model, "maxdisp", 192)
+    try:
+        dev = next(model.parameters()).device
+    except (StopIteration, AttributeError):
+        dev = torch.device("cpu")
+    meter = DisparityMeter(maxdisp, max_valid, dev)
+    EvalPipeline(model, meter, mode, crop[0], crop[1], depth, workers).run(quads)
+    rows = meter.rows()
+    return summarize(rows, meter.confusion() if meter._has_conf else None), rows

@@ -7,6 +7,7 @@ Mirrors, function by function:
   fit_to_crop          my_img.py:73-89   smaller images: zero-padded at the TOP and RIGHT into crop_h x crop_w;
                                          larger: rows cropped around the centre, columns from 0
   pad_to_multiple      main_dca.py:153-166  top / right zero padding to multiples of 16
+  fit_gt_to_crop, pad_gt_to_multiple       the same two framings for a ground-truth disparity map (padding 0 = no GT)
   crop_prediction      my_img.py:105-108, main_dca.py:171-174
   save_disparity_png   my_img.py:110     uint16(disp * 256), the KITTI submission format
   predict_files        my_img.py:91-110
@@ -56,6 +57,25 @@ def pad_to_multiple(img, multiple=16):
     top = (-H) % multiple
     right = (-W) % multiple
     return torch.nn.functional.pad(img, (0, right, top, 0)), top, right
+
+
+def fit_gt_to_crop(gt, crop_height=384, crop_width=1248):
+    """Ground truth [h,w] -> float32 [crop_h, crop_w] framed exactly as `fit_to_crop` frames the images, so GT pixel
+    (y, x) sits under prediction pixel (y, x); the padding is 0 (= no ground truth)."""
+    h, w = gt.shape
+    if h <= crop_height and w <= crop_width:
+        fitted = np.zeros((crop_height, crop_width), np.float32)
+        fitted[crop_height - h:, :w] = gt
+        return fitted
+    start_y = int((h - crop_height) / 2)
+    return np.ascontiguousarray(gt[start_y:start_y + crop_height, :crop_width], dtype=np.float32)
+
+
+def pad_gt_to_multiple(gt, multiple=16):
+    """Ground truth [H,W] -> (float32 zero-padded at the top and right like `pad_to_multiple`, top_pad, right_pad)."""
+    H, W = gt.shape
+    top, right = (-H) % multiple, (-W) % multiple
+    return np.pad(np.asarray(gt, np.float32), ((top, 0), (0, right))), top, right
 
 
 def crop_prediction(disp, h, w, crop_height=384, crop_width=1248):

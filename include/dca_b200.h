@@ -252,6 +252,35 @@ int dca_softmax_regress_upsample(const float* logits, const float* mask, float* 
 int dca_adaptive_avgpool3d_rows(const float* x, float* y, int B, int D, int H, int W, int h0, int Do, int Ho, int Wo,
                                 void* stream);
 
+/* (7) accuracy against ground-truth disparity: the evaluation loop of main_dca.py `mytest` (:143-232) ------------------ */
+/* Both kernels ADD into caller-zeroed 64-bit counters (integer sums: bit-reproducible in any launch order), never
+ * allocate or synchronise, and may be captured in a CUDA graph.  A GT pixel g is valid when
+ *   isfinite(g) && g > 0 && (max_valid <= 0 || g < max_valid)
+ * (the SceneFlow mask (gt > 0) & (gt < maxdisp) of the GwcNet / PSMNet test loops; KITTI's 0 and Middlebury's inf are
+ * invalid).  All arithmetic is IEEE fp32 without fast math. */
+#define DCA_METRIC_VALID 0         /* valid GT pixels */
+#define DCA_METRIC_SUM_ABS 1       /* sum over valid pixels with a finite prediction of E = |pred - gt|, in units of 2^-20 px:
+                                      min(E, 2^20) * 2^20 rounded to nearest-even.  Each pixel adds <= 2^40, so a row is exact
+                                      (no overflow) while the valid pixels added into it number at most 2^23. */
+#define DCA_METRIC_GT1 2           /* valid pixels with E > 1 */
+#define DCA_METRIC_GT2 3           /* valid pixels with E > 2 */
+#define DCA_METRIC_GT3 4           /* valid pixels with E > 3 */
+#define DCA_METRIC_D1 5            /* valid pixels with E > 3 && E / |gt| > 0.05f (GwcNet D1_metric, division form) */
+#define DCA_METRIC_PRED_NONFINITE 6 /* valid pixels whose prediction is NaN or inf: counted in GT1..D1, not in SUM_ABS */
+#define DCA_METRIC_COUNT 7
+/* pred, gt fp32 [B,H,W] in the same pixel frame (pred4 [B,1,H,W] is the same memory); rows [B][DCA_METRIC_COUNT]:
+ * rows[b][m] += counter m of image b.  B <= 65535. */
+int dca_disparity_metrics(const float* pred, const float* gt, unsigned long long* rows, int B, int H, int W,
+                          float max_valid, void* stream);
+/* Confusion matrix of the DCA disparity classes (main_dca.py:66-120, 209-232): logits fp32 [B,D8,H8,W8] (prob_volume2),
+ * gt fp32 [B,8*H8,8*W8] in the same frame; conf [D8][D8] += pixel count, row = GT class, column = predicted class.
+ * Predicted class = first argmax of the fp32 softmax, exactly as dca_class_stats.  GT class of 1/8-res pixel (i, j):
+ * g = gt[8i, 8j] (F.interpolate(gt, scale_factor=1/8, mode='nearest')), valid as above, class
+ * min(floorf(g * 0.125f + 0.5f), D8 - 1) = the nearest 1/8-res disparity plane (plane k is centred on 8k px).  This GT
+ * rule is this library's definition: the reference's own rule is not pinned by any fixture.  D8 <= 64. */
+int dca_class_confusion(const float* logits, const float* gt, unsigned long long* conf, int B, int D8, int H8, int W8,
+                        float max_valid, void* stream);
+
 /* layout + parameter preparation ---------------------------------------------------------------- */
 int dca_planes_from_ncdhw(const float* x, void* y, int planes, int B, int C, int Cp, int D, int H, int W,
                           void* stream);
