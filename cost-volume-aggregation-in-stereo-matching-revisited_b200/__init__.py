@@ -2,6 +2,7 @@
 from . import _lib, engine, evaluation, frontend, gwcnet, hshard, kitti_io, pipeline
 from . import gwcnet_dca0_g, gwcnet_dca1_g, gwcnet_dca2_g, gwcnet_dca4_g
 from .cva import Multi_Aggregation, cva
+from .engine import Confidence
 from .evaluation import DisparityMeter, evaluate_files, read_kitti_disparity, read_pfm
 from .gwcnet_dca_g import GwcNet, feature_extraction, hourglass
 from .pipeline import HotPathPipeline
@@ -13,4 +14,4 @@ from .submodule import (PropgationNet_4x, build_concat_volume, build_cost_planes
 __all__ = ["GwcNet", "feature_extraction", "hourglass", "cva", "Multi_Aggregation", "SemanticLevelContext",
            "SelfAttentionBlock", "PropgationNet_4x", "build_gwc_volume", "build_concat_volume", "build_cost_planes",
            "disparity_regression", "softmax_disparity_regression", "convbn", "convbn_3d", "engine", "hshard", "kitti_io", "HotPathPipeline",
-           "evaluation", "DisparityMeter", "evaluate_files", "read_pfm", "read_kitti_disparity"]
+           "evaluation", "DisparityMeter", "evaluate_files", "read_pfm", "read_kitti_disparity", "Confidence"]

@@ -5,6 +5,7 @@
 //
 //   disparity_metrics   per image: valid / sum |pred - gt| (fixed point) / E > 1, 2, 3 / D1 / non-finite predictions
 //   class_confusion     conf[gt class][predicted class] of the 1/8-res DCA class maps
+//   confidence_histograms  (count, sum |E|) per confidence bin and per error bin: the sparsification curves
 #include <limits.h>
 
 #include "dca_common.cuh"
@@ -27,13 +28,18 @@ struct MetricAcc {
   unsigned long long sum;
 };
 
+// |E| in the fixed point of DCA_METRIC_SUM_ABS (2^-20 px units)
+__device__ __forceinline__ unsigned long long abs_err_fix(float e) {
+  return __float2ull_rn(__fmul_rn(fminf(e, MT_CLAMP), MT_FIX));
+}
+
 __device__ __forceinline__ void metric_pixel(float p, float g, float max_valid, MetricAcc& a) {
   if (!gt_valid(g, max_valid)) return;
   const float e = fabsf(__fsub_rn(p, g));
   const bool bad = !isfinite(p);               // NaN / inf prediction: an error of every kind, kept out of the sum
   a.valid += 1;
   a.nonfinite += bad;
-  if (!bad) a.sum += __float2ull_rn(__fmul_rn(fminf(e, MT_CLAMP), MT_FIX));
+  if (!bad) a.sum += abs_err_fix(e);
   a.gt1 += bad || e > 1.f;
   a.gt2 += bad || e > 2.f;
   a.gt3 += bad || e > 3.f;
@@ -127,6 +133,46 @@ class_confusion_kernel(const float* __restrict__ logits, const float* __restrict
   }
 }
 
+// Pooled (count, sum |E|) tables over the pixels that enter DCA_METRIC_SUM_ABS, binned by the confidence and by the error
+// itself.  Both tables live in shared memory (36.9 KB) for the whole grid-stride loop and are flushed with one global
+// atomic per non-zero entry, as class_confusion_kernel does.
+constexpr int CH_THREADS = 256;
+constexpr int CH_ERR_SHIFT = 15;           // 2^-20 px units -> 1/32 px bins
+__global__ void __launch_bounds__(CH_THREADS)
+confidence_histograms_kernel(const float* __restrict__ pred, const float* __restrict__ gt, const float* __restrict__ peak,
+                             unsigned long long* __restrict__ conf_hist, unsigned long long* __restrict__ err_hist,
+                             size_t n, float max_valid) {
+  __shared__ unsigned long long s_conf[DCA_CONF_BINS][2];
+  __shared__ unsigned long long s_err[DCA_ERR_BINS][2];
+  for (int i = threadIdx.x; i < 2 * DCA_CONF_BINS; i += CH_THREADS) (&s_conf[0][0])[i] = 0ull;
+  for (int i = threadIdx.x; i < 2 * DCA_ERR_BINS; i += CH_THREADS) (&s_err[0][0])[i] = 0ull;
+  pdl_wait();
+  __syncthreads();
+  for (size_t i = (size_t)blockIdx.x * CH_THREADS + threadIdx.x; i < n; i += (size_t)gridDim.x * CH_THREADS) {
+    const float p = __ldg(pred + i), g = __ldg(gt + i);
+    if (!gt_valid(g, max_valid) || !isfinite(p)) continue;
+    const unsigned long long fix = abs_err_fix(fabsf(__fsub_rn(p, g)));
+    const float c = __ldg(peak + i);
+    const int cb = (isfinite(c) && c >= 0.f) ? (int)fminf(floorf(__fmul_rn(c, (float)DCA_CONF_BINS)),
+                                                          (float)(DCA_CONF_BINS - 1)) : 0;
+    const unsigned long long eb64 = fix >> CH_ERR_SHIFT;
+    const int eb = eb64 < (unsigned long long)(DCA_ERR_BINS - 1) ? (int)eb64 : DCA_ERR_BINS - 1;
+    atomicAdd(&s_conf[cb][0], 1ull);
+    atomicAdd(&s_conf[cb][1], fix);
+    atomicAdd(&s_err[eb][0], 1ull);
+    atomicAdd(&s_err[eb][1], fix);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < 2 * DCA_CONF_BINS; i += CH_THREADS) {
+    const unsigned long long v = (&s_conf[0][0])[i];
+    if (v) atomicAdd(conf_hist + i, v);
+  }
+  for (int i = threadIdx.x; i < 2 * DCA_ERR_BINS; i += CH_THREADS) {
+    const unsigned long long v = (&s_err[0][0])[i];
+    if (v) atomicAdd(err_hist + i, v);
+  }
+}
+
 }  // namespace dca
 
 using namespace dca;
@@ -155,6 +201,20 @@ extern "C" int dca_class_confusion(const float* logits, const float* gt, unsigne
   const int grid = chunks < 8 * dca_num_sms() ? chunks : 8 * dca_num_sms();
   dca_launch(class_confusion_kernel, dim3(grid), CS_THREADS, (size_t)D8 * D8 * sizeof(unsigned), (cudaStream_t)stream,
              logits, gt, conf, B, D8, H8, W8, max_valid);
+  DCA_RETURN_IF_LAUNCH_FAILED();
+  return DCA_OK;
+}
+
+extern "C" int dca_confidence_histograms(const float* pred, const float* gt, const float* peak,
+                                         unsigned long long* conf_hist, unsigned long long* err_hist, int B, int H,
+                                         int W, float max_valid, void* stream) {
+  if (!pred || !gt || !peak || !conf_hist || !err_hist || B <= 0 || H <= 0 || W <= 0 || max_valid != max_valid)
+    return DCA_ERR_ARG;
+  const size_t n = (size_t)B * H * W;
+  const size_t want = (n + CH_THREADS - 1) / CH_THREADS;
+  const size_t cap = 2 * (size_t)dca_num_sms();          // every block zeroes and flushes 36.9 KB of tables
+  dca_launch(confidence_histograms_kernel, dim3((unsigned)(want < cap ? want : cap)), CH_THREADS, 0,
+             (cudaStream_t)stream, pred, gt, peak, conf_hist, err_hist, n, max_valid);
   DCA_RETURN_IF_LAUNCH_FAILED();
   return DCA_OK;
 }

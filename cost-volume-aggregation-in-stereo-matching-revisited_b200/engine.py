@@ -9,6 +9,7 @@ planes=2 ("parity": hi + lo, 22-bit significand) or planes=1 ("fast": a single 1
 """
 from __future__ import annotations
 
+import collections
 import os
 
 import torch
@@ -554,6 +555,25 @@ def convex_upsample(mask, disp):
     return out
 
 
+# Per-pixel confidence of pred4 (include/dca_b200.h section 4): peak = convex-upsampled max_d p(d), in [0, 1]; std =
+# convex-upsampled 4 * (standard deviation of the disparity distribution), in full-res px.  fp32 [B,1,H,W] each.
+Confidence = collections.namedtuple("Confidence", ["peak", "std"])
+
+
+def softmax_confidence_upsample(logits, mask, quarter=False):
+    """logits [B,D,H,W] + prop-net mask -> (Confidence at 4H x 4W, peak_q, std_q); the 1/4-res maps [B,1,H,W] only when
+    `quarter`, else None."""
+    B, D, H, W = logits.shape
+    dev = logits.device
+    peak = torch.empty((B, 1, 4 * H, 4 * W), dtype=torch.float32, device=dev)
+    std = torch.empty((B, 1, 4 * H, 4 * W), dtype=torch.float32, device=dev)
+    pq = torch.empty((B, 1, H, W), dtype=torch.float32, device=dev) if quarter else None
+    sq = torch.empty((B, 1, H, W), dtype=torch.float32, device=dev) if quarter else None
+    _lib.call("dca_softmax_confidence_upsample", logits.data_ptr(), mask.data_ptr(), _ptr(pq), _ptr(sq), peak.data_ptr(),
+              std.data_ptr(), B, D, H, W, _stream())
+    return Confidence(peak, std), pq, sq
+
+
 def fused_volume(gwc_l, gwc_r, cat_l, cat_r, D, G, planes, Cv=None):
     _require_cuda(gwc_l, gwc_r, cat_l, cat_r)
     B, C, H, W = gwc_l.shape
@@ -843,9 +863,11 @@ def check_feature_shapes(pk, gwc_l, gwc_r, cat_l, cat_r, g):
                             "multiple of 8 (the reference's callers pad to 16, main_dca.py:153-166)")
 
 
-def hot_path_forward(pk: PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g, keep=None):
-    """Feature maps -> (pred4 [B,1,H,W], prob_volume2 logits [B,D8,H8,W8]).
-    Mirrors GwcNet.forward (eval) of the reference, models/gwcnet_dca_g.py:216-240,282."""
+def hot_path_forward(pk: PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g, keep=None, confidence=False):
+    """Feature maps -> (pred4 [B,1,H,W], prob_volume2 logits [B,D8,H8,W8]), plus a third item Confidence(peak, std)
+    (fp32 [B,1,H,W] each) when `confidence`.  Mirrors GwcNet.forward (eval) of the reference,
+    models/gwcnet_dca_g.py:216-240,282; the confidence is this library's addition (one more launch after the upsampling,
+    pred4 and prob_volume2 unchanged bit for bit)."""
     _require_cuda(gwc_l, gwc_r, cat_l, cat_r, g)
     check_feature_shapes(pk, gwc_l, gwc_r, cat_l, cat_r, g)
     P = pk.planes
@@ -855,12 +877,12 @@ def hot_path_forward(pk: PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g, keep=None
                        _f32c(cat_r) if cat_r is not None else None, D4, pk.num_groups, P)
     tc0 = Options.use_tc
     try:
-        return _hot_path_stages(pk, vol, side_job, tc0, keep)
+        return _hot_path_stages(pk, vol, side_job, tc0, keep, confidence)
     finally:
         Options.use_tc = tc0          # fp32_stages (diagnostics) toggles it per stage; never leak that into later calls
 
 
-def _hot_path_stages(pk, vol, side_job, tc0, keep):
+def _hot_path_stages(pk, vol, side_job, tc0, keep, confidence=False):
     Options.use_tc = tc0 and "dres" not in Options.fp32_stages
     c = conv(vol, pk.dres0_0, K3S1, ACT_RELU)
     c = conv(c, pk.dres0_2, K3S1, ACT_RELU)
@@ -878,8 +900,9 @@ def _hot_path_stages(pk, vol, side_job, tc0, keep):
     Options.use_tc = tc0 and "cls3" not in Options.fp32_stages
     P27 = conv_taps27(cur, pk.cls3_0, pk.cls3_2)
     if P27 is not None:
-        # the head's logits are only an OUTPUT when there is no cva stage (gwcnet_dca0_g.py:190) or when a caller keeps them
-        pred_q, logits = tap_gather_softmax_regress(P27, want_logits=(not pk.cva) or keep is not None)
+        # the head's logits are only an OUTPUT when there is no cva stage (gwcnet_dca0_g.py:190), when a caller keeps them
+        # or when the confidence is wanted
+        pred_q, logits = tap_gather_softmax_regress(P27, want_logits=(not pk.cva) or keep is not None or confidence)
     else:
         h = conv(cur, pk.cls3_0, K3S1, ACT_RELU)
         logits = conv_cout1_any(h, pk.cls3_2)
@@ -887,10 +910,15 @@ def _hot_path_stages(pk, vol, side_job, tc0, keep):
     Options.use_tc = tc0
     mask = _prop_mask_wait(side_job)
     pred4 = convex_upsample(mask, pred_q)
+    if confidence:
+        conf, peak_q, std_q = softmax_confidence_upsample(logits, mask, quarter=keep is not None)
     if keep is not None:
         keep.update(volume=vol, dres0=c, cost0=cost0, out1=out1, classif3_logits=logits, pred_quarter=pred_q, mask=mask)
         keep.update({f"cva{i + 1}": k for i, k in enumerate(kept)})
-    return pred4, (logits if not pk.cva else logits2)     # no cva stage (gwcnet_dca0_g.py:190): the head's own logits
+        if confidence:
+            keep.update(peak_quarter=peak_q, std_quarter=std_q)
+    pv = logits if not pk.cva else logits2     # no cva stage (gwcnet_dca0_g.py:190): the head's own logits
+    return (pred4, pv, conf) if confidence else (pred4, pv)
 
 
 # --------------------------------------------------------------------------------------------
@@ -904,7 +932,8 @@ class GraphedHotPath:
     The graph reads the caller's input tensors IN PLACE (their addresses are baked in): calling again with the same
     tensors (new contents) replays; other tensors capture another graph (a small LRU of them, all sharing one memory
     pool -- their replays are ordered on the calling stream, so they may reuse each other's activations).  Results are
-    returned as copies, so they survive the next replay.  Weights are baked in as well: `GwcNet` drops its graphs
+    returned as copies, so they survive the next replay.  `confidence` is part of the graph key: the forward with the
+    confidence maps is a graph of its own.  Weights are baked in as well: `GwcNet` drops its graphs
     whenever it drops its packed parameters."""
     MAX_GRAPHS = 8
 
@@ -918,35 +947,36 @@ class GraphedHotPath:
     def _key(tensors):
         return tuple((0, ()) if t is None else (t.data_ptr(), tuple(t.shape)) for t in tensors)
 
-    def _capture(self, ins):
+    def _capture(self, ins, confidence=False):
         s = torch.cuda.Stream(device=ins[0].device)
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s):                 # warm-up outside the capture: lazy module loads, persistent side buffers
             for _ in range(2):
-                hot_path_forward(self.pk, *ins)
+                hot_path_forward(self.pk, *ins, confidence=confidence)
         torch.cuda.current_stream().wait_stream(s)
         torch.cuda.synchronize(ins[0].device)
         g = torch.cuda.CUDAGraph()
         if self.pool is None:
             self.pool = torch.cuda.graph_pool_handle()
         with torch.cuda.graph(g, pool=self.pool):
-            out = hot_path_forward(self.pk, *ins)
+            out = hot_path_forward(self.pk, *ins, confidence=confidence)
         return g, out
 
-    def __call__(self, gwc_l, gwc_r, cat_l, cat_r, g):
+    def __call__(self, gwc_l, gwc_r, cat_l, cat_r, g, confidence=False):
         ins = (gwc_l, gwc_r, cat_l, cat_r, g)
         _require_cuda(*ins)
         for t in ins:
             if t is not None and (t.dtype != torch.float32 or not t.is_contiguous()):
                 raise _lib.DcaError("the graphed forward reads its inputs in place: contiguous fp32 tensors only")
-        key = self._key(ins)
+        confidence = bool(confidence)
+        key = self._key(ins) + (confidence,)
         hit = self.graphs.pop(key, None)
         if hit is None:
             if len(self.graphs) >= self.MAX_GRAPHS:
                 self.graphs.pop(next(iter(self.graphs)))
-            graph, out = self._capture(ins)
+            graph, out = self._capture(ins, confidence)
             hit = (graph, out, ins)
         self.graphs[key] = hit                     # most recently used last
         hit[0].replay()
         self.replays += 1
-        return tuple(o.clone() for o in hit[1])
+        return tuple(o.clone() if torch.is_tensor(o) else type(o)(*(t.clone() for t in o)) for o in hit[1])

@@ -3,12 +3,14 @@
   read_pfm, read_kitti_disparity   ground-truth readers (SceneFlow / Middlebury PFM, KITTI uint16 PNG)
   DisparityMeter                   device-side accumulator: per-image counters of dca_disparity_metrics (EPE, >1/2/3 px,
                                    D1, utils/metrics.py:45-63) and the DCA class-map confusion matrix of
-                                   dca_class_confusion (main_dca.py:66-120, 209-232); no host sync until read back
-  summarize                        counters -> EPE / bad-N / D1 under both conventions, pixel accuracy / mPA / mIoU
+                                   dca_class_confusion (main_dca.py:66-120, 209-232), and with a confidence map the
+                                   sparsification tables of dca_confidence_histograms; no host sync until read back
+  summarize                        counters -> EPE / bad-N / D1 under both conventions, pixel accuracy / mPA / mIoU,
+                                   sparsification curves and AUSE of the confidence
   evaluate_files                   the `mytest` loop as a streaming pipeline (ImagePipeline plus a GT slot per pair)
 
-Per-rank meters of a distributed run combine by concatenating their `rows()` (and summing `confusion()`) before
-`summarize`.  There is no CPU path: the kernels need CUDA tensors.
+Per-rank meters of a distributed run combine by concatenating their `rows()` (and summing `confusion()` and the
+`sparsification_histograms()`) before `summarize`.  There is no CPU path: the kernels need CUDA tensors.
 """
 import warnings
 
@@ -24,6 +26,10 @@ from .kitti_io import (ImagePipeline, crop_prediction, fit_gt_to_crop, load_pair
 VALID, SUM_ABS, GT1, GT2, GT3, D1, PRED_NONFINITE = range(7)
 METRIC_COUNT = 7
 SUM_ABS_UNIT = 2.0 ** -20          # SUM_ABS is fixed point: px = SUM_ABS * 2^-20
+CONF_BINS = 256                    # DCA_CONF_BINS: confidence bins of width 1/256
+ERR_BINS = 2048 + 1                # DCA_ERR_BINS: 1/32 px error bins over [0, 64) and one for E >= 64
+ERR_BIN_PX = 1.0 / 32
+SPARSIFICATION_DENSITY = [k / 20 for k in range(20, 0, -1)]        # 1.00, 0.95, ..., 0.05
 
 
 # ---- ground-truth readers (host) ---------------------------------------------------------------------------
@@ -73,6 +79,15 @@ def _class_confusion(logits, gt, conf, max_valid):
               torch.cuda.current_stream(logits.device).cuda_stream)
 
 
+def _confidence_histograms(pred, gt, peak, conf_hist, err_hist, max_valid):
+    """conf_hist int64 [CONF_BINS, 2], err_hist int64 [ERR_BINS, 2] += (count, SUM_ABS) per bin of pred / gt / peak fp32
+    [B,H,W] (dca_confidence_histograms)."""
+    _require_cuda(pred, gt, peak, conf_hist, err_hist)
+    B, H, W = pred.shape
+    _lib.call("dca_confidence_histograms", pred.data_ptr(), gt.data_ptr(), peak.data_ptr(), conf_hist.data_ptr(),
+              err_hist.data_ptr(), B, H, W, max_valid, torch.cuda.current_stream(pred.device).cuda_stream)
+
+
 def _as_bhw(t, what):
     if t.dim() == 4 and t.shape[1] == 1:
         t = t[:, 0]
@@ -103,8 +118,10 @@ class DisparityMeter:
             self.device = torch.device("cuda", torch.cuda.current_device())
         self._cap = max(1, int(capacity))
         self._rows = self._conf = None
+        self._conf_hist = self._err_hist = None
         self._n = 0
         self._has_conf = False
+        self._with_confidence = None      # set by the first update: every update carries a confidence map, or none does
         if self.device is not None:
             self._alloc()
 
@@ -115,10 +132,13 @@ class DisparityMeter:
     def __len__(self):
         return self._n
 
-    def update(self, pred4, disp_true, prob_volume=None):
+    def update(self, pred4, disp_true, prob_volume=None, confidence=None):
         """Score a batch: pred4 [B,1,H,W] (or [B,H,W]) against disp_true [B,H,W] (or [B,1,H,W]) in the same pixel
         frame, both fp32 on the same device; prob_volume [B,D8,H/8,W/8] (the model's second output) adds to the
-        confusion matrix."""
+        confusion matrix; confidence (the `peak` map of the model's Confidence output, in pred4's frame) adds to the
+        sparsification tables.  Either every update of a meter passes a confidence map or none does (ValueError
+        otherwise): the tables must cover the same pixels as the counter rows, so that the sparsification curves end
+        at epe_pooled."""
         pred, gt = _as_bhw(pred4, "pred4"), _as_bhw(disp_true, "disp_true")
         if gt.shape != pred.shape:
             raise ValueError(f"disp_true {tuple(gt.shape)} and pred4 {tuple(pred.shape)} differ")
@@ -135,6 +155,15 @@ class DisparityMeter:
                     or pv.dtype != torch.float32 or pv.device != self.device:
                 raise ValueError(f"prob_volume {tuple(pv.shape)} {pv.dtype}: expected float32 "
                                  f"[{B}, {self.D8}, {H}/8, {W}/8] on {self.device}")
+        if self._with_confidence is not None and (confidence is not None) != self._with_confidence:
+            raise ValueError("confidence: every update of a meter passes a confidence map or none does (this meter has "
+                             f"had updates {'with' if self._with_confidence else 'without'} one)")
+        pk = None
+        if confidence is not None:
+            pk = _as_bhw(confidence, "confidence")
+            if pk.shape != pred.shape or pk.device != self.device:
+                raise ValueError(f"confidence {tuple(pk.shape)} on {pk.device}: expected {tuple(pred.shape)} "
+                                 f"on {self.device}")
         B = pred.shape[0]
         if self._n + B > self._cap:
             while self._n + B > self._cap:
@@ -146,6 +175,12 @@ class DisparityMeter:
         if pv is not None:
             _class_confusion(pv, gt, self._conf, self.max_valid)
             self._has_conf = True
+        if pk is not None:
+            if self._conf_hist is None:
+                self._conf_hist = torch.zeros((CONF_BINS, 2), dtype=torch.int64, device=self.device)
+                self._err_hist = torch.zeros((ERR_BINS, 2), dtype=torch.int64, device=self.device)
+            _confidence_histograms(pred, gt, pk, self._conf_hist, self._err_hist, self.max_valid)
+        self._with_confidence = confidence is not None
         self._n += B
 
     def _readback(self, t):
@@ -165,8 +200,16 @@ class DisparityMeter:
             return np.zeros((self.D8, self.D8), np.uint64)
         return self._readback(self._conf)
 
+    def sparsification_histograms(self):
+        """(conf_hist [CONF_BINS, 2], err_hist [ERR_BINS, 2]) numpy uint64 of (count, SUM_ABS) per bin, or None before
+        any update with a confidence map."""
+        if self._conf_hist is None:
+            return None
+        return self._readback(self._conf_hist), self._readback(self._err_hist)
+
     def summary(self):
-        return summarize(self.rows(), self.confusion() if self._has_conf else None)
+        h = self.sparsification_histograms()
+        return summarize(self.rows(), self.confusion() if self._has_conf else None, *(h or (None, None)))
 
 
 def _nanmean(a):
@@ -175,8 +218,38 @@ def _nanmean(a):
         return float(np.nanmean(a)) if a.size else float("nan")
 
 
-def summarize(rows, confusion=None):
-    """Counter rows [N, METRIC_COUNT] (+ confusion [D8,D8]) -> dict of metrics.
+def _sparsification_curve(hist, order):
+    """EPE (px) of the most trusted fraction q of the pixels for every q of SPARSIFICATION_DENSITY: bins are taken
+    whole in `order`, the boundary bin with the same fraction of its count and of its sum."""
+    h = np.asarray(hist, dtype=np.uint64).reshape(-1, 2)[order]
+    n, s = [int(v) for v in h[:, 0]], [int(v) for v in h[:, 1]]      # Python ints: exact sums
+    total = sum(n)
+    out = []
+    for q in SPARSIFICATION_DENSITY:
+        if not total:
+            out.append(float("nan"))
+            continue
+        target = total * q
+        take_n = take_s = 0
+        part = 0.0
+        for k in range(len(n)):
+            if take_n + n[k] > target:
+                part = (target - take_n) / n[k] * s[k]
+                break
+            take_n += n[k]
+            take_s += s[k]
+        out.append((take_s + part) * SUM_ABS_UNIT / target)
+    return out
+
+
+def _auc(curve):
+    """Trapezoid of a sparsification curve over the removed fraction x = 1 - q in [0, 0.95]."""
+    x = [1.0 - q for q in SPARSIFICATION_DENSITY]
+    return float(sum(0.5 * (curve[i] + curve[i + 1]) * (x[i + 1] - x[i]) for i in range(len(x) - 1)))
+
+
+def summarize(rows, confusion=None, conf_hist=None, err_hist=None):
+    """Counter rows [N, METRIC_COUNT] (+ confusion [D8,D8]) (+ the sparsification tables) -> dict of metrics.
 
     epe, bad1, bad2, bad3, d1            mean over images of the per-image values (GwcNet / PSMNet test loops); images
                                          without valid pixels are skipped and counted in n_images_skipped
@@ -185,7 +258,18 @@ def summarize(rows, confusion=None):
     left out of the EPE sum (the EPE is over the valid pixels with a finite prediction; n_pred_nonfinite says how many
     were not).  From the confusion matrix, the segmentation Evaluator's formulas (main_dca.py:66-120):
     pixel_accuracy = trace / total, mpa = nanmean(diag / row sums), miou = nanmean(diag / (row + column sums - diag));
-    classes with neither GT nor predictions are nan and left out of the means."""
+    classes with neither GT nor predictions are nan and left out of the means.
+
+    With both sparsification tables (DisparityMeter.sparsification_histograms):
+    sparsification_density       q = 1.00, 0.95, ..., 0.05
+    sparsification_epe           EPE of the N*q most confident pixels (highest confidence bins first; the boundary bin
+                                 contributes the same fraction of its count and of its sum |E|)
+    sparsification_epe_ideal     the same with the lowest-error bins first: the best any ranking can do, to within one
+                                 error bin (1/32 px) as long as the boundary bin is not the E >= 64 px one (the
+                                 error-sorted curve of the sparsification literature; DESIGN.md section 4 on its name)
+    auc_epe, ause_epe            trapezoid of the confidence curve over the removed fraction 1 - q in [0, 0.95], and
+                                 that minus the same area of the ideal curve (px; 0 = a perfect ranking)
+    At q = 1 both curves equal epe_pooled exactly (the same integer sums)."""
     r = np.asarray(rows, dtype=np.uint64).reshape(-1, METRIC_COUNT).astype(np.float64)
     valid, nonfinite = r[:, VALID], r[:, PRED_NONFINITE]
     finite = valid - nonfinite
@@ -211,6 +295,14 @@ def summarize(rows, confusion=None):
             out["mpa"] = _nanmean(diag / gt_n)
             out["miou"] = _nanmean(diag / (gt_n + pred_n - diag))
             out["n_class_pixels"] = int(total)
+    if conf_hist is not None and err_hist is not None:
+        curve = _sparsification_curve(conf_hist, slice(None, None, -1))
+        ideal = _sparsification_curve(err_hist, slice(None))
+        out["sparsification_density"] = list(SPARSIFICATION_DENSITY)
+        out["sparsification_epe"] = curve
+        out["sparsification_epe_ideal"] = ideal
+        out["auc_epe"] = _auc(curve)
+        out["ause_epe"] = out["auc_epe"] - _auc(ideal)
     return out
 
 
@@ -227,11 +319,11 @@ class EvalPipeline(ImagePipeline):
     mode "fit": fit_to_crop / fit_gt_to_crop into crop_height x crop_width (my_img.py); "pad16": top/right zero padding
     to multiples of 16 (main_dca.py:153-166), slot buffers follow each pair's padded size."""
 
-    def __init__(self, model, meter, mode="fit", crop_height=384, crop_width=1248, depth=3, workers=2):
+    def __init__(self, model, meter, mode="fit", crop_height=384, crop_width=1248, depth=3, workers=2, confidence=False):
         if mode not in ("fit", "pad16"):
             raise ValueError(f"mode must be 'fit' or 'pad16', got {mode!r}")
         super().__init__(model, crop_height, crop_width, depth, workers)
-        self.meter, self.mode = meter, mode
+        self.meter, self.mode, self.confidence = meter, mode, confidence
         self.gt_host = [self._host(crop_height, crop_width) for _ in range(self.depth)]
         self.gt_dev = [torch.empty((crop_height, crop_width), dtype=torch.float32, device=self.dev)
                        for _ in range(self.depth)] if self.cuda else self.gt_host
@@ -268,6 +360,10 @@ class EvalPipeline(ImagePipeline):
 
     def _forward_eval(self, slot):
         x = self.in_dev[slot]
+        if self.confidence:          # (pred, prob_volume, Confidence(peak, std)): the peak map ranks the pixels
+            pred, pv, conf = self.model(x[None, 0:3], x[None, 3:6], confidence=True)
+            self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None, conf.peak)
+            return pred.reshape(x.shape[1], x.shape[2])
         out = self.model(x[None, 0:3], x[None, 3:6])
         pred, pv = (out[0], out[1]) if isinstance(out, (tuple, list)) else (out, None)
         self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None)
@@ -349,10 +445,12 @@ class EvalPipeline(ImagePipeline):
             raise err[0]
 
 
-def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=2, maxdisp=None, max_valid=None):
+def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=2, maxdisp=None, max_valid=None,
+                   confidence=False):
     """main_dca.py `mytest` over files: quads = (left, right, gt_path, savename or None); GT is a KITTI PNG or a PFM
     (by extension).  maxdisp defaults to model.maxdisp, max_valid as in DisparityMeter.  Returns (summary dict,
-    per-image counter rows [N, METRIC_COUNT] in input order); synchronises once, at the end."""
+    per-image counter rows [N, METRIC_COUNT] in input order); synchronises once, at the end.  confidence=True runs
+    model(left, right, confidence=True) and adds the sparsification curves of its `peak` map to the summary."""
     if maxdisp is None:
         maxdisp = getattr(model, "maxdisp", 192)
     try:
@@ -360,6 +458,7 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
     except (StopIteration, AttributeError):
         dev = torch.device("cpu")
     meter = DisparityMeter(maxdisp, max_valid, dev)
-    EvalPipeline(model, meter, mode, crop[0], crop[1], depth, workers).run(quads)
+    EvalPipeline(model, meter, mode, crop[0], crop[1], depth, workers, confidence).run(quads)
     rows = meter.rows()
-    return summarize(rows, meter.confusion() if meter._has_conf else None), rows
+    h = meter.sparsification_histograms()
+    return summarize(rows, meter.confusion() if meter._has_conf else None, *(h or (None, None))), rows

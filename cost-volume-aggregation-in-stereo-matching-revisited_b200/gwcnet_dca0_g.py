@@ -10,8 +10,8 @@ class GwcNet(_GwcNet3):
     PV_STAGE = 0
     SQUEEZE_PRED = True
 
-    def forward(self, left, right, disp_true=None):     # reference signature: forward(left, right)
-        return super().forward(left, right)
+    def forward(self, left, right, disp_true=None, *, confidence=False):     # reference signature: forward(left, right)
+        return super().forward(left, right, confidence=confidence)
 
 
 def GwcNet_G(d):

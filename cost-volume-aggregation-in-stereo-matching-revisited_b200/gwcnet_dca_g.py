@@ -179,16 +179,18 @@ class GwcNet(nn.Module):
         return super().load_state_dict(state_dict, strict=strict, **kw)
 
     # ---- forward -------------------------------------------------------------------------
-    def hot_path(self, gwc_l, gwc_r, cat_l, cat_r, g, keep=None):
-        """feature maps -> (pred4 [B,1,H,W], prob_volume2 [B,D8,H8,W8]); the graded path."""
-        return engine.hot_path_forward(self.packed(), gwc_l, gwc_r, cat_l, cat_r, g, keep)
+    def hot_path(self, gwc_l, gwc_r, cat_l, cat_r, g, keep=None, confidence=False):
+        """feature maps -> (pred4 [B,1,H,W], prob_volume2 [B,D8,H8,W8]); the graded path.  confidence=True adds a third
+        item, `Confidence(peak, std)` (fp32 [B,1,H,W] each, include/dca_b200.h section 4); pred4 and prob_volume2 stay
+        bit-identical."""
+        return engine.hot_path_forward(self.packed(), gwc_l, gwc_r, cat_l, cat_r, g, keep, confidence)
 
-    def hot_path_graphed(self, gwc_l, gwc_r, cat_l, cat_r, g):
+    def hot_path_graphed(self, gwc_l, gwc_r, cat_l, cat_r, g, confidence=False):
         """`hot_path` as one CUDA graph per set of input buffers (captured on first use, replayed afterwards; the inputs
         are read in place, results are returned as copies).  Same kernels, same results, one launch.  Graphs (and their
         shared activation pool) are kept per CALLING stream, so forwards replayed concurrently on several streams do not
-        share buffers."""
-        return self.graphed()(gwc_l, gwc_r, cat_l, cat_r, g)
+        share buffers.  With and without `confidence` are two graphs."""
+        return self.graphed()(gwc_l, gwc_r, cat_l, cat_r, g, confidence)
 
     def graphed(self):
         """The `engine.GraphedHotPath` of the current stream (created on first use; dropped with the packed parameters)."""
@@ -209,7 +211,9 @@ class GwcNet(nn.Module):
         return hshard.hot_path_forward_hsharded(self.packed(), gwc_l, gwc_r, cat_l, cat_r, g, rank, world, group,
                                                 transport)
 
-    def forward(self, left, right, disp_true=None):
+    def forward(self, left, right, disp_true=None, *, confidence=False):
+        """(pred, prob_volume) as the reference's eval forward; confidence=True adds `Confidence(peak, std)`, shaped like
+        pred (squeezed with it in the 0/1/2-stage variants)."""
         if self.training:
             raise NotImplementedError("dcanet_b200 is an inference engine: call .eval() (training-mode heads "
                                       "classif0-2 exist only so checkpoints load)")
@@ -219,5 +223,11 @@ class GwcNet(nn.Module):
             f = self.feature_extraction(torch.cat((left, right), dim=0))      # eval-mode BN: batching changes nothing
             g = self.guidance(left)["g"]
         gwc, cat = f["gwc_feature"], f.get("concat_feature")
-        pred, pv = self.hot_path(gwc[:B], gwc[B:], None if cat is None else cat[:B], None if cat is None else cat[B:], g)
-        return (pred.squeeze(1) if self.SQUEEZE_PRED else pred), pv
+        out = self.hot_path(gwc[:B], gwc[B:], None if cat is None else cat[:B], None if cat is None else cat[B:], g,
+                            confidence=confidence)
+        sq = (lambda t: t.squeeze(1)) if self.SQUEEZE_PRED else (lambda t: t)
+        if confidence:
+            pred, pv, conf = out
+            return sq(pred), pv, engine.Confidence(sq(conf.peak), sq(conf.std))
+        pred, pv = out
+        return sq(pred), pv

@@ -206,6 +206,23 @@ int dca_softmax_regress(const float* logits, float* pred, int B, int D, int H, i
 /* disparity_regression on its own (models/submodule.py:127-131): pred[b,h,w] = sum_d d * x[b,d,h,w], x not renormalised. */
 int dca_regress_f32(const float* x, float* pred, int B, int D, int H, int W, void* stream);
 int dca_convex_upsample(const float* mask, const float* disp, float* out, int B, int H, int W, void* stream);
+/* Per-pixel confidence of the disparity, from the classif head's logits l[d] [B,D,H,W] (D = D4 = maxdisp / 4) at 1/4 res.
+ * With p = softmax_d(l) and mu = sum_d d p(d) (= pred_quarter):
+ *   peak_q = max_d p(d)                          in [1/D, 1]
+ *   std_q  = sqrt(sum_d p(d) (d - mu)^2)         in 1/4-res disparity units; computed in centred form (max, then sum
+ *                                                and mean, then the centred second moment: three passes over the logits),
+ *                                                never as E[d^2] - mu^2, which in fp32 at D = 48 loses ~0.05 px on confident
+ *                                                pixels
+ * At full resolution both maps are convex-upsampled with the 9-neighbour softmax weights of `mask` (the prop net's fp32
+ * channels-last [B,H,W,144], as dca_convex_upsample) and the same zero padding outside the image as pred4:
+ *   peak = up(peak_q) in [0, 1],  std = up(4 std_q) in full-res px.
+ * The upsampled std is a convex combination of the neighbouring stds, not the std of the mixture of their distributions.
+ * The zero padding lowers the confidence along the image border (peak toward 0, std toward 0), exactly where pred4 is
+ * pulled toward 0 by the same padding.
+ * A CTA owns a 32 x 8 tile of 1/4-res pixels and recomputes the statistics of its 1-pixel ring (as
+ * dca_softmax_regress_upsample).  peak_q / std_q [B,H,W] are optional (NULL = not written); peak / std [B,1,4H,4W]. */
+int dca_softmax_confidence_upsample(const float* logits, const float* mask, float* peak_q, float* std_q, float* peak,
+                                    float* std, int B, int D, int H, int W, void* stream);
 
 /* (5) H-sharded single-pair mode: halo rows over NVLink peer memory ------------------------------ */
 /* Replaces, for BASELINE configs[4] (one pair row-sharded over the GPUs of a box, SURVEY section 8e), the exchange a
@@ -280,6 +297,17 @@ int dca_disparity_metrics(const float* pred, const float* gt, unsigned long long
  * rule is this library's definition: the reference's own rule is not pinned by any fixture.  D8 <= 64. */
 int dca_class_confusion(const float* logits, const float* gt, unsigned long long* conf, int B, int D8, int H8, int W8,
                         float max_valid, void* stream);
+/* Sparsification tables of a confidence map: pred, gt, peak fp32 [B,H,W] in the same pixel frame (peak = the full-res
+ * confidence of dca_softmax_confidence_upsample).  Over exactly the pixels that enter DCA_METRIC_SUM_ABS (valid GT, finite
+ * prediction), with F = the per-pixel fixed-point |E| of SUM_ABS:
+ *   conf_hist [DCA_CONF_BINS][2] += (1, F) at bin min(floorf(peak * 256), 255); a NaN, inf or negative peak -> bin 0
+ *   err_hist  [DCA_ERR_BINS][2]  += (1, F) at bin min(F >> 15, 2048): 1/32 px bins over [0, 64), the last one E >= 64
+ * Sums over either table equal SUM_ABS / (VALID - PRED_NONFINITE) of dca_disparity_metrics on the same inputs.  Integer
+ * sums, exact while they stay below 2^64 (E < 512 px: 2^35 pixels). */
+#define DCA_CONF_BINS 256
+#define DCA_ERR_BINS (2048 + 1)
+int dca_confidence_histograms(const float* pred, const float* gt, const float* peak, unsigned long long* conf_hist,
+                              unsigned long long* err_hist, int B, int H, int W, float max_valid, void* stream);
 
 /* layout + parameter preparation ---------------------------------------------------------------- */
 int dca_planes_from_ncdhw(const float* x, void* y, int planes, int B, int C, int Cp, int D, int H, int W,
