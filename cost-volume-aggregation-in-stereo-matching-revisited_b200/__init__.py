@@ -2,7 +2,7 @@
 from . import _lib, engine, evaluation, frontend, gwcnet, hshard, kitti_io, pipeline
 from . import gwcnet_dca0_g, gwcnet_dca1_g, gwcnet_dca2_g, gwcnet_dca4_g
 from .cva import Multi_Aggregation, cva
-from .engine import Confidence
+from .engine import LR_CONSISTENT, LR_MISMATCH, LR_OCCLUDED, LR_OUT_OF_VIEW, Confidence, LRCheck
 from .evaluation import DisparityMeter, evaluate_files, read_kitti_disparity, read_pfm
 from .gwcnet_dca_g import GwcNet, feature_extraction, hourglass
 from .pipeline import HotPathPipeline
@@ -11,7 +11,16 @@ from .semantic_level import SemanticLevelContext
 from .submodule import (PropgationNet_4x, build_concat_volume, build_cost_planes, build_gwc_volume, convbn,
                         convbn_3d, disparity_regression, softmax_disparity_regression)
 
+
+def lr_consistency(disp_left, disp_right, tau=1.0):
+    """Left-right consistency check of two disparities obtained elsewhere, fp32 CUDA [B,H,W] or [B,1,H,W] in their own
+    views -> LRCheck(disp_right, label, filled) shaped like disp_left (include/dca_b200.h section 8)."""
+    label, filled, _ = engine.lr_consistency(disp_left, disp_right, tau)
+    return LRCheck(disp_right, label, filled)
+
+
 __all__ = ["GwcNet", "feature_extraction", "hourglass", "cva", "Multi_Aggregation", "SemanticLevelContext",
            "SelfAttentionBlock", "PropgationNet_4x", "build_gwc_volume", "build_concat_volume", "build_cost_planes",
            "disparity_regression", "softmax_disparity_regression", "convbn", "convbn_3d", "engine", "hshard", "kitti_io", "HotPathPipeline",
-           "evaluation", "DisparityMeter", "evaluate_files", "read_pfm", "read_kitti_disparity", "Confidence"]
+           "evaluation", "DisparityMeter", "evaluate_files", "read_pfm", "read_kitti_disparity", "Confidence",
+           "LRCheck", "lr_consistency", "LR_CONSISTENT", "LR_OCCLUDED", "LR_MISMATCH", "LR_OUT_OF_VIEW"]

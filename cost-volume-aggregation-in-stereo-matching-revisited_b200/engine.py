@@ -574,6 +574,34 @@ def softmax_confidence_upsample(logits, mask, quarter=False):
     return Confidence(peak, std), pq, sq
 
 
+# Left-right consistency check (include/dca_b200.h section 8): the right view's disparity, a per-pixel label and the
+# background-filled disparity, each shaped like the left disparity.
+LRCheck = collections.namedtuple("LRCheck", ["disp_right", "label", "filled"])
+LR_CONSISTENT, LR_OCCLUDED, LR_MISMATCH, LR_OUT_OF_VIEW = 0, 1, 2, 3
+
+
+def lr_consistency(disp_left, disp_right, tau=1.0, mirrored=False, want_right=False):
+    """disp_left, disp_right fp32 [B,H,W] or [B,1,H,W] -> (label uint8, filled fp32, right fp32 or None), shaped like
+    disp_left.  `mirrored`: disp_right is net(flip(R), flip(L)) as the mirrored forward wrote it, i.e. flip(D_R), and is
+    read back to front.  `want_right` also returns D_R in the natural layout, written by the kernel from its staged rows.
+    One launch of dca_lr_consistency; W <= 4096 (DCA_LR_MAX_W)."""
+    _require_cuda(disp_left, disp_right)
+    if disp_left.shape != disp_right.shape or disp_left.dim() not in (3, 4) or \
+            (disp_left.dim() == 4 and disp_left.shape[1] != 1):
+        raise _lib.DcaError(f"disparities must be two equal [B,H,W] or [B,1,H,W] tensors, got "
+                            f"{tuple(disp_left.shape)} / {tuple(disp_right.shape)}")
+    if disp_left.dtype != torch.float32 or disp_right.dtype != torch.float32 or disp_left.device != disp_right.device:
+        raise _lib.DcaError("disparities must be float32 on one device")
+    dl, dr = disp_left.contiguous(), disp_right.contiguous()
+    B, H, W = dl.shape[0], dl.shape[-2], dl.shape[-1]
+    label = torch.empty(dl.shape, dtype=torch.uint8, device=dl.device)
+    filled = torch.empty_like(dl)
+    right = torch.empty_like(dl) if want_right else None
+    _lib.call("dca_lr_consistency", dl.data_ptr(), dr.data_ptr(), int(bool(mirrored)), label.data_ptr(),
+              filled.data_ptr(), _ptr(right), B, H, W, float(tau), _stream())
+    return label, filled, right
+
+
 def fused_volume(gwc_l, gwc_r, cat_l, cat_r, D, G, planes, Cv=None):
     _require_cuda(gwc_l, gwc_r, cat_l, cat_r)
     B, C, H, W = gwc_l.shape

@@ -7,7 +7,9 @@
                                    sparsification tables of dca_confidence_histograms; no host sync until read back
   summarize                        counters -> EPE / bad-N / D1 under both conventions, pixel accuracy / mPA / mIoU,
                                    sparsification curves and AUSE of the confidence
-  evaluate_files                   the `mytest` loop as a streaming pipeline (ImagePipeline plus a GT slot per pair)
+  evaluate_files                   the `mytest` loop as a streaming pipeline (ImagePipeline plus a GT slot per pair);
+                                   with lr_check=True also the metrics of the left-right consistent pixels and of the
+                                   background-filled disparity
 
 Per-rank meters of a distributed run combine by concatenating their `rows()` (and summing `confusion()` and the
 `sparsification_histograms()`) before `summarize`.  There is no CPU path: the kernels need CUDA tensors.
@@ -319,11 +321,16 @@ class EvalPipeline(ImagePipeline):
     mode "fit": fit_to_crop / fit_gt_to_crop into crop_height x crop_width (my_img.py); "pad16": top/right zero padding
     to multiples of 16 (main_dca.py:153-166), slot buffers follow each pair's padded size."""
 
-    def __init__(self, model, meter, mode="fit", crop_height=384, crop_width=1248, depth=3, workers=2, confidence=False):
+    def __init__(self, model, meter, mode="fit", crop_height=384, crop_width=1248, depth=3, workers=2, confidence=False,
+                 lr_check=False, lr_threshold=1.0):
         if mode not in ("fit", "pad16"):
             raise ValueError(f"mode must be 'fit' or 'pad16', got {mode!r}")
         super().__init__(model, crop_height, crop_width, depth, workers)
         self.meter, self.mode, self.confidence = meter, mode, confidence
+        self.lr_check, self.lr_threshold = lr_check, lr_threshold
+        # with lr_check: pred scored on the consistent pixels only, and the background-filled disparity on all of them
+        self.lr_meters = {k: DisparityMeter(meter.maxdisp, meter.max_valid, meter.device)
+                          for k in ("lr_consistent", "lr_filled")} if lr_check else {}
         self.gt_host = [self._host(crop_height, crop_width) for _ in range(self.depth)]
         self.gt_dev = [torch.empty((crop_height, crop_width), dtype=torch.float32, device=self.dev)
                        for _ in range(self.depth)] if self.cuda else self.gt_host
@@ -360,6 +367,16 @@ class EvalPipeline(ImagePipeline):
 
     def _forward_eval(self, slot):
         x = self.in_dev[slot]
+        if self.lr_check:            # (pred, prob_volume, [Confidence,] LRCheck), checked in the network frame
+            gt = self.gt_dev[slot][None]
+            out = self.model(x[None, 0:3], x[None, 3:6], confidence=self.confidence, lr_check=True,
+                             lr_threshold=self.lr_threshold)
+            pred, pv, lr = out[0], out[1], out[-1]
+            self.meter.update(pred, gt, pv if torch.is_tensor(pv) else None, out[2].peak if self.confidence else None)
+            # zero GT = no GT: the inconsistent pixels leave this meter without a change to the metrics kernel
+            self.lr_meters["lr_consistent"].update(pred, torch.where(lr.label.reshape(gt.shape) == 0, gt, 0.0))
+            self.lr_meters["lr_filled"].update(lr.filled, gt)
+            return pred.reshape(x.shape[1], x.shape[2])
         if self.confidence:          # (pred, prob_volume, Confidence(peak, std)): the peak map ranks the pixels
             pred, pv, conf = self.model(x[None, 0:3], x[None, 3:6], confidence=True)
             self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None, conf.peak)
@@ -446,11 +463,18 @@ class EvalPipeline(ImagePipeline):
 
 
 def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=2, maxdisp=None, max_valid=None,
-                   confidence=False):
+                   confidence=False, lr_check=False, lr_threshold=1.0):
     """main_dca.py `mytest` over files: quads = (left, right, gt_path, savename or None); GT is a KITTI PNG or a PFM
     (by extension).  maxdisp defaults to model.maxdisp, max_valid as in DisparityMeter.  Returns (summary dict,
     per-image counter rows [N, METRIC_COUNT] in input order); synchronises once, at the end.  confidence=True runs
-    model(left, right, confidence=True) and adds the sparsification curves of its `peak` map to the summary."""
+    model(left, right, confidence=True) and adds the sparsification curves of its `peak` map to the summary.
+
+    lr_check=True runs model(left, right, lr_check=True, lr_threshold=...) (the check in the network frame, before the
+    crop back); the summary keeps every key of the run without the flag and adds
+      lr_consistent   summarize() of pred against the GT of the pixels labelled consistent only
+      lr_filled       summarize() of the background-filled disparity against the whole GT
+      lr_density      lr_consistent's n_valid / n_valid: the fraction of the valid GT pixels that pass the check
+    The per-image rows returned are those of pred against the whole GT, as without the flag."""
     if maxdisp is None:
         maxdisp = getattr(model, "maxdisp", 192)
     try:
@@ -458,7 +482,14 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
     except (StopIteration, AttributeError):
         dev = torch.device("cpu")
     meter = DisparityMeter(maxdisp, max_valid, dev)
-    EvalPipeline(model, meter, mode, crop[0], crop[1], depth, workers, confidence).run(quads)
+    pipe = EvalPipeline(model, meter, mode, crop[0], crop[1], depth, workers, confidence, lr_check, lr_threshold)
+    pipe.run(quads)
     rows = meter.rows()
     h = meter.sparsification_histograms()
-    return summarize(rows, meter.confusion() if meter._has_conf else None, *(h or (None, None))), rows
+    summary = summarize(rows, meter.confusion() if meter._has_conf else None, *(h or (None, None)))
+    if lr_check:
+        for k, m in pipe.lr_meters.items():
+            summary[k] = summarize(m.rows())
+        n = summary["n_valid"]
+        summary["lr_density"] = summary["lr_consistent"]["n_valid"] / n if n else float("nan")
+    return summary, rows

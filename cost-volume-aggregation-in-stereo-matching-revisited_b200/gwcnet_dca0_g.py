@@ -10,8 +10,9 @@ class GwcNet(_GwcNet3):
     PV_STAGE = 0
     SQUEEZE_PRED = True
 
-    def forward(self, left, right, disp_true=None, *, confidence=False):     # reference signature: forward(left, right)
-        return super().forward(left, right, confidence=confidence)
+    def forward(self, left, right, disp_true=None, *, confidence=False, lr_check=False, lr_threshold=1.0):
+        # reference signature: forward(left, right)
+        return super().forward(left, right, confidence=confidence, lr_check=lr_check, lr_threshold=lr_threshold)
 
 
 def GwcNet_G(d):

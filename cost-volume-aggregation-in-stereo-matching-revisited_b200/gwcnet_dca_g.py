@@ -211,23 +211,38 @@ class GwcNet(nn.Module):
         return hshard.hot_path_forward_hsharded(self.packed(), gwc_l, gwc_r, cat_l, cat_r, g, rank, world, group,
                                                 transport)
 
-    def forward(self, left, right, disp_true=None, *, confidence=False):
+    def forward(self, left, right, disp_true=None, *, confidence=False, lr_check=False, lr_threshold=1.0):
         """(pred, prob_volume) as the reference's eval forward; confidence=True adds `Confidence(peak, std)`, shaped like
-        pred (squeezed with it in the 0/1/2-stage variants)."""
+        pred (squeezed with it in the 0/1/2-stage variants).  lr_check=True appends, last, `LRCheck(disp_right, label,
+        filled)` of the left-right consistency check with threshold `lr_threshold` px (include/dca_b200.h section 8),
+        each shaped like pred: the right view runs in the same forward as the mirrored pair (flip(R), flip(L)), at twice
+        the batch, and pred / prob_volume / Confidence are those of the forward without the flag."""
         if self.training:
             raise NotImplementedError("dcanet_b200 is an inference engine: call .eval() (training-mode heads "
                                       "classif0-2 exist only so checkpoints load)")
         from . import frontend
         B = left.shape[0]
+        nb = 2 * B if lr_check else B       # pairs through the hot path
         with frontend._no_tf32():          # whatever part of the front end runs on cuDNN runs in true fp32
-            f = self.feature_extraction(torch.cat((left, right), dim=0))      # eval-mode BN: batching changes nothing
-            g = self.guidance(left)["g"]
+            if lr_check:                   # left references (L, flip(R)), right images (R, flip(L)): one 4B front end
+                imgs = torch.cat((left, right.flip(-1), right, left.flip(-1)), dim=0)
+                f = self.feature_extraction(imgs)
+                g = self.guidance(imgs[:nb])["g"]
+            else:
+                f = self.feature_extraction(torch.cat((left, right), dim=0))      # eval-mode BN: batching changes nothing
+                g = self.guidance(left)["g"]
         gwc, cat = f["gwc_feature"], f.get("concat_feature")
-        out = self.hot_path(gwc[:B], gwc[B:], None if cat is None else cat[:B], None if cat is None else cat[B:], g,
+        out = self.hot_path(gwc[:nb], gwc[nb:], None if cat is None else cat[:nb], None if cat is None else cat[nb:], g,
                             confidence=confidence)
         sq = (lambda t: t.squeeze(1)) if self.SQUEEZE_PRED else (lambda t: t)
+        left_view = (lambda t: t[:B]) if lr_check else (lambda t: t)
+        pred, pv = out[0], out[1]
+        res = [sq(left_view(pred)), left_view(pv)]
         if confidence:
-            pred, pv, conf = out
-            return sq(pred), pv, engine.Confidence(sq(conf.peak), sq(conf.std))
-        pred, pv = out
-        return sq(pred), pv
+            conf = out[2]
+            res.append(engine.Confidence(sq(left_view(conf.peak)), sq(left_view(conf.std))))
+        if lr_check:
+            label, filled, right_disp = engine.lr_consistency(pred[:B], pred[B:], lr_threshold, mirrored=True,
+                                                              want_right=True)
+            res.append(engine.LRCheck(sq(right_disp), sq(label), sq(filled)))
+        return tuple(res)

@@ -309,6 +309,36 @@ int dca_class_confusion(const float* logits, const float* gt, unsigned long long
 int dca_confidence_histograms(const float* pred, const float* gt, const float* peak, unsigned long long* conf_hist,
                               unsigned long long* err_hist, int B, int H, int W, float max_valid, void* stream);
 
+/* (8) left-right consistency check and background fill ------------------------------------------------------------- */
+/* Right view.  DCANet is not mirror-symmetric (the guidance comes from the left image, the volume is built with the left
+ * image as reference), so the right view's disparity comes from the mirror trick: with flip = mirror of the W axis,
+ *   D_R = flip(net(flip(R), flip(L)))
+ * (the swapped, mirrored pair is again a left-referenced problem with positive disparities).
+ * Check of left pixel (y, x) with d = D_L(y, x), all in fp32 with explicit rounding (no contraction):
+ *   xr = x - d
+ *   not 0 <= xr <= W-1 (a non-finite d included)                                     -> DCA_LR_OUT_OF_VIEW
+ *   x0 = floor(xr), a = xr - x0;  v = D_R[x0] if x0 == W-1, else D_R[x0] + a * (D_R[x0+1] - D_R[x0])
+ *   |d - v| <= tau                                                                   -> DCA_LR_CONSISTENT
+ *   else v - d > tau (the right view sees a nearer surface there)                    -> DCA_LR_OCCLUDED
+ *   else (a non-finite v included)                                                   -> DCA_LR_MISMATCH
+ * Background fill, one row at a time: a consistent pixel keeps D_L; any other pixel takes min(D_L[l], D_L[r]) with l / r
+ * the nearest consistent pixels to its left / right on the same row, the one that exists when only one does, and D_L
+ * when the row has no consistent pixel.  This is the background fill of occlusion handling; mismatches are filled the
+ * same way on purpose, to keep the rule simple.
+ * disp_left, disp_right fp32 [B,H,W] (pred4 [B,1,H,W] is the same memory); right_mirrored != 0 reads disp_right in the
+ * layout of the mirrored forward (disp_right[b, y, W-1-x] = D_R(y, x)), so no flipped copy is needed.  Outputs [B,H,W]:
+ * label uint8 (DCA_LR_*), filled fp32, and disp_right_out (NULL = not written) the un-mirrored D_R.  One CTA per
+ * (image, row) stages a row in shared memory, 9 bytes per pixel: W <= DCA_LR_MAX_W keeps that under the 48 KB a CTA gets
+ * without an opt-in (DCA_ERR_UNSUPPORTED above).  DCA_ERR_ARG for NULL required pointers, B, H, W <= 0, B > 65535, and a
+ * tau that is NaN or negative. */
+#define DCA_LR_CONSISTENT 0
+#define DCA_LR_OCCLUDED 1
+#define DCA_LR_MISMATCH 2
+#define DCA_LR_OUT_OF_VIEW 3
+#define DCA_LR_MAX_W 4096
+int dca_lr_consistency(const float* disp_left, const float* disp_right, int right_mirrored, unsigned char* label,
+                       float* filled, float* disp_right_out, int B, int H, int W, float tau, void* stream);
+
 /* layout + parameter preparation ---------------------------------------------------------------- */
 int dca_planes_from_ncdhw(const float* x, void* y, int planes, int B, int C, int Cp, int D, int H, int W,
                           void* stream);
