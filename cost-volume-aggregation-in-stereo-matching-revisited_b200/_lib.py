@@ -35,7 +35,6 @@ SIGNATURES = {
     "dca_conv3d_tc_taps27": [_vp, _c_int, _vp, _c_int, _vp, _vp, _vp, _vp, _c_int] + [_c_int] * 5 + [_vp],
     "dca_tap_gather_softmax_regress": [_vp, _vp, _vp] + [_c_int] * 4 + [_vp],
     "dca_tap_gather3d": [_vp, _vp] + [_c_int] * 4 + [_vp],
-    "dca_tap_gather_class_stats": [_vp, _vp, _vp, _vp, _vp, _vp] + [_c_int] * 4 + [_vp],
     "dca_conv2d_tc": [_vp, _c_int, _vp, _vp, _vp, _vp, _c_int, _c_int] + [_c_int] * 5 + [_vp],
     "dca_conv2d_tc_ex": [_vp, _c_int, _vp, _vp, _vp, _vp, _c_int, _vp, _c_int, _c_int] + [_c_int] * 6 + [_vp],
     "dca_conv2d_stem": [_vp, _vp, _vp, _vp, _vp, _c_int, _c_int] + [_c_int] * 4 + [_vp],

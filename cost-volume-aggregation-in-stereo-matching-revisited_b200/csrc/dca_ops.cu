@@ -1240,83 +1240,6 @@ conv2d_stem_kernel(const float* __restrict__ x, const float* __restrict__ w, con
   }
 }
 
-// cva.classify.2 + SemanticLevelContext statistics in one kernel: logits = 27-tap shifted sum of P (exactly as
-// tap_gather3d_kernel: same loads, same summation order), written to HBM (they are an output of the stage) AND kept in shared
-// memory, where one warp per block runs the per-pixel class statistics of class_stats_kernel (same formulas) on them.
-// Saves the class-stats launch and its re-read of the logits -- but measured SLOWER than the two kernels (35 us at KITTI 1/8
-// res: the gather phase runs worse in these 768-thread blocks), so the engine keeps the two launches; kept as an entry point.
-// Block = 32 w-columns x GC_DG disparity groups of one image row.
-constexpr int GC_DG = 24;
-__global__ void __launch_bounds__(32 * GC_DG)
-tap_gather_class_stats_kernel(const float* __restrict__ P, float* __restrict__ logits_out, int* __restrict__ cls,
-                              float* __restrict__ e_out, float* __restrict__ S, unsigned long long* __restrict__ acc, int B,
-                              int D, int H, int W) {
-  extern __shared__ float gc_log[];                 // [D][33]
-  __shared__ int s_last;
-  const int lane = threadIdx.x & 31, g = threadIdx.x >> 5;
-  const int w = blockIdx.x * 32 + lane, h = blockIdx.y, b = blockIdx.z;
-  const size_t nvox = (size_t)B * D * H * W;
-  const int HW = H * W;
-  pdl_wait();
-  if (w < W) {
-    float ok9[9];
-    int off9[9];
-#pragma unroll
-    for (int kh = 0; kh < 3; ++kh)
-#pragma unroll
-      for (int kw = 0; kw < 3; ++kw) {
-        const bool ok = (h + kh - 1 >= 0) && (h + kh - 1 < H) && (w + kw - 1 >= 0) && (w + kw - 1 < W);
-        ok9[kh * 3 + kw] = ok ? 1.f : 0.f;
-        off9[kh * 3 + kw] = ok ? (kh - 1) * W + (kw - 1) : 0;
-      }
-    for (int d = g; d < D; d += GC_DG) {
-      const size_t v = (((size_t)b * D + d) * H + h) * W + w;
-      float val[27];
-#pragma unroll
-      for (int kd = 0; kd < 3; ++kd) {
-        const bool okd = (d + kd - 1 >= 0) && (d + kd - 1 < D);
-        const float* base = P + (size_t)(kd * 9) * nvox + v + (okd ? (long long)(kd - 1) * HW : 0ll);
-#pragma unroll
-        for (int t = 0; t < 9; ++t) val[kd * 9 + t] = __ldg(base + (size_t)t * nvox + off9[t]) * (okd ? ok9[t] : 0.f);
-      }
-      float logit = 0.f;
-#pragma unroll
-      for (int t = 0; t < 27; ++t) logit += val[t];
-      logits_out[v] = logit;
-      gc_log[d * 33 + lane] = logit;
-    }
-  }
-  __syncthreads();
-  if (g < CS_G) {                                   // the first CS_G warps: the block's 32 pixels x CS_G class groups
-    const bool valid = w < W;
-    int k = 0;
-    float e = 0.f;
-    pixel_class_stats<1>(*reinterpret_cast<CsSmem*>(gc_log + D * 33), lane, g, D, valid,
-                      [&](int d) { return gc_log[d * 33 + lane]; }, k, e);
-    if (g == 0) {
-      if (valid) {
-        const size_t pix = ((size_t)b * H + h) * W + w;
-        cls[pix] = k;
-        e_out[pix] = e;
-      }
-      warp_class_sums(acc + (size_t)b * D, lane, valid ? k : -1, valid ? __float2ull_rn(e * CS_FIX) : 0ull);
-      __threadfence();
-      if (lane == 0) {
-        const unsigned long long t = atomicAdd(&acc[(size_t)B * D], 1ull);
-        s_last = (t == (unsigned long long)gridDim.x * gridDim.y * gridDim.z - 1ull);
-      }
-    }
-  }
-  __syncthreads();
-  if (s_last) {
-    __threadfence();
-    for (int i = threadIdx.x; i < B * D; i += blockDim.x) {
-      const unsigned long long v = *reinterpret_cast<volatile unsigned long long*>(&acc[i]);
-      S[i] = (float)((double)v * (1.0 / 1099511627776.0));
-    }
-  }
-}
-
 static inline int grid_for(size_t total, int threads) {
   size_t g = (total + threads - 1) / threads;
   const size_t cap = (size_t)dca_num_sms() * 32;
@@ -1355,22 +1278,6 @@ extern "C" int dca_class_stats(const float* logits, int* cls, float* e, float* S
   const int HW = H * W;
   dca_launch(class_stats_kernel, dim3((HW + 31) / 32, B), CS_THREADS, 0, st, logits, cls, e, S,
              (unsigned long long*)scratch, D, HW, B * D);
-  DCA_RETURN_IF_LAUNCH_FAILED();
-  return DCA_OK;
-}
-
-// P fp32 tap-major [27][B*D*H*W] -> logits [B,D,H,W] (27-tap shifted sum) AND the class statistics of dca_class_stats on them
-// (cls, e, S; scratch as there): cva.classify.2 (cva.py:53) + semantic_level.py:98-116 in one launch.  Bit-identical to
-// dca_tap_gather3d followed by dca_class_stats.
-extern "C" int dca_tap_gather_class_stats(const float* P, float* logits, int* cls, float* e, float* S, void* scratch, int B,
-                                          int D, int H, int W, void* stream) {
-  if (!P || !logits || !cls || !e || !S || !scratch || ((uintptr_t)scratch & 7) || B <= 0 || D <= 0 || D > CS_MAXD || H <= 0 ||
-      W <= 0 || H > 65535 || B > 65535)
-    return DCA_ERR_ARG;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (cudaMemsetAsync(scratch, 0, ((size_t)B * D + 1) * sizeof(unsigned long long), st) != cudaSuccess) return DCA_ERR_LAUNCH;
-  dca_launch(tap_gather_class_stats_kernel, dim3((W + 31) / 32, H, B), 32 * GC_DG,
-             (size_t)D * 33 * sizeof(float) + sizeof(CsSmem), st, P, logits, cls, e, S, (unsigned long long*)scratch, B, D, H, W);
   DCA_RETURN_IF_LAUNCH_FAILED();
   return DCA_OK;
 }

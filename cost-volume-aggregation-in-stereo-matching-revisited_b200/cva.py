@@ -22,7 +22,7 @@ class Multi_Aggregation(nn.Module):
         engine._require_cuda(x)
         P = self.precision_planes
         pk = engine.cached_pack(self, ("agg", P), lambda: engine.PackedAgg(self, P))
-        return engine.agg_forward(pk, engine.Planes.from_ncdhw(x, P)).to_ncdhw()
+        return engine._result(engine.agg_steps(pk, engine.Planes.from_ncdhw(x, P))).to_ncdhw()
 
 
 class cva(nn.Module):
@@ -52,6 +52,7 @@ class cva(nn.Module):
         pk = engine.cached_pack(self, ("cva", self.precision_planes),
                                 lambda: engine.PackedCva(self, self.precision_planes))
         keep = {}
-        logits, out = engine.cva_forward(pk, engine.Planes.from_ncdhw(cost_volume, self.precision_planes), keep=keep)
+        cost = engine.Planes.from_ncdhw(cost_volume, self.precision_planes)
+        logits, out = engine._result(engine.cva_steps(pk, cost, keep=keep))
         self.last = keep
         return logits.unsqueeze(1), out.to_ncdhw()

@@ -6,11 +6,16 @@ cuDNN/cuBLAS, no CPU fallback.
 
 Data layout in HBM ("cost planes"): channels-last 16-bit `[planes][B][D][H][W][C]` (fp16 by default, see plane_dtype());
 planes=2 ("parity": hi + lo, 22-bit significand) or planes=1 ("fast": a single 16-bit plane).
+
+The forward is written once, as generators (`hot_path_steps`, `cva_steps`, `agg_steps`): unsharded they yield nothing
+and `_result` runs them to the end; with `sharded=True` they run on one rank's row slab and yield the `Rows` / `Sum`
+requests that hshard.py's drivers fulfil.
 """
 from __future__ import annotations
 
 import collections
 import os
+from dataclasses import dataclass
 
 import torch
 
@@ -149,9 +154,6 @@ class Options:
     fp32_stages = frozenset()     # diagnostics: stages whose convs run on the fp32 CUDA-core kernel: {'dres', 'cva', 'cls3'}
     use_up2 = True                # class-wise halo-slab kernel for the transposed conv and the trilinear fuse stage
     fuse_tail = True              # conv(32ch)+BN+ReLU -> Conv3d(32->1): per-tap products from the first conv's epilogue
-    fuse_gather_stats = False     # the shifted sum + class statistics of a cva stage as ONE kernel (dca_tap_gather_class_stats):
-                                  # bit-identical, but measured SLOWER (35 us vs 9.3 us + the class-stats kernel under ncu at
-                                  # KITTI: the gather runs worse in 768-thread blocks at one block per SM)
 
 
 def conv(x: Planes, pc: PackedConv, mode=K3S1, act=ACT_NONE, res_pre: Planes = None, res_post: Planes = None,
@@ -420,21 +422,6 @@ def tap_gather(P):
     return y
 
 
-def tap_gather_class_stats(P):
-    """P [27,B,D,H,W] -> (logits [B,D,H,W], cls [B,H,W] int32, e [B,H,W], S [B,D]): the shifted sum of the 32 -> 1 conv and the
-    class statistics on its result in one launch."""
-    _, B, D, H, W = P.shape
-    dev = P.device
-    logits = torch.empty((B, D, H, W), dtype=torch.float32, device=dev)
-    cls = torch.empty((B, H, W), dtype=torch.int32, device=dev)
-    e = torch.empty((B, H, W), dtype=torch.float32, device=dev)
-    S = torch.empty((B, D), dtype=torch.float32, device=dev)
-    scratch = torch.empty(B * D + 1, dtype=torch.int64, device=dev)
-    _lib.call("dca_tap_gather_class_stats", P.data_ptr(), logits.data_ptr(), cls.data_ptr(), e.data_ptr(), S.data_ptr(),
-              scratch.data_ptr(), B, D, H, W, _stream())
-    return logits, cls, e, S
-
-
 def tap_gather_softmax_regress(P, want_logits=False):
     """P [27,B,D,H,W] -> (pred [B,1,H,W], logits [B,D,H,W] or None): shifted sum + softmax + regression in one kernel."""
     _, B, D, H, W = P.shape
@@ -618,6 +605,47 @@ def _f32c(t):
 
 
 # --------------------------------------------------------------------------------------------
+# requests of the H-sharded sequence (fulfilled by the drivers in hshard.py)
+# --------------------------------------------------------------------------------------------
+H4_HALO = 2      # halo rows at 1/4 resolution (even: keeps the stride-2 alignment)
+H8_HALO = 1      # halo rows at 1/8 resolution
+H4_LIVE = 1      # 1/4-res halo rows that are ever read for an owned output (the outer one only keeps the alignment)
+
+
+@dataclass
+class Rows:
+    """Refresh the `h` halo rows at both ends of `dim` of `t` (owned rows = [h, n-h)).  Interior side: the neighbour's
+    owned rows next to the cut (only if `exchange`).  Image border: `fill` = "zero" | "replicate" | "keep" (all h rows).
+    `live`: only that many halo rows, the ones next to the owned rows, are read by any op that produces OWNED output
+    (the outer 1/4-res halo row exists for the stride-2 alignment only), so only they travel."""
+    t: torch.Tensor
+    dim: int
+    h: int
+    fill: str = "zero"
+    exchange: bool = True
+    live: int = 0         # rows (next to the owned ones) that actually travel; 0 = all h
+
+    @property
+    def nlive(self):
+        return self.live or self.h
+
+
+@dataclass
+class Sum:
+    """All-reduce (sum) `t` in place over the ranks."""
+    t: torch.Tensor
+
+
+def _result(steps):
+    """Run an unsharded sequence generator (it yields no request) and return its result."""
+    try:
+        next(steps)
+    except StopIteration as stop:
+        return stop.value
+    raise _lib.DcaError("an unsharded sequence yielded a halo request")
+
+
+# --------------------------------------------------------------------------------------------
 # packed parameter sets for the composite blocks
 # --------------------------------------------------------------------------------------------
 class PackedAttention:
@@ -698,10 +726,15 @@ class PackedAgg:
         self.conv3_fused = _pack_deconv_with_redir(agg, self.conv3, self.redir, planes) if c == 32 else None
 
 
-def agg_forward(pk: PackedAgg, x: Planes, res_post: Planes = None, keep=None):
-    """Multi_Aggregation.forward (cva.py:26-31): ReLU(BN(conv3(conv2(conv1 x))) + BN(redir x)) (+ res_post)."""
+def agg_steps(pk: PackedAgg, x: Planes, res_post: Planes = None, keep=None, sharded=False):
+    """Multi_Aggregation.forward (cva.py:26-31): ReLU(BN(conv3(conv2(conv1 x))) + BN(redir x)) (+ res_post).  Generator;
+    the result comes back through StopIteration."""
     c1 = conv(x, pk.conv1, K3S2, ACT_RELU)
+    if sharded:
+        yield Rows(c1.t, 3, H8_HALO)
     c2 = conv(c1, pk.conv2, K3S1, ACT_RELU)
+    if sharded:
+        yield Rows(c2.t, 3, H8_HALO)
     fd = pk.conv3_fused
     if Options.use_tc and Options.use_up2 and fd is not None and fd.tc_planes == c2.planes:
         out = up2(0, c2, x, fd.w_tc, fd.scale, fd.shift, ACT_RELU, 64, c2.D, c2.H, c2.W, res_post=res_post)
@@ -714,8 +747,12 @@ def agg_forward(pk: PackedAgg, x: Planes, res_post: Planes = None, keep=None):
                   res_post.planes if res_post is not None else 1, 0, 1, x.ptr, x.C, out.ptr, c2.planes,
                   ACT_RELU, c2.B, 64, 32, c2.D, c2.H, c2.W, out.D, out.H, out.W, _stream())
     else:
+        # also taken when the fused deconv + redir pack was declined (a tiny BN gamma of conv3, _pack_deconv_with_redir):
+        # redir is per voxel, so valid halo rows stay valid
         redir = conv(x, pk.redir, K1, ACT_NONE)
         out = conv(c2, pk.conv3, T3S2, ACT_RELU, res_pre=redir, res_post=res_post)
+    if sharded:
+        yield Rows(out.t, 3, H4_HALO, live=H4_LIVE)
     if keep is not None:
         keep.update(c1=c1, c2=c2)
     return out
@@ -753,23 +790,38 @@ def _pack_deconv_with_redir(agg, pc3, pcr, planes):
     return _FusedDeconv(buf, pc3.scale, (pc3.shift + pcr.shift).contiguous(), planes)
 
 
-def cva_forward(pk: PackedCva, cost: Planes, res_post: Planes = None, keep=None):
-    """cva.forward(downsample=True): returns (logits fp32 [B,D8,H8,W8], augmented cost Planes)."""
+def cva_steps(pk: PackedCva, cost: Planes, res_post: Planes = None, keep=None, sharded=False):
+    """cva.forward(downsample=True) (cva.py:59-72).  Generator; returns (logits fp32 [B,D8,H8,W8], augmented cost Planes)
+    through StopIteration.  Sharded, `cost` arrives with refreshed halo rows and `out` leaves with them."""
     pooled = avgpool(cost)
+    if sharded:
+        yield Rows(pooled.t, 3, H8_HALO)
     cost_down = conv(pooled, pk.down, K3S1, ACT_RELU)
+    if sharded:
+        yield Rows(cost_down.t, 3, H8_HALO)
     P27 = conv_taps27(cost_down, pk.cls0, pk.cls2)
-    if P27 is not None and Options.fuse_gather_stats:
-        logits, cls, e, S = tap_gather_class_stats(P27)
+    if P27 is not None:
+        if sharded:        # the per-tap products are a per-voxel function of the conv's output rows
+            yield Rows(P27, 3, H8_HALO)
+        logits = tap_gather(P27)
     else:
-        if P27 is not None:
-            logits = tap_gather(P27)
-        else:
-            h = conv(cost_down, pk.cls0, K3S1, ACT_RELU)
-            logits = conv_cout1_any(h, pk.cls2)
-        cls, e, S = class_stats(logits)
+        h = conv(cost_down, pk.cls0, K3S1, ACT_RELU)
+        if sharded:
+            yield Rows(h.t, 3, H8_HALO)
+        logits = conv_cout1_any(h, pk.cls2)
+    if sharded:
+        yield Rows(logits, 2, H8_HALO)
+    cls, e, S = class_stats(logits)
+    if sharded:            # S[b,k] over the OWNED pixels, summed over the ranks = over the image
+        _, _, S = class_stats(logits[:, :, H8_HALO:logits.shape[2] - H8_HALO].contiguous())
+        yield Sum(S)
     use_up2 = Options.use_tc and Options.use_up2 and pk.attn.has_wa
     bil = use_up2 and Options.up2_bilinear
     t = disp_attention(cost_down, cls, e, S, pk.attn.buf, pk.attn.has_wa, pad=(2 if bil else (1 if use_up2 else 0)))
+    if sharded:
+        # t: [2*D8][Hb8+2][W8+2], replicated 1-voxel border in h/w.  Interior cuts need nothing (the halo row is a valid
+        # per-pixel result); at the image border the clamp of the trilinear must start at the border row, not outside it.
+        yield Rows(t.t, 3, H8_HALO + 1, fill="replicate", exchange=False)
     if bil:
         # depth axis of the trilinear already resolved by the attention kernel's store; 4-class bilinear GEMM here
         fused = up2(2, t, cost, pk.fuse_up2b_w, pk.fuse_scale, pk.fuse_shift, ACT_NONE, 32, cost.D, cost_down.H,
@@ -783,7 +835,9 @@ def cva_forward(pk: PackedCva, cost: Planes, res_post: Planes = None, keep=None)
         fused = conv(cost, pk.fuse_c, K1, ACT_NONE, up=t)
     else:
         fused = upsample_fuse(t, cost, pk.fuse_wcT, pk.fuse_scale, pk.fuse_shift)
-    out = agg_forward(pk.agg, fused, res_post=res_post)
+    if sharded:
+        yield Rows(fused.t, 3, H4_HALO, live=H4_LIVE)
+    out = yield from agg_steps(pk.agg, fused, res_post=res_post, sharded=sharded)
     if keep is not None:
         keep.update(pooled=pooled, cost_down=cost_down, logits=logits, class_map=cls, e=e, S=S, t=t, fused=fused, out=out)
     return logits, out
@@ -816,11 +870,14 @@ class PackedHotPath:
 _SIDE_STREAMS = {}
 
 
-def _prop_mask(pk, g, P):
-    """PropgationNet_4x.conv on the guidance features (gwcnet_dca_g.py:112-115,119): fp32 channels-last mask logits."""
+def _prop_mask_steps(pk, g, P, sharded=False):
+    """PropgationNet_4x.conv on the guidance features (gwcnet_dca_g.py:112-115,119): fp32 channels-last mask logits.
+    Generator; the mask comes back through StopIteration."""
     gp = Planes.from_ncdhw(g, planes=P)
     if Options.use_tc and Options.prop_on_tc:
         m1 = conv2d_tc(gp, pk.prop0_tc, ACT_RELU)
+        if sharded:
+            yield Rows(m1.t, 3, H4_HALO, live=H4_LIVE)
         return conv2d_tc(m1, pk.prop2_tc, ACT_NONE, out_fp32=True)
     m1 = conv(gp, pk.prop0, C2D3, ACT_RELU)
     return conv(m1, pk.prop2, C2D3, ACT_NONE, out_fp32=True)
@@ -829,8 +886,6 @@ def _prop_mask(pk, g, P):
 def _prop_mask_start(pk, g, P):
     """The mask branch only depends on the guidance features, so it is issued on a second stream at the start of the
     forward: its 5 short launches (234 tiles each) fill SMs that the cost-volume kernels leave idle at their tails."""
-    if not Options.prop_side_stream:
-        return (None, pk, g, P)
     main = torch.cuda.current_stream()
     dev = (g.device.index, main.cuda_stream)   # one side stream AND one buffer set per calling stream: forwards issued
     side = _SIDE_STREAMS.get(dev)              # concurrently on several streams must not share the mask buffers
@@ -858,14 +913,11 @@ def _prop_mask_start(pk, g, P):
             conv2d_tc(gp, pk.prop0_tc, ACT_RELU, out=m1)
             conv2d_tc(m1, pk.prop2_tc, ACT_NONE, out_fp32=True, out=mask)
         else:
-            mask = _prop_mask(pk, g, P)
+            mask = _result(_prop_mask_steps(pk, g, P))
     return (side, mask, main, bufs)
 
 
 def _prop_mask_wait(job):
-    if job[0] is None:
-        _, pk, g, P = job
-        return _prop_mask(pk, g, P)
     side, mask, main, bufs = job
     main.wait_stream(side)
     if bufs is None and not torch.cuda.is_current_stream_capturing():
@@ -898,29 +950,43 @@ def hot_path_forward(pk: PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g, keep=None
     pred4 and prob_volume2 unchanged bit for bit)."""
     _require_cuda(gwc_l, gwc_r, cat_l, cat_r, g)
     check_feature_shapes(pk, gwc_l, gwc_r, cat_l, cat_r, g)
-    P = pk.planes
-    D4 = pk.maxdisp // 4
-    side_job = _prop_mask_start(pk, _f32c(g), P)
-    vol = fused_volume(_f32c(gwc_l), _f32c(gwc_r), _f32c(cat_l) if cat_l is not None else None,
-                       _f32c(cat_r) if cat_r is not None else None, D4, pk.num_groups, P)
     tc0 = Options.use_tc
     try:
-        return _hot_path_stages(pk, vol, side_job, tc0, keep, confidence)
+        return _result(hot_path_steps(pk, gwc_l, gwc_r, cat_l, cat_r, g, keep, confidence))
     finally:
         Options.use_tc = tc0          # fp32_stages (diagnostics) toggles it per stage; never leak that into later calls
 
 
-def _hot_path_stages(pk, vol, side_job, tc0, keep, confidence=False):
+def hot_path_steps(pk: PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g, keep=None, confidence=False, sharded=False):
+    """The launches of `hot_path_forward`, as a generator returning its result through StopIteration.  Sharded, the
+    feature maps are one rank's row slab with H4_HALO refreshed halo rows per side (hshard.py), a `Rows` request follows
+    every layer whose halo rows need a refresh and a `Sum` request the per-class sums S[b,k]; the results keep their
+    halo rows.  Unsharded, nothing is yielded."""
+    P = pk.planes
+    D4 = pk.maxdisp // 4
+    g = _f32c(g)
+    side_job = _prop_mask_start(pk, g, P) if Options.prop_side_stream and not sharded else None
+    vol = fused_volume(_f32c(gwc_l), _f32c(gwc_r), _f32c(cat_l) if cat_l is not None else None,
+                       _f32c(cat_r) if cat_r is not None else None, D4, pk.num_groups, P)
+    tc0 = Options.use_tc
     Options.use_tc = tc0 and "dres" not in Options.fp32_stages
     c = conv(vol, pk.dres0_0, K3S1, ACT_RELU)
+    if sharded:
+        yield Rows(c.t, 3, H4_HALO, live=H4_LIVE)
     c = conv(c, pk.dres0_2, K3S1, ACT_RELU)
+    if sharded:
+        yield Rows(c.t, 3, H4_HALO, live=H4_LIVE)
     r = conv(c, pk.dres1_0, K3S1, ACT_RELU)
+    if sharded:
+        yield Rows(r.t, 3, H4_HALO, live=H4_LIVE)
     cost0 = conv(r, pk.dres1_2, K3S1, ACT_NONE, res_post=c)
+    if sharded:
+        yield Rows(cost0.t, 3, H4_HALO, live=H4_LIVE)
     Options.use_tc = tc0 and "cva" not in Options.fp32_stages
     kept = [{} if keep is not None else None for _ in pk.cva]
     cur, out1, logits2 = cost0, None, None
     for i, stage in enumerate(pk.cva):      # cva1 adds cost0 back (gwcnet_dca_g.py:229), the others chain
-        lg, cur = cva_forward(stage, cur, res_post=cost0 if i == 0 else None, keep=kept[i])
+        lg, cur = yield from cva_steps(stage, cur, res_post=cost0 if i == 0 else None, keep=kept[i], sharded=sharded)
         if i == 0:
             out1 = cur
         if i + 1 == pk.pv_stage:
@@ -928,15 +994,26 @@ def _hot_path_stages(pk, vol, side_job, tc0, keep, confidence=False):
     Options.use_tc = tc0 and "cls3" not in Options.fp32_stages
     P27 = conv_taps27(cur, pk.cls3_0, pk.cls3_2)
     if P27 is not None:
+        if sharded:
+            yield Rows(P27, 3, H4_HALO, live=H4_LIVE)
         # the head's logits are only an OUTPUT when there is no cva stage (gwcnet_dca0_g.py:190), when a caller keeps them
         # or when the confidence is wanted
         pred_q, logits = tap_gather_softmax_regress(P27, want_logits=(not pk.cva) or keep is not None or confidence)
     else:
         h = conv(cur, pk.cls3_0, K3S1, ACT_RELU)
+        if sharded:         # only one halo row of h is live: the logits are valid on the owned rows
+            yield Rows(h.t, 3, H4_HALO, live=H4_LIVE)
         logits = conv_cout1_any(h, pk.cls3_2)
         pred_q = softmax_regress(logits)
     Options.use_tc = tc0
-    mask = _prop_mask_wait(side_job)
+    if side_job is not None:
+        mask = _prop_mask_wait(side_job)
+    else:
+        mask = yield from _prop_mask_steps(pk, g, P, sharded)
+    if sharded:
+        # the convex upsampling reads the 3x3 neighbourhood of the regressed disparity: one row from each neighbour, and
+        # zero DISPARITY outside the image (F.unfold(padding=1) of the reference)
+        yield Rows(pred_q, 2, H4_HALO, fill="zero", live=H4_LIVE)
     pred4 = convex_upsample(mask, pred_q)
     if confidence:
         conf, peak_q, std_q = softmax_confidence_upsample(logits, mask, quarter=keep is not None)

@@ -4,8 +4,9 @@ layer that looks at neighbouring rows and one [B, D/8] sum all-reduce per cva st
 
 STATUS: host logic and exchange plan are covered on CPU (tests/test_hshard_plan.py: the drivers below run the same
 plan over the CPU checker's ATen ops, in-process with 2/3/4 virtual ranks and over gloo with world_size 2, against
-the un-sharded CPU result).  The kernel sequence `hot_path_steps` is covered on the GPU by tests/test_gpu_hshard.py
-(virtual ranks on one device, and one process per GPU over both transports when >= 2 GPUs are visible).
+the un-sharded CPU result; tests/test_host_sequence.py: the launches and requests of a rank, by a dry run).  The kernel
+sequence `hot_path_steps` is covered on the GPU by tests/test_gpu_hshard.py (virtual ranks on one device, and one
+process per GPU over both transports when >= 2 GPUs are visible).
 
 Frame of one rank.  The rank owns the 1/4-res rows [r0, r1) (both even, so its 1/8-res rows [r0/2, r1/2) align).
 Every local tensor carries halo rows: 2 at 1/4 res (buffer = global rows [r0-2, r1+2)), 1 at 1/8 res (global rows
@@ -20,24 +21,24 @@ Per-pixel ops (1x1x1 convs, attention over the disparity axis, softmax + regress
 The only quantity that spans the image is S[b,k] = sum over the pixels of class k of exp(P) (`semantic_level.py:112-116`):
 each rank sums its OWNED rows and the [B, D/8] vectors are all-reduced.
 
-The sequence is written as a generator that yields `Rows` / `Sum` requests, so the same code runs under
-`drive_distributed` (one process per GPU, torch.distributed) and `drive_lockstep` (N virtual ranks in one process,
-for single-device verification).
+The layer sequence is the single-GPU one: `engine.hot_path_steps(..., sharded=True)` yields a `Rows` request after
+every layer whose halo rows need a refresh and a `Sum` request for S[b,k].  This module keeps what is specific to
+slabs: the row partition, the padding and exchange of the five feature maps, the crop of the results to the owned rows,
+and the drivers that fulfil the requests -- `drive_distributed` (one process per GPU, torch.distributed) and
+`drive_lockstep` (N virtual ranks in one process, for single-device verification).  Every rank issues the same
+sequence of requests, so the exchanges stay in lockstep.
 """
 from __future__ import annotations
 
 import os
-from dataclasses import dataclass
 
 import torch
 
 from . import _lib
 from . import engine as E
+from .engine import H4_HALO, H4_LIVE, H8_HALO, Rows, Sum
 
 FUSED_EXCHANGE = os.environ.get("DCA_HALO_FUSED", "1") != "0"   # one launch per exchange instead of push + wait/unpack
-H4_HALO = 2      # halo rows at 1/4 resolution (even: keeps the stride-2 alignment)
-H8_HALO = 1      # halo rows at 1/8 resolution
-H4_LIVE = 1      # 1/4-res halo rows that are ever read for an owned output (the outer one only keeps the alignment)
 
 
 # --------------------------------------------------------------------------------------------
@@ -69,32 +70,8 @@ def owned_rows(t, world, rank, dim=2, scale=1):
 
 
 # --------------------------------------------------------------------------------------------
-# exchange requests and their drivers
+# drivers of the exchange requests (engine.Rows / engine.Sum)
 # --------------------------------------------------------------------------------------------
-@dataclass
-class Rows:
-    """Refresh the `h` halo rows at both ends of `dim` of `t` (owned rows = [h, n-h)).  Interior side: the neighbour's
-    owned rows next to the cut (only if `exchange`).  Image border: `fill` = "zero" | "replicate" | "keep" (all h rows).
-    `live`: only that many halo rows, the ones next to the owned rows, are read by any op that produces OWNED output
-    (the outer 1/4-res halo row exists for the stride-2 alignment only), so only they travel."""
-    t: torch.Tensor
-    dim: int
-    h: int
-    fill: str = "zero"
-    exchange: bool = True
-    live: int = 0         # rows (next to the owned ones) that actually travel; 0 = all h
-
-    @property
-    def nlive(self):
-        return self.live or self.h
-
-
-@dataclass
-class Sum:
-    """All-reduce (sum) `t` in place over the ranks."""
-    t: torch.Tensor
-
-
 def _fill_border(req: Rows, top: bool):
     t, d, h = req.t, req.dim, req.h
     n = t.shape[d]
@@ -313,49 +290,6 @@ def _require_default_route(pk):
             raise _lib.DcaError("the H-sharded mode needs the fuse conv folded into the attention pack")
 
 
-def _cva_steps(pk, cost, res_post=None):
-    """cva.forward (`cva.py:59-72`) on a slab; `cost` arrives with refreshed halos.  Returns (logits, out) through
-    StopIteration; `out` leaves with refreshed halos."""
-    pooled = E.avgpool(cost)
-    yield Rows(pooled.t, 3, H8_HALO)
-    cost_down = E.conv(pooled, pk.down, E.K3S1, E.ACT_RELU)
-    yield Rows(cost_down.t, 3, H8_HALO)
-    P27 = E.conv_taps27(cost_down, pk.cls0, pk.cls2)           # fused tail: per-tap products [27, B, D8, Hb8, W8]
-    if P27 is not None:
-        yield Rows(P27, 3, H8_HALO)                            # (they are a per-voxel function of the conv's output rows)
-        logits = E.tap_gather(P27)                             # fp32 [B, D8, Hb8, W8]
-    else:
-        h = E.conv(cost_down, pk.cls0, E.K3S1, E.ACT_RELU)
-        yield Rows(h.t, 3, H8_HALO)
-        logits = E.conv_cout1_any(h, pk.cls2)
-    yield Rows(logits, 2, H8_HALO)
-    cls, e, _ = E.class_stats(logits)                           # per pixel, halo rows included
-    own = logits[:, :, H8_HALO:logits.shape[2] - H8_HALO].contiguous()
-    _, _, S = E.class_stats(own)                                # S[b,k] over the OWNED pixels ...
-    yield Sum(S)                                                # ... summed over the ranks = over the image
-    t = E.disp_attention(cost_down, cls, e, S, pk.attn.buf, pk.attn.has_wa, pad=2)
-    # t: [2*D8][Hb8+2][W8+2], replicated 1-voxel border in h/w.  Interior cuts need nothing (the halo row is a valid
-    # per-pixel result); at the image border the clamp of the trilinear must start at the border row, not outside it.
-    yield Rows(t.t, 3, H8_HALO + 1, fill="replicate", exchange=False)
-    fused = E.up2(2, t, cost, pk.fuse_up2b_w, pk.fuse_scale, pk.fuse_shift, E.ACT_NONE, 32, cost.D, cost_down.H,
-                  cost_down.W)
-    yield Rows(fused.t, 3, H4_HALO, live=H4_LIVE)
-    c1 = E.conv(fused, pk.conv1, E.K3S2, E.ACT_RELU)
-    yield Rows(c1.t, 3, H8_HALO)
-    c2 = E.conv(c1, pk.conv2, E.K3S1, E.ACT_RELU)
-    yield Rows(c2.t, 3, H8_HALO)
-    fd = pk.conv3_fused
-    if fd is not None and fd.tc_planes == c2.planes:
-        out = E.up2(0, c2, fused, fd.w_tc, fd.scale, fd.shift, E.ACT_RELU, 64, c2.D, c2.H, c2.W, res_post=res_post)
-    else:
-        # the fused deconv + redir pack was declined (a tiny BN gamma of conv3, engine._pack_deconv_with_redir): redir as
-        # its own 1x1x1 conv (per voxel: valid halos stay valid), added before the ReLU of the transposed conv
-        redir = E.conv(fused, pk.redir, E.K1, E.ACT_NONE)
-        out = E.conv(c2, pk.conv3, E.T3S2, E.ACT_RELU, res_pre=redir, res_post=res_post)
-    yield Rows(out.t, 3, H4_HALO, live=H4_LIVE)
-    return logits, out
-
-
 def hot_path_steps(pk: E.PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g):
     """GwcNet.forward (eval, `gwcnet_dca_g.py:216-240,282`) for the rows this rank owns.  Inputs: the rank's OWNED rows
     of the fp32 feature maps [B,C,Hl,W4].  Result: (pred4 [B,1,4*Hl,4*W4], prob_volume2 [B,D8,Hl/2,W8])."""
@@ -364,7 +298,6 @@ def hot_path_steps(pk: E.PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g):
     E.check_feature_shapes(pk, gwc_l, gwc_r, cat_l, cat_r, g)
     if gwc_l.shape[2] % 2 or gwc_l.shape[2] < 4:
         raise _lib.DcaError("a rank must own an even number (>= 4) of 1/4-resolution rows")
-    P, D4 = pk.planes, pk.maxdisp // 4
     feats = []
     for f in (gwc_l, gwc_r, cat_l, cat_r, g):
         if f is None:
@@ -373,46 +306,10 @@ def hot_path_steps(pk: E.PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g):
         fp = _pad_rows(E._f32c(f), H4_HALO)
         yield Rows(fp, 2, H4_HALO, live=H4_LIVE)
         feats.append(fp)
-    gl, gr, cl, cr, gd = feats
-    # guidance/mask branch of PropgationNet_4x (`gwcnet_dca_g.py:112-115,119`); main stream in this mode
-    gp = E.Planes.from_ncdhw(gd, planes=P)
-    m1 = E.conv2d_tc(gp, pk.prop0_tc, E.ACT_RELU)
-    yield Rows(m1.t, 3, H4_HALO, live=H4_LIVE)
-    mask = E.conv2d_tc(m1, pk.prop2_tc, E.ACT_NONE, out_fp32=True)          # per-pixel use from here on
-    vol = E.fused_volume(gl, gr, cl, cr, D4, pk.num_groups, P)               # row-local; zero rows give a zero volume
-    c = E.conv(vol, pk.dres0_0, E.K3S1, E.ACT_RELU)
-    yield Rows(c.t, 3, H4_HALO, live=H4_LIVE)
-    c = E.conv(c, pk.dres0_2, E.K3S1, E.ACT_RELU)
-    yield Rows(c.t, 3, H4_HALO, live=H4_LIVE)
-    r = E.conv(c, pk.dres1_0, E.K3S1, E.ACT_RELU)
-    yield Rows(r.t, 3, H4_HALO, live=H4_LIVE)
-    cost0 = E.conv(r, pk.dres1_2, E.K3S1, E.ACT_NONE, res_post=c)
-    yield Rows(cost0.t, 3, H4_HALO, live=H4_LIVE)
-    cur, logits2 = cost0, None
-    for i, stage in enumerate(pk.cva):
-        lg, cur = yield from _cva_steps(stage, cur, res_post=cost0 if i == 0 else None)
-        if i + 1 == pk.pv_stage:
-            logits2 = lg
-    P27 = E.conv_taps27(cur, pk.cls3_0, pk.cls3_2)
-    if P27 is not None:
-        yield Rows(P27, 3, H4_HALO, live=H4_LIVE)
-        pred_q, logits = E.tap_gather_softmax_regress(P27, want_logits=not pk.cva)     # [B,1,Hb4,W4]
-    else:
-        h = E.conv(cur, pk.cls3_0, E.K3S1, E.ACT_RELU)
-        yield Rows(h.t, 3, H4_HALO, live=H4_LIVE)
-        logits = E.conv_cout1_any(h, pk.cls3_2)           # valid on the owned rows (only one halo row of h is live)
-        pred_q = E.softmax_regress(logits)                # [B,1,Hb4,W4]
-    # the convex upsampling reads the 3x3 neighbourhood of the regressed disparity: one row from each neighbour, and
-    # zero DISPARITY outside the image (F.unfold(padding=1) of the reference)
-    yield Rows(pred_q, 2, H4_HALO, fill="zero", live=H4_LIVE)
-    pred4 = E.convex_upsample(mask, pred_q)
-    Hb4 = pred_q.shape[2]
-    pred4 = pred4[:, :, 4 * H4_HALO:4 * (Hb4 - H4_HALO)].contiguous()
-    if logits2 is None:                                   # no cva stage: the head's own 1/4-res logits
-        pv2 = logits[:, :, H4_HALO:Hb4 - H4_HALO].contiguous()
-    else:
-        pv2 = logits2[:, :, H8_HALO:logits2.shape[2] - H8_HALO].contiguous()
-    return pred4, pv2
+    pred4, pv = yield from E.hot_path_steps(pk, *feats, sharded=True)
+    pred4 = pred4[:, :, 4 * H4_HALO:pred4.shape[2] - 4 * H4_HALO].contiguous()
+    h = H8_HALO if pk.cva else H4_HALO       # no cva stage: prob_volume2 is the head's own 1/4-res logits
+    return pred4, pv[:, :, h:pv.shape[2] - h].contiguous()
 
 
 _PEERS = {}

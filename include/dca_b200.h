@@ -102,11 +102,6 @@ int dca_tap_gather3d(const float* P, float* out, int B, int D, int H, int W, voi
  * pack; 0: halo-slab kernel, w = dca_pack_weights_tc pack.  w27_host is a HOST pointer ([27][32] fp32, launch params). */
 int dca_conv3d_tc_taps27(const void* x, int planes, const void* w, int use_march, const float* scale, const float* shift,
                          const float* w27_host, float* P, int act, int B, int Cin, int D, int H, int W, void* stream);
-/* cva.classify.2 (cva.py:53) + the per-pixel class statistics of SemanticLevelContext (semantic_level.py:98-116) in one
- * launch: logits [B,D,H,W] = 27-tap shifted sum of P, and cls / e / S as dca_class_stats computes them from those logits
- * (scratch as there).  Bit-identical to dca_tap_gather3d followed by dca_class_stats. */
-int dca_tap_gather_class_stats(const float* P, float* logits, int* cls, float* e, float* S, void* scratch, int B, int D,
-                               int H, int W, void* stream);
 /* Fused tail, second half: logits = 27-tap shifted sum of P, softmax over D, disparity regression
  * (gwcnet_dca_g.py:235-239, submodule.py:127-131): pred [B,H,W]; logits_out optional [B,D,H,W].  Neither the logits nor
  * the probability volume are materialised. */

@@ -166,7 +166,7 @@ def test_run_convbn_3d(cin, cout, k, s):
                                                  (1, 6, 40, 30, True)])
 def test_up2_kind0_transposed_conv_plus_redir(B, Dl, Hl, Wl, with_res, pair):
     """dca_up2_tc kind 0 = ReLU(BN(ConvTranspose3d(x)) + BN(redir(side))) + res_post (cva.py:20-31), the kernel
-    cva_forward ships, at shapes that are not multiples of the 8x16 tile."""
+    cva_steps ships, at shapes that are not multiples of the 8x16 tile."""
     d, E = _mods()
     m = _init(d.Multi_Aggregation(32), 12)
     x, side = rnd(B, 64, Dl, Hl, Wl, seed=1), rnd(B, 32, 2 * Dl, 2 * Hl, 2 * Wl, seed=2)

@@ -396,18 +396,3 @@ def test_convex_upsample_and_regression():
     close(got, ref, 1e-5, "convex")
     logits = rnd(2, 48, 6, 17, seed=18) * 4
     close(E.softmax_regress(logits.cuda()), O.disparity_regression(F.softmax(logits, 1), 48), 1e-5, "regress")
-
-
-@pytest.mark.parametrize("B,D,H,W", [(1, 24, 48, 156), (2, 6, 5, 37), (1, 30, 7, 64), (1, 48, 9, 33)])
-def test_tap_gather_class_stats_equals_its_two_parts(B, D, H, W):
-    """dca_tap_gather_class_stats (shifted sum of the 32 -> 1 conv + class statistics in one launch) against
-    dca_tap_gather3d followed by dca_class_stats: logits, class map, e and S bit for bit (odd sizes, D up to 48, ties)."""
-    d, E, O = _mods()
-    P = torch.randn(27, B, D, H, W, generator=torch.Generator().manual_seed(D + W)).cuda()
-    P[:, 0, 3, 2, 5] = P[:, 0, 1, 2, 5]                 # an exact tie between two disparity classes of one pixel
-    logits_ref = E.tap_gather(P)
-    cls_ref, e_ref, S_ref = E.class_stats(logits_ref)
-    for _ in range(3):
-        logits, cls, e, S = E.tap_gather_class_stats(P)
-        assert torch.equal(logits, logits_ref) and torch.equal(cls, cls_ref)
-        assert torch.equal(e, e_ref) and torch.equal(S, S_ref)

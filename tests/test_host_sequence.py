@@ -29,8 +29,8 @@ def test_default_forward_launches_the_recorded_kernel_sequence():
 
 def test_hsharded_forward_host_flow():
     """hshard.hot_path_steps with 3 virtual ranks: every rank launches the un-sharded sequence at its slab shape
-    (owned rows + 2 halo rows per side) plus one extra dca_class_stats per cva (S over the owned rows), and the
-    stitched outputs have the full-image shapes."""
+    (owned rows + 2 halo rows per side) plus one extra dca_class_stats per cva (S over the owned rows), the stitched
+    outputs have the full-image shapes, and a rank issues the recorded number of halo and sum requests."""
     import dcanet_b200 as d
     hs = d.hshard
     H4, W4, world = 24, 40, 3
@@ -45,15 +45,20 @@ def test_hsharded_forward_host_flow():
     assert pred4.shape == (1, 1, 4 * H4, 4 * W4) and pv.shape == (1, 6, H4 // 2, W4 // 2)
     # un-sharded forward on ONE slab shape (all three ranks own 8 rows -> 12-row buffers)
     slab, _ = _dryrun.forward_trace(d.GwcNet(48).eval(), 8 + 2 * hs.H4_HALO, W4)
-    want = collections.Counter()
-    for t in slab:        # the un-sharded forward gathers the taps and takes the class statistics in ONE launch; a slab needs
-        if t[0] == "dca_tap_gather_class_stats":       # them apart (halo refresh of the logits in between)
-            want.update({("dca_tap_gather3d",) + t[1:]: 1, ("dca_class_stats",) + t[1:]: 1})
-        else:
-            want.update({t: 1})
+    want = collections.Counter(slab)
     want.update({("dca_class_stats", 1, 6, 4, W4 // 2, 0): 3})          # S[b,k] over the 4 owned 1/8-res rows, per cva
     got = collections.Counter(sharded)
     assert got == collections.Counter({k: v * world for k, v in want.items()})
+    # the requests of one rank: 5 feature maps + mask + 4 dres + 3 x (6 at 1/8 res + fused + out) + head + pred_q
+    # exchanged, one live row each; the attention output's border-only replicate fill and the S all-reduce once per cva
+    with _dryrun.recording():
+        with torch.no_grad():
+            reqs = list(hs.hot_path_steps(pk, *[hs.owned_rows(f, world, 1) for f in feats]))
+    rows = [r for r in reqs if isinstance(r, hs.Rows)]
+    assert len(reqs) == 42 and sum(isinstance(r, hs.Sum) for r in reqs) == 3
+    assert all(r.nlive == 1 for r in rows if r.exchange)
+    assert collections.Counter(r.h for r in rows if r.exchange) == {2: 18, 1: 18}
+    assert [(r.h, r.fill) for r in rows if not r.exchange] == [(2, "replicate")] * 3
 
 
 def test_default_forward_buffer_dataflow():

@@ -65,9 +65,6 @@ def _oracle_steps(sd, gl, gr, cl, cr, g):
         yield Rows(fp, 2, 2, live=1)
         feats.append(fp)
     gl, gr, cl, cr, g = feats
-    m1 = F.relu(ctx.bn(ctx.conv2d(g, "prop.conv.0.0.weight"), "prop.conv.0.1")).contiguous()
-    yield Rows(m1, 2, 2, live=1)
-    mlog = ctx.conv2d(m1, "prop.conv.2.weight")
     vol = torch.cat([O.build_gwc_volume(gl, gr, D4, 40), O.build_concat_volume(cl, cr, D4)], dim=1)
     c = ctx.convbn3d(vol, "dres0.0", 1, 1, "relu")
     yield Rows(c, 3, 2, live=1)
@@ -84,6 +81,9 @@ def _oracle_steps(sd, gl, gr, cl, cr, g):
     yield Rows(h, 3, 2, live=1)
     logits = ctx.conv3d(h, "classif3.2.weight", 1, 1).squeeze(1)
     pred_q = O.disparity_regression(F.softmax(logits, dim=1), D4).contiguous()
+    m1 = F.relu(ctx.bn(ctx.conv2d(g, "prop.conv.0.0.weight"), "prop.conv.0.1")).contiguous()
+    yield Rows(m1, 2, 2, live=1)
+    mlog = ctx.conv2d(m1, "prop.conv.2.weight")
     yield Rows(pred_q, 2, 2, fill="zero", live=1)
     B, _, H, W = pred_q.shape
     m = F.softmax(mlog.view(B, 9, 4, 4, H, W), dim=1)
