@@ -1,9 +1,11 @@
 """B200-native DCANet cost-volume hot path (feature maps -> disparity) behind the reference's module API."""
-from . import _lib, engine, evaluation, frontend, gwcnet, hshard, kitti_io, pipeline
+from . import _lib, engine, evaluation, frontend, geometry, gwcnet, hshard, kitti_io, pipeline
 from . import gwcnet_dca0_g, gwcnet_dca1_g, gwcnet_dca2_g, gwcnet_dca4_g
 from .cva import Multi_Aggregation, cva
 from .engine import LR_CONSISTENT, LR_MISMATCH, LR_OCCLUDED, LR_OUT_OF_VIEW, Confidence, LRCheck
 from .evaluation import DisparityMeter, evaluate_files, read_kitti_disparity, read_pfm
+from .geometry import (PointCloud, StereoCalib, read_kitti_calib, read_middlebury_calib, reproject,
+                       reproject_files, save_depth_png, save_ply)
 from .gwcnet_dca_g import GwcNet, feature_extraction, hourglass
 from .pipeline import HotPathPipeline
 from .self_attention import SelfAttentionBlock
@@ -23,4 +25,6 @@ __all__ = ["GwcNet", "feature_extraction", "hourglass", "cva", "Multi_Aggregatio
            "SelfAttentionBlock", "PropgationNet_4x", "build_gwc_volume", "build_concat_volume", "build_cost_planes",
            "disparity_regression", "softmax_disparity_regression", "convbn", "convbn_3d", "engine", "hshard", "kitti_io", "HotPathPipeline",
            "evaluation", "DisparityMeter", "evaluate_files", "read_pfm", "read_kitti_disparity", "Confidence",
-           "LRCheck", "lr_consistency", "LR_CONSISTENT", "LR_OCCLUDED", "LR_MISMATCH", "LR_OUT_OF_VIEW"]
+           "LRCheck", "lr_consistency", "LR_CONSISTENT", "LR_OCCLUDED", "LR_MISMATCH", "LR_OUT_OF_VIEW", "geometry",
+           "StereoCalib", "PointCloud", "read_kitti_calib", "read_middlebury_calib", "reproject", "reproject_files",
+           "save_ply", "save_depth_png"]

@@ -6,6 +6,7 @@
 //   disparity_metrics   per image: valid / sum |pred - gt| (fixed point) / E > 1, 2, 3 / D1 / non-finite predictions
 //   class_confusion     conf[gt class][predicted class] of the 1/8-res DCA class maps
 //   confidence_histograms  (count, sum |E|) per confidence bin and per error bin: the sparsification curves
+//   depth_metrics       per image: the depth errors of the Eigen et al. protocol from disparities and one calibration
 #include <limits.h>
 
 #include "dca_common.cuh"
@@ -173,9 +174,85 @@ confidence_histograms_kernel(const float* __restrict__ pred, const float* __rest
   }
 }
 
+// Depth errors (DCA_DEPTH_*): the grid and the reduction of disparity_metrics_kernel; the four sums use SUM_ABS's
+// fixed-point conversion (fminf(NaN, 2^20) = 2^20)
+struct DepthParams {
+  float max_valid, fb, doffs, min_depth, max_depth;
+};
+
+__global__ void __launch_bounds__(MT_THREADS)
+depth_metrics_kernel(const float* __restrict__ pred, const float* __restrict__ gt, unsigned long long* __restrict__ rows,
+                     int HW, const DepthParams P) {
+  __shared__ unsigned long long red[MT_WARPS][DCA_DEPTH_COUNT];
+  pdl_wait();
+  const int b = blockIdx.y;
+  const float* pb = pred + (size_t)b * HW;
+  const float* gb = gt + (size_t)b * HW;
+  unsigned long long v[DCA_DEPTH_COUNT];
+#pragma unroll
+  for (int m = 0; m < DCA_DEPTH_COUNT; ++m) v[m] = 0ull;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < HW; i += gridDim.x * blockDim.x) {
+    const float g = __ldg(gb + i);
+    if (!gt_valid(g, P.max_valid)) continue;
+    const float zg = __fdiv_rn(P.fb, __fadd_rn(g, P.doffs));
+    if (!(zg >= P.min_depth && zg <= P.max_depth)) continue;
+    const float pd = __fadd_rn(__ldg(pb + i), P.doffs);
+    float zp = (isfinite(pd) && pd > 0.f) ? __fdiv_rn(P.fb, pd) : P.max_depth;
+    zp = fminf(fmaxf(zp, P.min_depth), P.max_depth);
+    const float e = __fsub_rn(zp, zg);
+    const float e2 = __fmul_rn(e, e);
+    const float lg = __fsub_rn(logf(zp), logf(zg));
+    const float ratio = fmaxf(__fdiv_rn(zp, zg), __fdiv_rn(zg, zp));
+    v[DCA_DEPTH_VALID] += 1;
+    v[DCA_DEPTH_ABS_REL] += abs_err_fix(__fdiv_rn(fabsf(e), zg));
+    v[DCA_DEPTH_SQ_REL] += abs_err_fix(__fdiv_rn(e2, zg));
+    v[DCA_DEPTH_SQ] += abs_err_fix(e2);
+    v[DCA_DEPTH_LOG_SQ] += abs_err_fix(__fmul_rn(lg, lg));
+    v[DCA_DEPTH_A1] += ratio < 1.25f;
+    v[DCA_DEPTH_A2] += ratio < 1.5625f;
+    v[DCA_DEPTH_A3] += ratio < 1.953125f;
+  }
+  const unsigned full = 0xffffffffu;
+#pragma unroll
+  for (int m = 0; m < DCA_DEPTH_COUNT; ++m) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v[m] += __shfl_xor_sync(full, v[m], o);
+  }
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (lane == 0) {
+#pragma unroll
+    for (int m = 0; m < DCA_DEPTH_COUNT; ++m) red[warp][m] = v[m];
+  }
+  __syncthreads();
+  if (threadIdx.x < DCA_DEPTH_COUNT) {
+    unsigned long long t = 0;
+#pragma unroll
+    for (int w = 0; w < MT_WARPS; ++w) t += red[w][threadIdx.x];
+    if (t) atomicAdd(rows + (size_t)b * DCA_DEPTH_COUNT + threadIdx.x, t);
+  }
+}
+
 }  // namespace dca
 
 using namespace dca;
+
+extern "C" int dca_depth_metrics(const float* pred, const float* gt, unsigned long long* rows, int B, int H, int W,
+                                 float max_valid, float focal_baseline, float doffs, float min_depth, float max_depth,
+                                 void* stream) {
+  if (!pred || !gt || !rows || B <= 0 || H <= 0 || W <= 0 || B > 65535 || max_valid != max_valid) return DCA_ERR_ARG;
+  if (!(focal_baseline > 0.f) || isinf(focal_baseline) || !isfinite(doffs) || !(min_depth > 0.f) ||
+      !(max_depth >= min_depth) || isinf(max_depth))
+    return DCA_ERR_ARG;
+  if ((long long)H * W > INT_MAX - MT_THREADS) return DCA_ERR_UNSUPPORTED;
+  const int HW = H * W;
+  int bx = (HW + MT_THREADS - 1) / MT_THREADS;
+  const int cap = (4 * dca_num_sms() + B - 1) / B;
+  if (bx > cap) bx = cap;
+  const DepthParams P = {max_valid, focal_baseline, doffs, min_depth, max_depth};
+  dca_launch(depth_metrics_kernel, dim3(bx, B), MT_THREADS, 0, (cudaStream_t)stream, pred, gt, rows, HW, P);
+  DCA_RETURN_IF_LAUNCH_FAILED();
+  return DCA_OK;
+}
 
 extern "C" int dca_disparity_metrics(const float* pred, const float* gt, unsigned long long* rows, int B, int H, int W,
                                      float max_valid, void* stream) {

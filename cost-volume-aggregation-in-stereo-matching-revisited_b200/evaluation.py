@@ -6,7 +6,8 @@
                                    dca_class_confusion (main_dca.py:66-120, 209-232), and with a confidence map the
                                    sparsification tables of dca_confidence_histograms; no host sync until read back
   summarize                        counters -> EPE / bad-N / D1 under both conventions, pixel accuracy / mPA / mIoU,
-                                   sparsification curves and AUSE of the confidence
+                                   sparsification curves and AUSE of the confidence, and with a calibration the depth
+                                   errors of dca_depth_metrics (abs rel, sq rel, RMSE, RMSE log, delta < 1.25^k)
   evaluate_files                   the `mytest` loop as a streaming pipeline (ImagePipeline plus a GT slot per pair);
                                    with lr_check=True also the metrics of the left-right consistent pixels and of the
                                    background-filled disparity
@@ -14,6 +15,7 @@
 Per-rank meters of a distributed run combine by concatenating their `rows()` (and summing `confusion()` and the
 `sparsification_histograms()`) before `summarize`.  There is no CPU path: the kernels need CUDA tensors.
 """
+import math
 import warnings
 
 import numpy as np
@@ -31,6 +33,9 @@ SUM_ABS_UNIT = 2.0 ** -20          # SUM_ABS is fixed point: px = SUM_ABS * 2^-2
 CONF_BINS = 256                    # DCA_CONF_BINS: confidence bins of width 1/256
 ERR_BINS = 2048 + 1                # DCA_ERR_BINS: 1/32 px error bins over [0, 64) and one for E >= 64
 ERR_BIN_PX = 1.0 / 32
+# column order of the depth rows (DCA_DEPTH_* of include/dca_b200.h); the four sums are fixed point, unit 2^-20
+DEPTH_VALID, DEPTH_ABS_REL, DEPTH_SQ_REL, DEPTH_SQ, DEPTH_LOG_SQ, DEPTH_A1, DEPTH_A2, DEPTH_A3 = range(8)
+DEPTH_COUNT = 8
 SPARSIFICATION_DENSITY = [k / 20 for k in range(20, 0, -1)]        # 1.00, 0.95, ..., 0.05
 
 
@@ -90,6 +95,15 @@ def _confidence_histograms(pred, gt, peak, conf_hist, err_hist, max_valid):
               err_hist.data_ptr(), B, H, W, max_valid, torch.cuda.current_stream(pred.device).cuda_stream)
 
 
+def _depth_metrics(pred, gt, rows, max_valid, focal_baseline, doffs, min_depth, max_depth):
+    """rows int64 [B, DEPTH_COUNT] += depth errors of pred / gt fp32 [B,H,W] under one calibration
+    (dca_depth_metrics)."""
+    _require_cuda(pred, gt, rows)
+    B, H, W = pred.shape
+    _lib.call("dca_depth_metrics", pred.data_ptr(), gt.data_ptr(), rows.data_ptr(), B, H, W, max_valid,
+              focal_baseline, doffs, min_depth, max_depth, torch.cuda.current_stream(pred.device).cuda_stream)
+
+
 def _as_bhw(t, what):
     if t.dim() == 4 and t.shape[1] == 1:
         t = t[:, 0]
@@ -107,11 +121,12 @@ class DisparityMeter:
     max_valid   GT upper bound of the valid mask: None = maxdisp (the (gt > 0) & (gt < maxdisp) mask of the GwcNet /
                 PSMNet test loops), 0 = no upper bound (KITTI devkit)
     device      where the counter tables live; None = the device of the first prediction
+    min_depth, max_depth   the depth range (metres) of the depth errors of updates with a calibration
 
     `update` launches the two kernels on the current stream and never synchronises; it allocates only when the row
     table doubles.  `rows()` / `confusion()` / `summary()` are the read-back points."""
 
-    def __init__(self, maxdisp, max_valid=None, device=None, capacity=64):
+    def __init__(self, maxdisp, max_valid=None, device=None, capacity=64, min_depth=1e-3, max_depth=80.0):
         self.maxdisp = int(maxdisp)
         self.D8 = self.maxdisp // 8
         self.max_valid = float(self.maxdisp if max_valid is None else max_valid)
@@ -124,6 +139,9 @@ class DisparityMeter:
         self._n = 0
         self._has_conf = False
         self._with_confidence = None      # set by the first update: every update carries a confidence map, or none does
+        self.min_depth, self.max_depth = float(min_depth), float(max_depth)
+        self._depth_rows = None
+        self._with_calib = None           # the same rule for calibrations: depth rows cover the same images as the rows
         if self.device is not None:
             self._alloc()
 
@@ -134,13 +152,14 @@ class DisparityMeter:
     def __len__(self):
         return self._n
 
-    def update(self, pred4, disp_true, prob_volume=None, confidence=None):
+    def update(self, pred4, disp_true, prob_volume=None, confidence=None, calib=None):
         """Score a batch: pred4 [B,1,H,W] (or [B,H,W]) against disp_true [B,H,W] (or [B,1,H,W]) in the same pixel
         frame, both fp32 on the same device; prob_volume [B,D8,H/8,W/8] (the model's second output) adds to the
         confusion matrix; confidence (the `peak` map of the model's Confidence output, in pred4's frame) adds to the
         sparsification tables.  Either every update of a meter passes a confidence map or none does (ValueError
         otherwise): the tables must cover the same pixels as the counter rows, so that the sparsification curves end
-        at epe_pooled."""
+        at epe_pooled.  calib (a geometry.StereoCalib shared by the batch) adds one row of depth errors per image; the
+        same rule applies: every update passes one or none does."""
         pred, gt = _as_bhw(pred4, "pred4"), _as_bhw(disp_true, "disp_true")
         if gt.shape != pred.shape:
             raise ValueError(f"disp_true {tuple(gt.shape)} and pred4 {tuple(pred.shape)} differ")
@@ -160,6 +179,9 @@ class DisparityMeter:
         if self._with_confidence is not None and (confidence is not None) != self._with_confidence:
             raise ValueError("confidence: every update of a meter passes a confidence map or none does (this meter has "
                              f"had updates {'with' if self._with_confidence else 'without'} one)")
+        if self._with_calib is not None and (calib is not None) != self._with_calib:
+            raise ValueError("calib: every update of a meter passes a calibration or none does (this meter has had "
+                             f"updates {'with' if self._with_calib else 'without'} one)")
         pk = None
         if confidence is not None:
             pk = _as_bhw(confidence, "confidence")
@@ -173,6 +195,10 @@ class DisparityMeter:
             grown = torch.zeros((self._cap, METRIC_COUNT), dtype=torch.int64, device=self.device)
             grown[:self._n].copy_(self._rows[:self._n])
             self._rows = grown
+            if self._depth_rows is not None:
+                grown = torch.zeros((self._cap, DEPTH_COUNT), dtype=torch.int64, device=self.device)
+                grown[:self._n].copy_(self._depth_rows[:self._n])
+                self._depth_rows = grown
         _disparity_metrics(pred, gt, self._rows[self._n:self._n + B], self.max_valid)
         if pv is not None:
             _class_confusion(pv, gt, self._conf, self.max_valid)
@@ -182,7 +208,13 @@ class DisparityMeter:
                 self._conf_hist = torch.zeros((CONF_BINS, 2), dtype=torch.int64, device=self.device)
                 self._err_hist = torch.zeros((ERR_BINS, 2), dtype=torch.int64, device=self.device)
             _confidence_histograms(pred, gt, pk, self._conf_hist, self._err_hist, self.max_valid)
+        if calib is not None:
+            if self._depth_rows is None:
+                self._depth_rows = torch.zeros((self._cap, DEPTH_COUNT), dtype=torch.int64, device=self.device)
+            _depth_metrics(pred, gt, self._depth_rows[self._n:self._n + B], self.max_valid, calib.focal_baseline,
+                           calib.doffs, self.min_depth, self.max_depth)
         self._with_confidence = confidence is not None
+        self._with_calib = calib is not None
         self._n += B
 
     def _readback(self, t):
@@ -209,9 +241,17 @@ class DisparityMeter:
             return None
         return self._readback(self._conf_hist), self._readback(self._err_hist)
 
+    def depth_rows(self):
+        """numpy uint64 [N, DEPTH_COUNT]: one depth-error row per image, in update order, or None when the updates
+        carried no calibration."""
+        if self._depth_rows is None:
+            return None
+        return self._readback(self._depth_rows[:self._n])
+
     def summary(self):
         h = self.sparsification_histograms()
-        return summarize(self.rows(), self.confusion() if self._has_conf else None, *(h or (None, None)))
+        return summarize(self.rows(), self.confusion() if self._has_conf else None, *(h or (None, None)),
+                         depth_rows=self.depth_rows())
 
 
 def _nanmean(a):
@@ -250,7 +290,7 @@ def _auc(curve):
     return float(sum(0.5 * (curve[i] + curve[i + 1]) * (x[i + 1] - x[i]) for i in range(len(x) - 1)))
 
 
-def summarize(rows, confusion=None, conf_hist=None, err_hist=None):
+def summarize(rows, confusion=None, conf_hist=None, err_hist=None, depth_rows=None):
     """Counter rows [N, METRIC_COUNT] (+ confusion [D8,D8]) (+ the sparsification tables) -> dict of metrics.
 
     epe, bad1, bad2, bad3, d1            mean over images of the per-image values (GwcNet / PSMNet test loops); images
@@ -271,7 +311,13 @@ def summarize(rows, confusion=None, conf_hist=None, err_hist=None):
                                  error-sorted curve of the sparsification literature; DESIGN.md section 4 on its name)
     auc_epe, ause_epe            trapezoid of the confidence curve over the removed fraction 1 - q in [0, 0.95], and
                                  that minus the same area of the ideal curve (px; 0 = a perfect ranking)
-    At q = 1 both curves equal epe_pooled exactly (the same integer sums)."""
+    At q = 1 both curves equal epe_pooled exactly (the same integer sums).
+
+    With depth rows (DisparityMeter.depth_rows), `depth` = the Eigen et al. errors, each as the mean over images of the
+    per-image value (images without valid pixels skipped) and as *_pooled over all pixels:
+    abs_rel = mean |Zp-Zg|/Zg, sq_rel = mean (Zp-Zg)^2/Zg (m), rmse = sqrt(mean (Zp-Zg)^2) (m),
+    rmse_log = sqrt(mean (ln Zp - ln Zg)^2), a1 / a2 / a3 = fraction with max(Zp/Zg, Zg/Zp) < 1.25 / 1.25^2 / 1.25^3;
+    plus n_valid, the pixels scored."""
     r = np.asarray(rows, dtype=np.uint64).reshape(-1, METRIC_COUNT).astype(np.float64)
     valid, nonfinite = r[:, VALID], r[:, PRED_NONFINITE]
     finite = valid - nonfinite
@@ -305,6 +351,27 @@ def summarize(rows, confusion=None, conf_hist=None, err_hist=None):
         out["sparsification_epe_ideal"] = ideal
         out["auc_epe"] = _auc(curve)
         out["ause_epe"] = out["auc_epe"] - _auc(ideal)
+    if depth_rows is not None:
+        out["depth"] = _depth_summary(depth_rows)
+    return out
+
+
+def _depth_summary(depth_rows):
+    r = np.asarray(depth_rows, dtype=np.uint64).reshape(-1, DEPTH_COUNT).astype(np.float64)
+    n = r[:, DEPTH_VALID]
+    has = n > 0
+    cols = {"abs_rel": (DEPTH_ABS_REL, SUM_ABS_UNIT, False), "sq_rel": (DEPTH_SQ_REL, SUM_ABS_UNIT, False),
+            "rmse": (DEPTH_SQ, SUM_ABS_UNIT, True), "rmse_log": (DEPTH_LOG_SQ, SUM_ABS_UNIT, True),
+            "a1": (DEPTH_A1, 1.0, False), "a2": (DEPTH_A2, 1.0, False), "a3": (DEPTH_A3, 1.0, False)}
+    out = {"n_valid": int(n.sum())}
+    total = n.sum()
+    for name, (col, unit, root) in cols.items():
+        per = r[has, col] * unit / n[has]
+        pooled = r[:, col].sum() * unit / total if total else float("nan")
+        if root:
+            per, pooled = np.sqrt(per), math.sqrt(pooled) if total else float("nan")
+        out[name] = float(per.mean()) if per.size else float("nan")
+        out[name + "_pooled"] = float(pooled)
     return out
 
 
@@ -322,12 +389,14 @@ class EvalPipeline(ImagePipeline):
     to multiples of 16 (main_dca.py:153-166), slot buffers follow each pair's padded size."""
 
     def __init__(self, model, meter, mode="fit", crop_height=384, crop_width=1248, depth=3, workers=2, confidence=False,
-                 lr_check=False, lr_threshold=1.0):
+                 lr_check=False, lr_threshold=1.0, calib=None):
         if mode not in ("fit", "pad16"):
             raise ValueError(f"mode must be 'fit' or 'pad16', got {mode!r}")
         super().__init__(model, crop_height, crop_width, depth, workers)
         self.meter, self.mode, self.confidence = meter, mode, confidence
         self.lr_check, self.lr_threshold = lr_check, lr_threshold
+        self.calib = calib             # None, one StereoCalib, or one per pair: the meter's depth errors
+        self._pair_calib = None
         # with lr_check: pred scored on the consistent pixels only, and the background-filled disparity on all of them
         self.lr_meters = {k: DisparityMeter(meter.maxdisp, meter.max_valid, meter.device)
                           for k in ("lr_consistent", "lr_filled")} if lr_check else {}
@@ -372,18 +441,20 @@ class EvalPipeline(ImagePipeline):
             out = self.model(x[None, 0:3], x[None, 3:6], confidence=self.confidence, lr_check=True,
                              lr_threshold=self.lr_threshold)
             pred, pv, lr = out[0], out[1], out[-1]
-            self.meter.update(pred, gt, pv if torch.is_tensor(pv) else None, out[2].peak if self.confidence else None)
+            self.meter.update(pred, gt, pv if torch.is_tensor(pv) else None, out[2].peak if self.confidence else None,
+                              calib=self._pair_calib)
             # zero GT = no GT: the inconsistent pixels leave this meter without a change to the metrics kernel
             self.lr_meters["lr_consistent"].update(pred, torch.where(lr.label.reshape(gt.shape) == 0, gt, 0.0))
             self.lr_meters["lr_filled"].update(lr.filled, gt)
             return pred.reshape(x.shape[1], x.shape[2])
         if self.confidence:          # (pred, prob_volume, Confidence(peak, std)): the peak map ranks the pixels
             pred, pv, conf = self.model(x[None, 0:3], x[None, 3:6], confidence=True)
-            self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None, conf.peak)
+            self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None, conf.peak,
+                              calib=self._pair_calib)
             return pred.reshape(x.shape[1], x.shape[2])
         out = self.model(x[None, 0:3], x[None, 3:6])
         pred, pv = (out[0], out[1]) if isinstance(out, (tuple, list)) else (out, None)
-        self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None)
+        self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None, calib=self._pair_calib)
         return pred.reshape(x.shape[1], x.shape[2])
 
     def _crop_back(self, disp, h, w, top):
@@ -398,6 +469,9 @@ class EvalPipeline(ImagePipeline):
         import threading
         from concurrent.futures import ThreadPoolExecutor
         quads = list(quads)
+        calibs = self.calib if isinstance(self.calib, (list, tuple)) else [self.calib] * len(quads)
+        if len(calibs) != len(quads):
+            raise ValueError(f"{len(calibs)} calibrations for {len(quads)} pairs")
         slot_sem = threading.Semaphore(self.depth)          # a slot is reusable once the writer is done with it
         q = queue.Queue()
         err = []
@@ -434,6 +508,7 @@ class EvalPipeline(ImagePipeline):
                     np.copyto(self.in_host[slot].numpy(), fitted)
                     np.copyto(self.gt_host[slot].numpy(), gt)
                     savename = quad[3]
+                    self._pair_calib = calibs[i]
                     if self.cuda:
                         with torch.cuda.stream(self.copy_stream):
                             if i >= self.depth:
@@ -463,7 +538,7 @@ class EvalPipeline(ImagePipeline):
 
 
 def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=2, maxdisp=None, max_valid=None,
-                   confidence=False, lr_check=False, lr_threshold=1.0):
+                   confidence=False, lr_check=False, lr_threshold=1.0, calib=None, min_depth=1e-3, max_depth=80.0):
     """main_dca.py `mytest` over files: quads = (left, right, gt_path, savename or None); GT is a KITTI PNG or a PFM
     (by extension).  maxdisp defaults to model.maxdisp, max_valid as in DisparityMeter.  Returns (summary dict,
     per-image counter rows [N, METRIC_COUNT] in input order); synchronises once, at the end.  confidence=True runs
@@ -474,19 +549,24 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
       lr_consistent   summarize() of pred against the GT of the pixels labelled consistent only
       lr_filled       summarize() of the background-filled disparity against the whole GT
       lr_density      lr_consistent's n_valid / n_valid: the fraction of the valid GT pixels that pass the check
-    The per-image rows returned are those of pred against the whole GT, as without the flag."""
+    The per-image rows returned are those of pred against the whole GT, as without the flag.
+
+    calib (one geometry.StereoCalib, or a list aligned with quads) adds `depth`: the depth errors of summarize() with
+    the GT depth fB / (gt + doffs) in [min_depth, max_depth] metres (80 m: the KITTI convention)."""
     if maxdisp is None:
         maxdisp = getattr(model, "maxdisp", 192)
     try:
         dev = next(model.parameters()).device
     except (StopIteration, AttributeError):
         dev = torch.device("cpu")
-    meter = DisparityMeter(maxdisp, max_valid, dev)
-    pipe = EvalPipeline(model, meter, mode, crop[0], crop[1], depth, workers, confidence, lr_check, lr_threshold)
+    meter = DisparityMeter(maxdisp, max_valid, dev, min_depth=min_depth, max_depth=max_depth)
+    pipe = EvalPipeline(model, meter, mode, crop[0], crop[1], depth, workers, confidence, lr_check, lr_threshold,
+                        calib)
     pipe.run(quads)
     rows = meter.rows()
     h = meter.sparsification_histograms()
-    summary = summarize(rows, meter.confusion() if meter._has_conf else None, *(h or (None, None)))
+    summary = summarize(rows, meter.confusion() if meter._has_conf else None, *(h or (None, None)),
+                        depth_rows=meter.depth_rows())
     if lr_check:
         for k, m in pipe.lr_meters.items():
             summary[k] = summarize(m.rows())

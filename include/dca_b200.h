@@ -303,6 +303,28 @@ int dca_class_confusion(const float* logits, const float* gt, unsigned long long
 #define DCA_ERR_BINS (2048 + 1)
 int dca_confidence_histograms(const float* pred, const float* gt, const float* peak, unsigned long long* conf_hist,
                               unsigned long long* err_hist, int B, int H, int W, float max_valid, void* stream);
+/* Depth errors of the Eigen et al. protocol (monodepth, pseudo-LiDAR) for a batch that shares one calibration,
+ * fB = focal_baseline (fx B, metres x px) and doffs (px), all in IEEE fp32:
+ *   pixels   valid GT as above, with Zg = fB / (gt + doffs) and min_depth <= Zg <= max_depth
+ *   Zp       fB / (pred + doffs), or max_depth when pred + doffs is not finite or <= 0; then clamped into
+ *            [min_depth, max_depth]
+ * rows [B][DCA_DEPTH_COUNT] += the counters of image b.  The four sums are fixed point like DCA_METRIC_SUM_ABS: each
+ * per-pixel term t is added as min(t, 2^20) * 2^20 rounded to nearest-even (unit 2^-20 of the term's unit), so a pixel
+ * adds <= 2^40 and a row is exact while it holds at most 2^23 valid pixels.  DCA_ERR_ARG for NULL pointers, B, H, W <= 0,
+ * B > 65535, a NaN max_valid, fB <= 0 or not finite, a non-finite doffs, min_depth <= 0 and max_depth not finite or
+ * < min_depth; DCA_ERR_UNSUPPORTED for H W > 2^31 - 257. */
+#define DCA_DEPTH_VALID 0      /* pixels scored */
+#define DCA_DEPTH_ABS_REL 1    /* sum |Zp - Zg| / Zg                   (unit 2^-20) */
+#define DCA_DEPTH_SQ_REL 2     /* sum (Zp - Zg)^2 / Zg                 (unit 2^-20 m) */
+#define DCA_DEPTH_SQ 3         /* sum (Zp - Zg)^2                      (unit 2^-20 m^2) */
+#define DCA_DEPTH_LOG_SQ 4     /* sum (ln Zp - ln Zg)^2 (logf)         (unit 2^-20) */
+#define DCA_DEPTH_A1 5         /* pixels with max(Zp / Zg, Zg / Zp) < 1.25 */
+#define DCA_DEPTH_A2 6         /* ... < 1.25^2 */
+#define DCA_DEPTH_A3 7         /* ... < 1.25^3 */
+#define DCA_DEPTH_COUNT 8
+int dca_depth_metrics(const float* pred, const float* gt, unsigned long long* rows, int B, int H, int W,
+                      float max_valid, float focal_baseline, float doffs, float min_depth, float max_depth,
+                      void* stream);
 
 /* (8) left-right consistency check and background fill ------------------------------------------------------------- */
 /* Right view.  DCANet is not mirror-symmetric (the guidance comes from the left image, the volume is built with the left
@@ -333,6 +355,31 @@ int dca_confidence_histograms(const float* pred, const float* gt, const float* p
 #define DCA_LR_MAX_W 4096
 int dca_lr_consistency(const float* disp_left, const float* disp_right, int right_mirrored, unsigned char* label,
                        float* filled, float* disp_right_out, int B, int H, int W, float tau, void* stream);
+
+/* (9) metric depth and 3-D points: reprojection of a disparity window ------------------------------------------------ */
+/* Pixel (y, x) of an H x W window, with d = disp, all in fp32 with explicit rounding (no contraction), each matrix row
+ * applied as ((m0 a + m1 b) + m2 c) + m3:
+ *   u = x + u0, v = y + v0 (exact)
+ *   (X', Y', Z', W') = Q (u, v, d, 1),  X = X' / W', Y = Y' / W', Z = Z' / W'   (OpenCV's reprojectImageTo3D convention;
+ *                                       for a rectified pair Q = [[1,0,0,-cx],[0,fx/fy,0,-cy fx/fy],[0,0,0,fx],
+ *                                       [0,0,1/B,doffs/B]] gives Z = fx B / (d + doffs))
+ * The pixel is KEPT iff d is finite, W' > 0, min_depth <= Z <= max_depth, (peak == NULL or peak >= min_peak) and
+ * (label == NULL or label == DCA_LR_CONSISTENT).  A kept pixel appends P = T (X, Y, Z, 1) ((X, Y, Z) when T is NULL) to
+ * xyz[b], its window index y W + x to index[b], and sets depth[b, y, x] = Z (camera-frame Z, before T); any other pixel
+ * sets depth[b, y, x] = 0 (KITTI's "no depth") and appends nothing.  Points are in row-major pixel order whatever the
+ * scheduling; count[b] = the number kept, rows of xyz[b] / index[b] past it are not written.
+ * disp, peak (fp32, optional) and label (uint8 DCA_LR_*, optional) share one layout: element (b, y, x) at
+ * b pitch_img + y pitch_row + x, so a cropped view of pred4 needs no copy.  Q_host [4][4] and T_host [3][4] (or NULL) are
+ * HOST pointers, row-major, that travel as launch parameters.  Outputs: depth fp32 [B,H,W] (NULL = not written),
+ * xyz fp32 [B][H W][3], index int32 [B][H W], count int64 [B]; workspace int32 [B][ceil(H W / DCA_REPROJECT_TILE)]
+ * holds the per-tile counts between the two launches (count, then an ordered scatter; no CTA waits on another).
+ * DCA_ERR_ARG for NULL required pointers, B, H, W <= 0, B > 65535, H W >= 2^31, pitch_row < W, pitch_img < H pitch_row,
+ * a NaN min_peak / min_depth / max_depth and min_depth > max_depth. */
+#define DCA_REPROJECT_TILE 1024
+int dca_reproject(const float* disp, const float* peak, const unsigned char* label, long long pitch_row,
+                  long long pitch_img, int B, int H, int W, int u0, int v0, const float* Q_host, const float* T_host,
+                  float min_peak, float min_depth, float max_depth, float* depth, float* xyz, int* index,
+                  long long* count, int* workspace, void* stream);
 
 /* layout + parameter preparation ---------------------------------------------------------------- */
 int dca_planes_from_ncdhw(const float* x, void* y, int planes, int B, int C, int Cp, int D, int H, int W,
