@@ -8,6 +8,8 @@ from .geometry import (PointCloud, StereoCalib, read_kitti_calib, read_middlebur
                        reproject_files, save_depth_png, save_ply)
 from .gwcnet_dca_g import GwcNet, feature_extraction, hourglass
 from .pipeline import HotPathPipeline
+from .rectify import (RectifyPipeline, Rectified, StereoRectifier, read_kitti_raw_rectifier, rectify,
+                      rectify_files)
 from .self_attention import SelfAttentionBlock
 from .semantic_level import SemanticLevelContext
 from .submodule import (PropgationNet_4x, build_concat_volume, build_cost_planes, build_gwc_volume, convbn,
@@ -27,4 +29,5 @@ __all__ = ["GwcNet", "feature_extraction", "hourglass", "cva", "Multi_Aggregatio
            "evaluation", "DisparityMeter", "evaluate_files", "read_pfm", "read_kitti_disparity", "Confidence",
            "LRCheck", "lr_consistency", "LR_CONSISTENT", "LR_OCCLUDED", "LR_MISMATCH", "LR_OUT_OF_VIEW", "geometry",
            "StereoCalib", "PointCloud", "read_kitti_calib", "read_middlebury_calib", "reproject", "reproject_files",
-           "save_ply", "save_depth_png"]
+           "save_ply", "save_depth_png", "StereoRectifier", "read_kitti_raw_rectifier", "rectify", "Rectified",
+           "RectifyPipeline", "rectify_files"]

@@ -86,6 +86,8 @@ SIGNATURES = {
     "dca_lr_consistency": [_vp, _vp, _c_int, _vp, _vp, _vp] + [_c_int] * 3 + [_f, _vp],
     "dca_reproject": [_vp, _vp, _vp, _ll, _ll] + [_c_int] * 5 + [_vp, _vp, _f, _f, _f] + [_vp] * 6,
     "dca_depth_metrics": [_vp, _vp, _vp] + [_c_int] * 3 + [_f] * 5 + [_vp],
+    "dca_rectify": [_vp, _vp, _c_int, _ll, _ll] + [_c_int] * 3 + [_vp] + [_c_int] * 2 + [_vp] * 3,
+    "dca_standardise_frame": [_vp, _vp] + [_c_int] * 3 + [_vp, _vp] + [_c_int] * 6 + [_vp],
 }
 _RESTYPES = {"dca_pack_weights_tc_bytes": ctypes.c_longlong, "dca_pack_weights_tc2d_bytes": ctypes.c_longlong,
              "dca_pack_weights_tc_march_bytes": ctypes.c_longlong}

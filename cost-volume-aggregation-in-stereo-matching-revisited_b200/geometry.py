@@ -242,11 +242,15 @@ class ReprojectPipeline(ImagePipeline):
                        asynchronous D2H of xyz, index, count and the depth map into the slot's pinned buffers
       writer thread    gathers the colours through index, writes the PLY and the depth PNG
 
-    mode "fit" / "pad16" frame the pair as EvalPipeline does; points carry the original image's pixel coordinates."""
+    mode "fit" / "pad16" frame the pair as EvalPipeline does; points carry the original image's pixel coordinates.
+
+    With a rectifier (rectify.StereoRectifier) the pairs are raw: the loaders only decode, the slots carry the raw uint8
+    pair, the compute stream runs rectify.rectify before the forward, and the colours come from the rectified left image
+    (one asynchronous D2H of the window into a pinned slot).  Points then carry rectified-image pixel coordinates."""
 
     def __init__(self, model, calibs, mode="fit", crop_height=384, crop_width=1248, min_confidence=None,
                  lr_check=False, lr_threshold=1.0, frame="camera", min_depth=0.0, max_depth=math.inf, depth=3,
-                 workers=2):
+                 workers=2, rectifier=None):
         if mode not in ("fit", "pad16"):
             raise ValueError(f"mode must be 'fit' or 'pad16', got {mode!r}")
         super().__init__(model, crop_height, crop_width, depth, workers)
@@ -254,6 +258,15 @@ class ReprojectPipeline(ImagePipeline):
         self.min_confidence, self.lr_check, self.lr_threshold = min_confidence, lr_check, lr_threshold
         self.frame, self.min_depth, self.max_depth = frame, min_depth, max_depth
         self.slot_out = [None] * self.depth          # (xyz, index, count, depth) host buffers per slot
+        self.rectifier = rectifier
+        if rectifier is not None:
+            from .rectify import RawSlots, framing
+            W, H = rectifier.rect_size
+            self.rect_window = framing(H, W, mode, (crop_height, crop_width))[1]
+            self.in_host = self.in_dev = None                  # the fp32 input slots are not used
+            self.raw = RawSlots(self, rectifier)
+            h, w = self.rect_window[2:4]
+            self.rgb_out = [self._host((h, w, 3), torch.uint8) for _ in range(self.depth)]
 
     def _host(self, shape, dtype):
         t = torch.empty(shape, dtype=dtype)
@@ -289,14 +302,24 @@ class ReprojectPipeline(ImagePipeline):
         return fitted[0].numpy(), np.ascontiguousarray(imgs[0][:, :, :3]), (top, 0, h, w, 0)
 
     def _reproject(self, slot, calib, window):
+        if self.rectifier is not None:
+            from .rectify import rectify
+            raw = self.raw.dev[slot]
+            x = rectify(raw[0:1], raw[1:2], self.rectifier, self.mode, (self.ch, self.cw))
+            y0, x0, h, w, vo = x.window
+            self.rgb_out[slot].copy_(x.rgb[0, 0, vo:vo + h, x0:x0 + w], non_blocking=self.cuda)
+            return self._forward_reproject(x.left, x.right, calib, x.window)
         x = self.in_dev[slot]
+        return self._forward_reproject(x[None, 0:3], x[None, 3:6], calib, window)
+
+    def _forward_reproject(self, left, right, calib, window):
         conf = self.min_confidence is not None
         kw = {}
         if conf:
             kw["confidence"] = True
         if self.lr_check:
             kw.update(lr_check=True, lr_threshold=self.lr_threshold)
-        out = self.model(x[None, 0:3], x[None, 3:6], **kw)
+        out = self.model(left, right, **kw)
         pred = out[0] if isinstance(out, (tuple, list)) else out
         return reproject(pred, calib, confidence=out[2].peak if conf else None,
                          min_confidence=self.min_confidence if conf else 0.0,
@@ -310,6 +333,8 @@ class ReprojectPipeline(ImagePipeline):
         import threading
         from concurrent.futures import ThreadPoolExecutor
         items = list(items)
+        if self.rectifier is not None:
+            return self._run_raw(items)
         calibs = self.calibs if isinstance(self.calibs, (list, tuple)) else [self.calibs] * len(items)
         if len(calibs) != len(items):
             raise ValueError(f"{len(calibs)} calibrations for {len(items)} items")
@@ -383,14 +408,108 @@ class ReprojectPipeline(ImagePipeline):
             raise err[0]
         return results
 
+    def _run_raw(self, items):
+        """run() on raw pairs (self.rectifier set): the same slot ring, with uint8 raw pairs in and the rectified left
+        window's colours out."""
+        import queue
+        import threading
+        from concurrent.futures import ThreadPoolExecutor
+        calibs = self.calibs if self.calibs is not None else self.rectifier.calib
+        calibs = calibs if isinstance(calibs, (list, tuple)) else [calibs] * len(items)
+        if len(calibs) != len(items):
+            raise ValueError(f"{len(calibs)} calibrations for {len(items)} items")
+        _, _, h, w, _ = self.rect_window
+        results = [None] * len(items)
+        slot_sem = threading.Semaphore(self.depth)
+        q = queue.Queue()
+        err = []
 
-def reproject_files(model, items, calib, mode="fit", crop=(384, 1248), min_confidence=None, lr_check=False,
-                    lr_threshold=1.0, frame="camera", min_depth=0.0, max_depth=math.inf, depth=3, workers=2):
+        def writer():
+            while True:
+                item = q.get()
+                if item is None:
+                    return
+                i, slot, ply, png = item
+                try:
+                    if self.cuda:
+                        self.done[slot].synchronize()
+                    xyz_h, idx_h, cnt_h, dep_h = self.slot_out[slot]
+                    n = int(cnt_h[0])
+                    xyz = xyz_h[:n].numpy().copy()
+                    col = self.rgb_out[slot].numpy().reshape(-1, 3)[idx_h[:n].numpy()]
+                    if ply is not None:
+                        save_ply(ply, xyz, col)
+                    if png is not None:
+                        save_depth_png(png, dep_h.numpy())
+                    results[i] = (xyz, col)
+                except Exception as e:          # surfaced by run()
+                    err.append(e)
+                finally:
+                    slot_sem.release()
+
+        wt = threading.Thread(target=writer, daemon=True)
+        wt.start()
+        was_training = getattr(self.model, "training", False)
+        if hasattr(self.model, "eval"):
+            self.model.eval()
+        try:
+            with ThreadPoolExecutor(self.workers) as pool, torch.no_grad():
+                futs = [pool.submit(self.raw.load, it[0], it[1]) for it in items]
+                for i, (fut, it) in enumerate(zip(futs, items)):
+                    raw = fut.result()
+                    slot_sem.acquire()
+                    slot = i % self.depth
+                    self._ensure_out(slot, h, w)
+                    self.raw.put(slot, raw)
+                    outs = self.slot_out[slot]
+                    if self.cuda:
+                        with torch.cuda.stream(self.copy_stream):
+                            if i >= self.depth:
+                                self.copy_stream.wait_event(self.free[slot])     # kernels of the slot's previous pair
+                            self.raw.h2d(slot)
+                            self.h2d[slot].record(self.copy_stream)
+                        with torch.cuda.stream(self.compute_stream):
+                            self.compute_stream.wait_event(self.h2d[slot])
+                            pc = self._reproject(slot, calibs[i], None)
+                            self.free[slot].record(self.compute_stream)
+                            for hb, dv in zip(outs, (pc.xyz[0], pc.index[0], pc.count, pc.depth[0])):
+                                hb.copy_(dv, non_blocking=True)
+                            self.done[slot].record(self.compute_stream)
+                    else:
+                        pc = self._reproject(slot, calibs[i], None)
+                        for hb, dv in zip(outs, (pc.xyz[0], pc.index[0], pc.count, pc.depth[0])):
+                            hb.copy_(dv)
+                    q.put((i, slot, it[2], it[3]))
+        finally:
+            q.put(None)
+            wt.join()
+            if was_training and hasattr(self.model, "train"):
+                self.model.train()
+        if err:
+            raise err[0]
+        return results
+
+    def _ensure_out(self, slot, h, w):
+        o = self.slot_out[slot]
+        if o is None or tuple(o[3].shape) != (h, w):
+            self.slot_out[slot] = (self._host((h * w, 3), torch.float32), self._host((h * w,), torch.int32),
+                                   self._host((1,), torch.int64), self._host((h, w), torch.float32))
+
+
+def reproject_files(model, items, calib=None, mode="fit", crop=(384, 1248), min_confidence=None, lr_check=False,
+                    lr_threshold=1.0, frame="camera", min_depth=0.0, max_depth=math.inf, depth=3, workers=2,
+                    rectifier=None):
     """Stereo pairs on disk -> coloured point clouds.  items = (left, right, ply_path or None, depth_png_path or None);
     calib = one StereoCalib or a list aligned with items.  min_confidence drops pixels whose Confidence.peak is below
     it (the forward runs with confidence=True); lr_check=True keeps the left-right consistent pixels only.  Depth PNGs
     cover the image (fit with padding, pad16) or the centre crop (fit of a larger image).  Returns [(xyz float32 [n,3],
-    rgb uint8 [n,3])] in input order; PLY and PNG files are written as results arrive."""
+    rgb uint8 [n,3])] in input order; PLY and PNG files are written as results arrive.
+
+    rectifier = a rectify.StereoRectifier: the items are RAW pairs of rectifier.raw_size, rectified and standardised on
+    the device (rectify.rectify with this mode and crop); calib defaults to rectifier.calib, the colours come from the
+    rectified left image and the points carry rectified-image pixel coordinates."""
+    if calib is None and rectifier is None:
+        raise ValueError("reproject_files needs a calibration (calib=) or a rectifier (rectifier=)")
     pipe = ReprojectPipeline(model, calib, mode, crop[0], crop[1], min_confidence, lr_check, lr_threshold, frame,
-                             min_depth, max_depth, depth, workers)
+                             min_depth, max_depth, depth, workers, rectifier)
     return pipe.run(items)

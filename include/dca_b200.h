@@ -381,6 +381,47 @@ int dca_reproject(const float* disp, const float* peak, const unsigned char* lab
                   float min_peak, float min_depth, float max_depth, float* depth, float* xyz, int* index,
                   long long* count, int* workspace, void* stream);
 
+/* (10) rectification of raw stereo pairs and the standardised network input -------------------------------------- */
+/* dca_rectify.  maps fp32 [2][H][W][2] (view 0 = left, 1 = right): the source coordinate (sx, sy) of rectified pixel
+ * (y, x), pixel centres at integer coordinates (OpenCV's initUndistortRectifyMap convention, built once on the host).
+ * Per rectified pixel, view and channel c = 0..2, all in fp32 with explicit rounding (no contraction):
+ *   x0 = floorf(sx), ax = sx - x0, y0 = floorf(sy), ay = sy - y0
+ *   p00, p01, p10, p11 = the source bytes at (x0, y0), (x0+1, y0), (x0, y0+1), (x0+1, y0+1); a tap outside the source
+ *                        image is 0 (OpenCV's BORDER_CONSTANT, value 0); a non-finite sx or sy gives v = 0
+ *   v = (1-ay) ((1-ax) p00 + ax p01) + ay ((1-ax) p10 + ax p11), evaluated as written: each product rounded, then each
+ *       sum, (1-a) rounded first
+ *   q = clamp(rint(v), 0, 255)   (round half to even: __float2int_rn)
+ * Rounding to uint8 is deliberate: the result is what rectifying to a PNG and loading it gives, and the moments below are
+ * exact integers.  It is NOT bit-compatible with cv2.remap, which quantises the map to 1/32 px.
+ * Sources: left / right uint8 [B][Hs][Ws][channels], channels 3 (RGB) or 4 (RGBA, channel 3 unused); byte (b, y, x, c) at
+ * b pitch_img + y pitch_row + x channels + c, so a strided view or a pinned slot needs no copy.  Outputs: rgb uint8
+ * [B][2][H][W][3] (HWC, view 0 = left), and moments uint64 [B][2][3][2] += (sum q, sum q^2) of each image and channel;
+ * the caller zeroes moments.  Each CTA adds its 32-bit sums with one integer atomic per counter, so the totals are
+ * exact and deterministic.  One CTA per DCA_RECTIFY_TILE rectified pixels of one image.
+ *
+ * dca_standardise_frame.  Per image and channel, with N = H W, S = sum q, SS = sum q^2 from moments:
+ *   mean = S / N                                   fp64, correctly rounded (numpy's mean of the uint8 channel)
+ *   var  = fp64(N SS - S^2) / (fp64(N) fp64(N))    the numerator exact in 128-bit integers, then correctly rounded to
+ *                                                  fp64; the denominator one fp64 product; one fp64 division
+ *   std  = sqrt(var)                               fp64, correctly rounded
+ *   out  = fp32((q - mean) / std)                  fp64 subtraction and division, one rounding to fp32 (a constant
+ *                                                  channel gives NaN, as kitti_io.load_pair does)
+ * Framing: outputs left / right fp32 [B][3][Hn][Wn] (two tensors, NCHW); frame pixel (yn, xn) with
+ * dst_y0 <= yn < dst_y0 + win_h and xn < win_w takes rectified pixel (yn - dst_y0 + src_y0, xn), every other frame pixel
+ * is 0.  kitti_io.fit_to_crop of a smaller image is (Hn, Wn) = (crop_h, crop_w), dst_y0 = crop_h - H, src_y0 = 0,
+ * window H x W; of a larger one dst_y0 = 0, src_y0 = int((H - crop_h) / 2), window crop_h x crop_w; pad_to_multiple(16)
+ * is Hn, Wn = H, W rounded up to 16, dst_y0 = Hn - H, src_y0 = 0, window H x W.
+ *
+ * Both: DCA_ERR_ARG for NULL pointers, sizes <= 0, B > 65535, channels other than 3 or 4, pitch_row < Ws channels,
+ * pitch_img < Hs pitch_row, and a copy window outside the frame or the rectified image; DCA_ERR_UNSUPPORTED for
+ * H W, Hs Ws or Hn Wn >= 2^31 and Hs or Ws > 2^24. */
+#define DCA_RECTIFY_TILE 1024
+int dca_rectify(const unsigned char* left, const unsigned char* right, int channels, long long pitch_row,
+                long long pitch_img, int B, int Hs, int Ws, const float* maps, int H, int W, unsigned char* rgb,
+                unsigned long long* moments, void* stream);
+int dca_standardise_frame(const unsigned char* rgb, const unsigned long long* moments, int B, int H, int W, float* left,
+                          float* right, int Hn, int Wn, int dst_y0, int src_y0, int win_h, int win_w, void* stream);
+
 /* layout + parameter preparation ---------------------------------------------------------------- */
 int dca_planes_from_ncdhw(const float* x, void* y, int planes, int B, int C, int Cp, int D, int H, int W,
                           void* stream);
