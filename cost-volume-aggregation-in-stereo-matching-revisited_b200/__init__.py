@@ -1,5 +1,5 @@
 """B200-native DCANet cost-volume hot path (feature maps -> disparity) behind the reference's module API."""
-from . import _lib, engine, evaluation, frontend, geometry, gwcnet, hshard, kitti_io, pipeline
+from . import _lib, engine, evaluation, frontend, geometry, gwcnet, hshard, kitti_io, pipeline, wls
 from . import gwcnet_dca0_g, gwcnet_dca1_g, gwcnet_dca2_g, gwcnet_dca4_g
 from .cva import Multi_Aggregation, cva
 from .engine import LR_CONSISTENT, LR_MISMATCH, LR_OCCLUDED, LR_OUT_OF_VIEW, Confidence, LRCheck
@@ -12,6 +12,7 @@ from .rectify import (RectifyPipeline, Rectified, StereoRectifier, read_kitti_ra
                       rectify_files)
 from .self_attention import SelfAttentionBlock
 from .semantic_level import SemanticLevelContext
+from .wls import Refined, wls_filter
 from .submodule import (PropgationNet_4x, build_concat_volume, build_cost_planes, build_gwc_volume, convbn,
                         convbn_3d, disparity_regression, softmax_disparity_regression)
 
@@ -30,4 +31,4 @@ __all__ = ["GwcNet", "feature_extraction", "hourglass", "cva", "Multi_Aggregatio
            "LRCheck", "lr_consistency", "LR_CONSISTENT", "LR_OCCLUDED", "LR_MISMATCH", "LR_OUT_OF_VIEW", "geometry",
            "StereoCalib", "PointCloud", "read_kitti_calib", "read_middlebury_calib", "reproject", "reproject_files",
            "save_ply", "save_depth_png", "StereoRectifier", "read_kitti_raw_rectifier", "rectify", "Rectified",
-           "RectifyPipeline", "rectify_files"]
+           "RectifyPipeline", "rectify_files", "wls", "wls_filter", "Refined"]

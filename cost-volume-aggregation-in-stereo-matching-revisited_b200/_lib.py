@@ -88,6 +88,8 @@ SIGNATURES = {
     "dca_depth_metrics": [_vp, _vp, _vp] + [_c_int] * 3 + [_f] * 5 + [_vp],
     "dca_rectify": [_vp, _vp, _c_int, _ll, _ll] + [_c_int] * 3 + [_vp] + [_c_int] * 2 + [_vp] * 3,
     "dca_standardise_frame": [_vp, _vp] + [_c_int] * 3 + [_vp, _vp] + [_c_int] * 6 + [_vp],
+    "dca_wls_filter": [_vp, _vp, _vp, _ll, _ll] + [_c_int] * 3 + [_vp, _c_int, _ll, _ll, _vp, _f, _c_int, _f]
+                      + [_vp] * 4,
 }
 _RESTYPES = {"dca_pack_weights_tc_bytes": ctypes.c_longlong, "dca_pack_weights_tc2d_bytes": ctypes.c_longlong,
              "dca_pack_weights_tc_march_bytes": ctypes.c_longlong}

@@ -10,7 +10,7 @@
                                    errors of dca_depth_metrics (abs rel, sq rel, RMSE, RMSE log, delta < 1.25^k)
   evaluate_files                   the `mytest` loop as a streaming pipeline (ImagePipeline plus a GT slot per pair);
                                    with lr_check=True also the metrics of the left-right consistent pixels and of the
-                                   background-filled disparity
+                                   background-filled disparity, with wls= those of the refined disparity (wls.py)
 
 Per-rank meters of a distributed run combine by concatenating their `rows()` (and summing `confusion()` and the
 `sparsification_histograms()`) before `summarize`.  There is no CPU path: the kernels need CUDA tensors.
@@ -23,8 +23,8 @@ import torch
 
 from . import _lib
 from .engine import _require_cuda
-from .kitti_io import (ImagePipeline, crop_prediction, fit_gt_to_crop, load_pair, pad_gt_to_multiple, pad_to_multiple,
-                       save_disparity_png)
+from .kitti_io import ImagePipeline, crop_prediction, fit_gt_to_crop, pad_gt_to_multiple, save_disparity_png
+from .wls import wls_filter
 
 # column order of the counter rows (DCA_METRIC_* of include/dca_b200.h)
 VALID, SUM_ABS, GT1, GT2, GT3, D1, PRED_NONFINITE = range(7)
@@ -386,10 +386,15 @@ class EvalPipeline(ImagePipeline):
       writer thread    crops the prediction back and writes the KITTI PNG, as ImagePipeline does
 
     mode "fit": fit_to_crop / fit_gt_to_crop into crop_height x crop_width (my_img.py); "pad16": top/right zero padding
-    to multiples of 16 (main_dca.py:153-166), slot buffers follow each pair's padded size."""
+    to multiples of 16 (main_dca.py:153-166), slot buffers follow each pair's padded size.
+
+    wls (a dict of wls_filter's lam / sigma / num_iter / min_support, or None): the slots also carry the uint8 left
+    image of the window, and after the forward wls_filter refines the window of pred (of LRCheck.filled, with
+    LRCheck.label, when lr_check is set; with Confidence.peak when confidence is set) and `wls_meter` scores it against
+    the GT of the window."""
 
     def __init__(self, model, meter, mode="fit", crop_height=384, crop_width=1248, depth=3, workers=2, confidence=False,
-                 lr_check=False, lr_threshold=1.0, calib=None):
+                 lr_check=False, lr_threshold=1.0, calib=None, wls=None):
         if mode not in ("fit", "pad16"):
             raise ValueError(f"mode must be 'fit' or 'pad16', got {mode!r}")
         super().__init__(model, crop_height, crop_width, depth, workers)
@@ -403,6 +408,13 @@ class EvalPipeline(ImagePipeline):
         self.gt_host = [self._host(crop_height, crop_width) for _ in range(self.depth)]
         self.gt_dev = [torch.empty((crop_height, crop_width), dtype=torch.float32, device=self.dev)
                        for _ in range(self.depth)] if self.cuda else self.gt_host
+        self.wls = wls
+        self.wls_meter = DisparityMeter(meter.maxdisp, meter.max_valid, meter.device) if wls is not None else None
+        # with wls: the uint8 left image of the window per slot, flat buffers sized for the crop and grown only for
+        # larger windows (pad16), so pairs of varying size reuse the pinned memory through contiguous views
+        self.rgb_host = [None] * self.depth
+        self.rgb_dev = [None] * self.depth
+        self._pair_window = None
 
     def _host(self, *shape):
         t = torch.empty(shape, dtype=torch.float32)
@@ -420,19 +432,32 @@ class EvalPipeline(ImagePipeline):
         else:
             self.in_dev[slot], self.gt_dev[slot] = self.in_host[slot], self.gt_host[slot]
 
+    def _rgb_slot(self, slot, h, w):
+        """(host, device) contiguous uint8 [h,w,3] views of the slot's flat left-image buffers (the slot is idle here)."""
+        n = h * w * 3
+        t = self.rgb_host[slot]
+        if t is None or t.numel() < n:
+            t = torch.empty((max(n, self.ch * self.cw * 3),), dtype=torch.uint8)
+            self.rgb_host[slot] = t.pin_memory() if self.cuda else t
+            self.rgb_dev[slot] = torch.empty(t.shape, dtype=torch.uint8, device=self.dev) if self.cuda \
+                else self.rgb_host[slot]
+        return self.rgb_host[slot][:n].view(h, w, 3), self.rgb_dev[slot][:n].view(h, w, 3)
+
     def _load_eval(self, left, right, gt_path):
         gt = read_pfm(gt_path) if str(gt_path).lower().endswith(".pfm") else read_kitti_disparity(gt_path)
-        if self.mode == "fit":
-            fitted, h, w = self._load(left, right)
-            if gt.shape != (h, w):
-                raise ValueError(f"{gt_path}: ground truth {gt.shape} does not match the images ({h}, {w})")
-            return fitted, fit_gt_to_crop(gt, self.ch, self.cw), h, w, 0
-        pair = load_pair(left, right)
-        _, h, w = pair.shape
+        fitted, rgb, window, h, w = self._load_framed(left, right, self.mode)
         if gt.shape != (h, w):
             raise ValueError(f"{gt_path}: ground truth {gt.shape} does not match the images ({h}, {w})")
-        fitted, top, _ = pad_to_multiple(torch.from_numpy(pair)[None], 16)
-        return fitted[0].numpy(), pad_gt_to_multiple(gt, 16)[0], h, w, top
+        if self.mode == "fit":
+            return fitted, fit_gt_to_crop(gt, self.ch, self.cw), h, w, 0, rgb, window
+        return fitted, pad_gt_to_multiple(gt, 16)[0], h, w, window[0], rgb, window
+
+    def _wls_update(self, slot, pred, peak, lr):
+        y0, x0, h, w, _ = self._pair_window
+        src, label = (lr.filled, lr.label) if lr is not None else (pred, None)
+        rgb = self.rgb_dev[slot][:h * w * 3].view(h, w, 3)
+        ref = wls_filter(src, rgb, confidence=peak, label=label, window=self._pair_window, **self.wls)
+        self.wls_meter.update(ref.disp, self.gt_dev[slot][None, y0:y0 + h, x0:x0 + w])
 
     def _forward_eval(self, slot):
         x = self.in_dev[slot]
@@ -446,15 +471,21 @@ class EvalPipeline(ImagePipeline):
             # zero GT = no GT: the inconsistent pixels leave this meter without a change to the metrics kernel
             self.lr_meters["lr_consistent"].update(pred, torch.where(lr.label.reshape(gt.shape) == 0, gt, 0.0))
             self.lr_meters["lr_filled"].update(lr.filled, gt)
+            if self.wls is not None:
+                self._wls_update(slot, pred, out[2].peak if self.confidence else None, lr)
             return pred.reshape(x.shape[1], x.shape[2])
         if self.confidence:          # (pred, prob_volume, Confidence(peak, std)): the peak map ranks the pixels
             pred, pv, conf = self.model(x[None, 0:3], x[None, 3:6], confidence=True)
             self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None, conf.peak,
                               calib=self._pair_calib)
+            if self.wls is not None:
+                self._wls_update(slot, pred, conf.peak, None)
             return pred.reshape(x.shape[1], x.shape[2])
         out = self.model(x[None, 0:3], x[None, 3:6])
         pred, pv = (out[0], out[1]) if isinstance(out, (tuple, list)) else (out, None)
         self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None, calib=self._pair_calib)
+        if self.wls is not None:
+            self._wls_update(slot, pred, None, None)
         return pred.reshape(x.shape[1], x.shape[2])
 
     def _crop_back(self, disp, h, w, top):
@@ -501,12 +532,16 @@ class EvalPipeline(ImagePipeline):
             with ThreadPoolExecutor(self.workers) as pool, torch.no_grad():
                 futs = [pool.submit(self._load_eval, l, r, g) for l, r, g, _ in quads]
                 for i, (fut, quad) in enumerate(zip(futs, quads)):
-                    fitted, gt, h, w, top = fut.result()
+                    fitted, gt, h, w, top, rgb, window = fut.result()
                     slot_sem.acquire()
                     slot = i % self.depth
                     self._ensure(slot, fitted.shape[1], fitted.shape[2])
                     np.copyto(self.in_host[slot].numpy(), fitted)
                     np.copyto(self.gt_host[slot].numpy(), gt)
+                    if self.wls is not None:
+                        rgb_h, rgb_d = self._rgb_slot(slot, rgb.shape[0], rgb.shape[1])
+                        np.copyto(rgb_h.numpy(), rgb)
+                        self._pair_window = window
                     savename = quad[3]
                     self._pair_calib = calibs[i]
                     if self.cuda:
@@ -515,6 +550,8 @@ class EvalPipeline(ImagePipeline):
                                 self.copy_stream.wait_event(self.free[slot])     # kernels of the slot's previous pair
                             self.in_dev[slot].copy_(self.in_host[slot], non_blocking=True)
                             self.gt_dev[slot].copy_(self.gt_host[slot], non_blocking=True)
+                            if self.wls is not None:
+                                rgb_d.copy_(rgb_h, non_blocking=True)
                             self.h2d[slot].record(self.copy_stream)
                         with torch.cuda.stream(self.compute_stream):
                             self.compute_stream.wait_event(self.h2d[slot])
@@ -537,8 +574,12 @@ class EvalPipeline(ImagePipeline):
             raise err[0]
 
 
+WLS_KEYS = ("lam", "sigma", "num_iter", "min_support")
+
+
 def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=2, maxdisp=None, max_valid=None,
-                   confidence=False, lr_check=False, lr_threshold=1.0, calib=None, min_depth=1e-3, max_depth=80.0):
+                   confidence=False, lr_check=False, lr_threshold=1.0, calib=None, min_depth=1e-3, max_depth=80.0,
+                   wls=None):
     """main_dca.py `mytest` over files: quads = (left, right, gt_path, savename or None); GT is a KITTI PNG or a PFM
     (by extension).  maxdisp defaults to model.maxdisp, max_valid as in DisparityMeter.  Returns (summary dict,
     per-image counter rows [N, METRIC_COUNT] in input order); synchronises once, at the end.  confidence=True runs
@@ -552,7 +593,18 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
     The per-image rows returned are those of pred against the whole GT, as without the flag.
 
     calib (one geometry.StereoCalib, or a list aligned with quads) adds `depth`: the depth errors of summarize() with
-    the GT depth fB / (gt + doffs) in [min_depth, max_depth] metres (80 m: the KITTI convention)."""
+    the GT depth fB / (gt + doffs) in [min_depth, max_depth] metres (80 m: the KITTI convention).
+
+    wls=True (the defaults of wls.wls_filter) or a dict of its lam / sigma / num_iter / min_support adds `wls`:
+    summarize() of the refined disparity of the image window against the GT of the window.  The refinement uses the
+    left image, Confidence.peak when confidence=True, and LRCheck.filled with LRCheck.label when lr_check=True."""
+    if wls is not None and wls is not False:
+        wls = {} if wls is True else dict(wls)
+        bad = set(wls) - set(WLS_KEYS)
+        if bad:
+            raise ValueError(f"wls: unknown keys {sorted(bad)}, expected a subset of {WLS_KEYS}")
+    else:
+        wls = None
     if maxdisp is None:
         maxdisp = getattr(model, "maxdisp", 192)
     try:
@@ -561,7 +613,7 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
         dev = torch.device("cpu")
     meter = DisparityMeter(maxdisp, max_valid, dev, min_depth=min_depth, max_depth=max_depth)
     pipe = EvalPipeline(model, meter, mode, crop[0], crop[1], depth, workers, confidence, lr_check, lr_threshold,
-                        calib)
+                        calib, wls)
     pipe.run(quads)
     rows = meter.rows()
     h = meter.sparsification_histograms()
@@ -572,4 +624,6 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
             summary[k] = summarize(m.rows())
         n = summary["n_valid"]
         summary["lr_density"] = summary["lr_consistent"]["n_valid"] / n if n else float("nan")
+    if wls is not None:
+        summary["wls"] = summarize(pipe.wls_meter.rows())
     return summary, rows

@@ -18,7 +18,7 @@ import numpy as np
 import torch
 
 from . import _lib, engine
-from .kitti_io import ImagePipeline, load_pair, pad_to_multiple
+from .kitti_io import ImagePipeline
 
 REPROJECT_TILE = 1024          # DCA_REPROJECT_TILE: pixels per tile of the workspace
 
@@ -283,23 +283,8 @@ class ReprojectPipeline(ImagePipeline):
                                    self._host((1,), torch.int64), self._host((h, w), torch.float32))
 
     def _load_item(self, left, right):
-        from PIL import Image
-        imgs = [np.asarray(Image.open(x) if isinstance(x, (str, bytes)) or hasattr(x, "__fspath__") else x)
-                for x in (left, right)]
-        if self.mode == "fit":
-            fitted, h, w = self._load(imgs[0], imgs[1])
-            if h <= self.ch and w <= self.cw:
-                window = (self.ch - h, 0, h, w, 0)
-                rgb = imgs[0][:, :, :3]
-            else:
-                top = int((h - self.ch) / 2)
-                window = (0, 0, self.ch, self.cw, top)
-                rgb = imgs[0][top:top + self.ch, :self.cw, :3]
-            return fitted, np.ascontiguousarray(rgb), window
-        pair = load_pair(imgs[0], imgs[1])
-        _, h, w = pair.shape
-        fitted, top, _ = pad_to_multiple(torch.from_numpy(pair)[None], 16)
-        return fitted[0].numpy(), np.ascontiguousarray(imgs[0][:, :, :3]), (top, 0, h, w, 0)
+        fitted, rgb, window, _, _ = self._load_framed(left, right, self.mode)
+        return fitted, np.ascontiguousarray(rgb), window
 
     def _reproject(self, slot, calib, window):
         if self.rectifier is not None:

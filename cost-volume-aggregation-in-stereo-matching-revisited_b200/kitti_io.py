@@ -151,6 +151,29 @@ class ImagePipeline:
             fitted = np.ascontiguousarray(pair[:, start_y:start_y + self.ch, :self.cw], dtype=np.float32)
         return fitted, h, w
 
+    def _load_framed(self, left, right, mode):
+        """Decode, standardise and frame a pair, keeping the left image under the window: mode "fit" (fit_to_crop) or
+        "pad16" (pad_to_multiple(16)) -> (fitted float32 [6,Hn,Wn], left uint8 RGB [h,w,3] of the window (a view of
+        the decoded image), window, image height, image width).  window = (y0, x0, h, w, v_origin) selects the image part of a network-frame map
+        (geometry.reproject, wls.wls_filter)."""
+        from PIL import Image
+        imgs = [np.asarray(Image.open(x) if isinstance(x, (str, bytes)) or hasattr(x, "__fspath__") else x)
+                for x in (left, right)]
+        if mode == "fit":
+            fitted, h, w = self._load(imgs[0], imgs[1])
+            if h <= self.ch and w <= self.cw:
+                window = (self.ch - h, 0, h, w, 0)
+                rgb = imgs[0][:, :, :3]
+            else:
+                top = int((h - self.ch) / 2)
+                window = (0, 0, self.ch, self.cw, top)
+                rgb = imgs[0][top:top + self.ch, :self.cw, :3]
+            return fitted, rgb, window, h, w
+        pair = load_pair(imgs[0], imgs[1])
+        _, h, w = pair.shape
+        fitted, top, _ = pad_to_multiple(torch.from_numpy(pair)[None], 16)
+        return fitted[0].numpy(), imgs[0][:, :, :3], (top, 0, h, w, 0), h, w
+
     def _forward(self, slot):
         x = self.in_dev[slot]
         out = self.model(x[None, 0:3], x[None, 3:6])

@@ -422,6 +422,78 @@ int dca_rectify(const unsigned char* left, const unsigned char* right, int chann
 int dca_standardise_frame(const unsigned char* rgb, const unsigned long long* moments, int B, int H, int W, float* left,
                           float* right, int Hn, int Wn, int dst_y0, int src_y0, int win_h, int win_w, void* stream);
 
+/* (11) edge-aware refinement: confidence-weighted fast global smoother guided by the left image ------------------- */
+/* The fast global smoother of Min et al. (IEEE TIP 2014), the solver inside OpenCV's ximgproc DisparityWLSFilter.  The
+ * result is NOT bit-compatible with OpenCV's implementation (different weights, schedule rounding and solve order).
+ * Pixel p = (b, y, x) of an H x W window, all in fp32 with explicit rounding (no contraction); (+) (-) (x) (/) are the
+ * correctly rounded fp32 operations:
+ *   c = clamp(peak, 0, 1), 0 for a NaN peak, 1 without peak;  c = 0 where label != DCA_LR_CONSISTENT (with label) and
+ *       where d = disp is not finite
+ *   U = c (x) d where c > 0, else 0 (a non-finite d never enters);  V = c
+ *   w(p, q) = lut[sum over the channels 0..2 of (g_p - g_q)^2] for horizontal and vertical neighbours p, q (the sum is an
+ *       exact integer <= 3 255^2); lut[k] = fp32(exp(-sqrt(k) / sigma)) built in float64 on the host, so no
+ *       transcendental function runs on the device
+ *   for t = 1..T: lambda_t = fp32(((lambda 1.5) 4^(T-t)) / (4^T - 1)) in float64 (the FGS schedule, OpenCV's
+ *       lambda_attenuation = 0.25), computed by this entry point on the host; then one pass over every row (lines of
+ *       n = W along x), then one pass over every column (lines of n = H along y).  A pass solves, on each line, for U and
+ *       for V with the same matrix,
+ *         (1 + e_{i-1} + e_i) u_i - e_{i-1} u_{i-1} - e_i u_{i+1} = f_i,   e_i = lambda_t (x) w(i, i+1),
+ *         e_{-1} = e_{n-1} = 0,   b_i = (1 (+) e_{i-1}) (+) e_i
+ *       partitioned as follows (K = DCA_WLS_SEGMENT).  The separators are the elements c = K-1, 2K-1, ... with
+ *       c <= n-2; they split the line into S = DCA_WLS_SEGMENTS(n) segments [a, c) of 1..K elements (a = 0 or one past a
+ *       separator, c = the next separator or n), with eL = e_{a-1} (0 for a = 0) and eR = e_{c-1}.
+ *       THOMAS(f) of a segment, Thomas elimination in reciprocal form with e_{a-1} = eL, p = g = 0 before a, u = 0 at c:
+ *         forward  i = a..c-1:  m_i = 1 (/) (b_i (-) e_{i-1} (x) p_{i-1})
+ *                               p_i = e_i (x) m_i
+ *                               g_i = (f_i (+) e_{i-1} (x) g_{i-1}) (x) m_i
+ *         backward i = c-1..a:  u_i = g_i (+) p_i (x) u_{i+1}
+ *       (1) boundary values of each segment (only when S > 1), for U and V:
+ *           last element:  y_last = g_{c-1} of the forward sweep on f;  phi_last = G_{c-1} with G_a = eL (x) m_a,
+ *                          G_i = (e_{i-1} (x) G_{i-1}) (x) m_i;  psi_last = eR (x) m_{c-1}
+ *           first element: the reverse sweep i = c-1..a with r = h = 0 after c-1:
+ *                          q_i = 1 (/) (b_i (-) e_i (x) r_{i+1}),  r_i = e_{i-1} (x) q_i,
+ *                          h_i = (f_i (+) e_i (x) h_{i+1}) (x) q_i;  y_first = h_a;  phi_first = eL (x) q_a;
+ *                          psi_first = Q_a with Q_{c-1} = eR (x) q_{c-1}, Q_i = (e_i (x) Q_{i+1}) (x) q_i
+ *       (2) the separators x_0..x_{S-2} (x_s at c_s = (s+1) K - 1, between segments s and s+1), for U and V:
+ *           lo_s = e_{c-1} (x) phi_last(s),  up_s = e_c (x) psi_first(s+1),
+ *           D_s = (b_c (-) e_{c-1} (x) psi_last(s)) (-) e_c (x) phi_first(s+1),
+ *           r_s = (f_c (+) e_{c-1} (x) y_last(s)) (+) e_c (x) y_first(s+1);
+ *           forward s = 0..S-2 with P = G = 0 before 0:  M = 1 (/) (D_s (-) lo_s (x) P_{s-1}),  P_s = up_s (x) M,
+ *           G_s = (r_s (+) lo_s (x) G_{s-1}) (x) M;  backward with x_{S-1} = 0:  x_s = G_s (+) P_s (x) x_{s+1}
+ *       (3) each segment: THOMAS(f') with f' = f except f'_a = f_a (+) eL (x) x_{s-1} when a > 0, then
+ *           f'_{c-1} = f'_{c-1} (+) eR (x) x_s when c < n (in that order when a = c-1)
+ *       The solution (the separators' x, the segments' u) replaces f.  With S = 1 (n <= K) the pass is THOMAS(f) on
+ *       the whole line.
+ *   support = V after the last pass: in [0, 1] up to the rounding of the fp32 solves (the exact solve averages, so a
+ *       pixel far from any confident pixel gets a small support);  refined = U (/) V where V >= min_support, else disp
+ * min_support = 0 makes 0 / 0 = NaN possible where V = 0; the default of the Python wrapper is 1e-3, because where
+ * every path to a confident pixel crosses strong colour edges V underflows towards the denormals and U / V loses all
+ * precision (DESIGN.md, "Refinement").
+ * disp, peak (fp32, optional) and label (uint8 DCA_LR_*, optional) share one layout: element (b, y, x) at
+ * b pitch_img + y pitch_row + x, so a cropped view of pred4 needs no copy.  guide uint8 [B][H][W][channels], channels
+ * 3 (RGB) or 4 (RGBA, channel 3 unused): byte (b, y, x, c) at b guide_pitch_img + y guide_pitch_row + x channels + c.
+ * lut fp32 [DCA_WLS_LUT_SIZE] on the device.  Outputs refined, support fp32 [B,H,W] (contiguous; they hold U and V
+ * between the passes).  workspace = DCA_WLS_WORKSPACE_BYTES(B, H, W) bytes: the horizontal and vertical weights and 8
+ * boundary values per segment of each pass.  A pass is 3 launches (1 when its lines have no separator), so a call is
+ * at most 1 + 6T; no host sync, no allocation: capturable in a CUDA graph.  DCA_ERR_ARG for NULL required pointers,
+ * B, H, W <= 0, B > 65535, channels other than 3 or 4, pitch_row < W, pitch_img < H pitch_row,
+ * guide_pitch_row < W channels, guide_pitch_img < H guide_pitch_row, num_iter outside 1..DCA_WLS_MAX_ITER, a lambda that
+ * is NaN, infinite or negative and a NaN or negative min_support; DCA_ERR_UNSUPPORTED for H W >= 2^31 and for more
+ * than 65535 segments per line (H or W > 65535 K). */
+#define DCA_WLS_LUT_SIZE (3 * 255 * 255 + 1)
+#define DCA_WLS_MAX_ITER 8
+#define DCA_WLS_SEGMENT 64
+#define DCA_WLS_SEGMENTS(n) (((n) - 1) / DCA_WLS_SEGMENT + 1)
+#define DCA_WLS_WORKSPACE_BYTES(B, H, W)                                                                              \
+  (4ull * (unsigned long long)(B) *                                                                                   \
+   (2ull * (unsigned long long)(H) * (unsigned long long)(W) +                                                        \
+    8ull * ((unsigned long long)(H) * DCA_WLS_SEGMENTS((unsigned long long)(W)) +                                     \
+            (unsigned long long)(W) * DCA_WLS_SEGMENTS((unsigned long long)(H)))))
+int dca_wls_filter(const float* disp, const float* peak, const unsigned char* label, long long pitch_row,
+                   long long pitch_img, int B, int H, int W, const unsigned char* guide, int channels,
+                   long long guide_pitch_row, long long guide_pitch_img, const float* lut, float lambda, int num_iter,
+                   float min_support, float* refined, float* support, void* workspace, void* stream);
+
 /* layout + parameter preparation ---------------------------------------------------------------- */
 int dca_planes_from_ncdhw(const float* x, void* y, int planes, int B, int C, int Cp, int D, int H, int W,
                           void* stream);
