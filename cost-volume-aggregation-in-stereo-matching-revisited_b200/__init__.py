@@ -1,9 +1,10 @@
 """B200-native DCANet cost-volume hot path (feature maps -> disparity) behind the reference's module API."""
-from . import _lib, engine, evaluation, frontend, geometry, gwcnet, hshard, kitti_io, pipeline, wls
+from . import _lib, engine, evaluation, frontend, fusion, geometry, gwcnet, hshard, kitti_io, pipeline, wls
 from . import gwcnet_dca0_g, gwcnet_dca1_g, gwcnet_dca2_g, gwcnet_dca4_g
 from .cva import Multi_Aggregation, cva
 from .engine import LR_CONSISTENT, LR_MISMATCH, LR_OCCLUDED, LR_OUT_OF_VIEW, Confidence, LRCheck
 from .evaluation import DisparityMeter, evaluate_files, read_kitti_disparity, read_pfm
+from .fusion import SurfacePoints, TSDFVolume, fuse_files, read_kitti_poses
 from .geometry import (PointCloud, StereoCalib, read_kitti_calib, read_middlebury_calib, reproject,
                        reproject_files, save_depth_png, save_ply)
 from .gwcnet_dca_g import GwcNet, feature_extraction, hourglass
@@ -31,4 +32,5 @@ __all__ = ["GwcNet", "feature_extraction", "hourglass", "cva", "Multi_Aggregatio
            "LRCheck", "lr_consistency", "LR_CONSISTENT", "LR_OCCLUDED", "LR_MISMATCH", "LR_OUT_OF_VIEW", "geometry",
            "StereoCalib", "PointCloud", "read_kitti_calib", "read_middlebury_calib", "reproject", "reproject_files",
            "save_ply", "save_depth_png", "StereoRectifier", "read_kitti_raw_rectifier", "rectify", "Rectified",
-           "RectifyPipeline", "rectify_files", "wls", "wls_filter", "Refined"]
+           "RectifyPipeline", "rectify_files", "wls", "wls_filter", "Refined", "fusion", "TSDFVolume", "SurfacePoints",
+           "fuse_files", "read_kitti_poses"]

@@ -90,6 +90,10 @@ SIGNATURES = {
     "dca_standardise_frame": [_vp, _vp] + [_c_int] * 3 + [_vp, _vp] + [_c_int] * 6 + [_vp],
     "dca_wls_filter": [_vp, _vp, _vp, _ll, _ll] + [_c_int] * 3 + [_vp, _c_int, _ll, _ll, _vp, _f, _c_int, _f]
                       + [_vp] * 4,
+    "dca_tsdf_integrate": [_vp] + [_c_int] * 4 + [_f] * 4 + [_c_int] * 6 + [_vp, _vp, _ll, _ll] + [_c_int] * 3
+                          + [_vp, _c_int, _ll, _ll] + [_f] * 4 + [_c_int] * 2 + [_vp] + [_f] * 3 + [_vp],
+    "dca_tsdf_count_surface": [_vp] + [_c_int] * 4 + [_f, _vp, _vp, _vp],
+    "dca_tsdf_extract_surface": [_vp] + [_c_int] * 4 + [_f] * 5 + [_vp, _ll, _vp, _vp, _vp, _vp],
 }
 _RESTYPES = {"dca_pack_weights_tc_bytes": ctypes.c_longlong, "dca_pack_weights_tc2d_bytes": ctypes.c_longlong,
              "dca_pack_weights_tc_march_bytes": ctypes.c_longlong}

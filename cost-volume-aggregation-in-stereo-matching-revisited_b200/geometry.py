@@ -204,10 +204,16 @@ def reproject(disp, calib, *, confidence=None, min_confidence=0.0, label=None, f
 
 
 # ---- writers --------------------------------------------------------------------------------------------------
-def save_ply(path, xyz, rgb=None):
-    """Binary little-endian PLY: float x y z per vertex, plus uchar red green blue when rgb [n,3] is given."""
+def save_ply(path, xyz, rgb=None, normal=None):
+    """Binary little-endian PLY: float x y z per vertex, plus float nx ny nz when normal [n,3] is given and uchar red
+    green blue when rgb [n,3] is given."""
     xyz = np.asarray(xyz, np.float32).reshape(-1, 3)
     fields = [("x", "<f4"), ("y", "<f4"), ("z", "<f4")]
+    if normal is not None:
+        normal = np.asarray(normal, np.float32).reshape(-1, 3)
+        if len(normal) != len(xyz):
+            raise ValueError(f"{len(xyz)} points and {len(normal)} normals")
+        fields += [("nx", "<f4"), ("ny", "<f4"), ("nz", "<f4")]
     if rgb is not None:
         rgb = np.asarray(rgb, np.uint8).reshape(-1, 3)
         if len(rgb) != len(xyz):
@@ -215,6 +221,8 @@ def save_ply(path, xyz, rgb=None):
         fields += [("red", "u1"), ("green", "u1"), ("blue", "u1")]
     v = np.empty(len(xyz), dtype=fields)
     v["x"], v["y"], v["z"] = xyz[:, 0], xyz[:, 1], xyz[:, 2]
+    if normal is not None:
+        v["nx"], v["ny"], v["nz"] = normal[:, 0], normal[:, 1], normal[:, 2]
     if rgb is not None:
         v["red"], v["green"], v["blue"] = rgb[:, 0], rgb[:, 1], rgb[:, 2]
     props = "".join(f"property {'float' if t == '<f4' else 'uchar'} {n}\n" for n, t in fields)

@@ -494,6 +494,69 @@ int dca_wls_filter(const float* disp, const float* peak, const unsigned char* la
                    long long guide_pitch_row, long long guide_pitch_img, const float* lut, float lambda, int num_iter,
                    float min_support, float* refined, float* support, void* workspace, void* stream);
 
+/* (12) TSDF fusion of posed depth maps and the surface of the fused volume ----------------------------------------- */
+/* Curless & Levoy (SIGGRAPH 1996) in the projective form of KinectFusion (Newcombe et al., ISMAR 2011), on a dense grid.
+ * All in fp32 with explicit rounding (no contraction); (+) (-) (x) (/) are the correctly rounded fp32 operations and each
+ * matrix row is applied as ((m0 a (+) m1 b) (+) m2 c) (+) m3.
+ * Volume: nx x ny x nz voxels; voxel (i, j, k) has linear index v = (k ny + j) nx + i (x fastest) and centre
+ * p = (ox (+) vs (x) fp32(i), oy (+) vs (x) fp32(j), oz (+) vs (x) fp32(k)) in world metres.  State: planar fp32 with
+ * plane stride N = nx ny nz, plane 0 = tsdf T (initialised to 1), 1 = weight W (initialised to 0), 2..4 = colour r, g, b
+ * (initialised to 0; planes = 5) or no colour (planes = 2).  The caller initialises the state.
+ *
+ * dca_tsdf_integrate.  Only the voxels of the box i0..i0+bi-1, j0..j0+bj-1, k0..k0+bk-1 are read or written.  Per voxel,
+ * the state is held in registers while the frames b = 0..B-1 are applied in order (so one call with B frames equals B
+ * calls with one frame each, bit for bit); frame b is skipped at the first failing step:
+ *   (Xc, Yc, Zc) = T_b p, with T_b = T_host[b] the world-to-camera 3x4 (row-major);  skip unless Zc > 0
+ *   x = ((fx (x) Xc) (/) Zc) (+) cx (-) fp32(u0),  y = ((fy (x) Yc) (/) Zc) (+) cy (-) fp32(v0)
+ *   xf = floorf(x (+) 0.5), yf = floorf(y (+) 0.5);  skip unless 0 <= xf < W and 0 <= yf < H (in float, so NaN skips)
+ *   z = depth[b, yf, xf];  skip unless z is finite and 0 < z <= max_depth
+ *   w = the observation weight: 1 without a weight map, else the map clamped to [0, 1], 0 where it holds NaN;
+ *       skip unless w > 0
+ *   sdf = z (-) Zc;  skip if sdf < -trunc;  f = min(1, sdf (/) trunc)
+ *   Wn = W (+) w;  T = ((T (x) W) (+) (f (x) w)) (/) Wn;  with colour, for c = r, g, b with q = fp32 of the pixel's byte
+ *       C = ((C (x) W) (+) (q (x) w)) (/) Wn;  then W = min(Wn, max_weight)
+ * A voxel that no frame updates is left as it was.  depth (and weight, optional) fp32: element (b, y, x) at
+ * b pitch_img + y pitch_row + x (window pixel (x, y) is image pixel (x + u0, y + v0), as in dca_reproject).  rgb uint8
+ * [B][H][W][channels], channels 3 (RGB) or 4 (RGBA, channel 3 unused): byte (b, y, x, c) at
+ * b rgb_pitch_img + y rgb_pitch_row + x channels + c; it is required with planes = 5 and must be NULL with planes = 2.
+ * T_host [B][12] is a HOST pointer that travels as launch parameters.  One launch, no atomics, no host sync, no
+ * allocation: capturable in a CUDA graph.
+ * DCA_ERR_ARG for NULL volume / depth / T_host, planes other than 2 or 5, nx, ny, nz, H, W <= 0, B outside
+ * 1..DCA_TSDF_MAX_FRAMES, pitch_row < W, pitch_img < H pitch_row, an rgb given or missing against planes, channels other
+ * than 3 or 4, rgb_pitch_row < W channels, rgb_pitch_img < H rgb_pitch_row, a box that is empty or leaves the grid, NaN
+ * ox / oy / oz / fx / fy / cx / cy / max_depth, voxel_size, trunc or max_weight not > 0 (max_weight = inf: no cap);
+ * DCA_ERR_UNSUPPORTED for N >= 2^31, H or W >= 2^24 and |u0| or |v0| >= 2^24.
+ *
+ * Surface crossings.  For voxel v and axis a in (x, y, z) whose neighbour n = v + e_a lies inside the grid, there is a
+ * crossing when W(v) >= min_weight, W(n) >= min_weight and (T(v) < 0) != (T(n) < 0).  Its point is p(v) with component
+ * a replaced by p_a(v) (+) (t (x) vs), t = T(v) (/) (T(v) (-) T(n)).  Points are ordered by v, then by axis x, y, z.
+ *   normal: g = (T(i+1) (-) T(i-1), T(j+1) (-) T(j-1), T(k+1) (-) T(k-1)) at v, each neighbour index clamped into the
+ *           grid; len = __fsqrt_rn((gx (x) gx (+) gy (x) gy) (+) gz (x) gz); g (/) len, or (0, 0, 0) when len = 0.  It
+ *           points from negative (behind the surface) to positive (towards the cameras).
+ *   colour: per channel clamp(rint(C(v) (+) t (x) (C(n) (-) C(v))), 0, 255) (round half to even), uint8.
+ * dca_tsdf_count_surface writes the crossings of each tile of DCA_TSDF_TILE voxels (in linear index order) to
+ * workspace int64 [ceil(N / DCA_TSDF_TILE)], then, in one CTA, replaces them by their exclusive prefix sums (each tile's
+ * first output row) and writes the total to count (int64, device).  dca_tsdf_extract_surface, on the same volume and
+ * min_weight after it, recomputes the crossings of each tile and writes rows o < capacity: xyz fp32 [capacity][3],
+ * normal fp32 [capacity][3] (NULL = not written), rgb uint8 [capacity][3] (NULL = not written; planes = 5 only).  count
+ * keeps the true total, so a caller sees a truncated extraction.  Three launches in all, no atomics, no CTA waits on
+ * another.  DCA_ERR_ARG for a NULL volume / workspace / count, planes other than 2 or 5, nx, ny, nz <= 0, a NaN
+ * min_weight, NaN ox / oy / oz, voxel_size not > 0, capacity < 0, a NULL xyz with capacity > 0 and rgb with planes = 2;
+ * DCA_ERR_UNSUPPORTED for N >= 2^31. */
+#define DCA_TSDF_MAX_FRAMES 16
+#define DCA_TSDF_TILE 1024
+int dca_tsdf_integrate(float* volume, int planes, int nx, int ny, int nz, float ox, float oy, float oz,
+                       float voxel_size, int i0, int j0, int k0, int bi, int bj, int bk, const float* depth,
+                       const float* weight, long long pitch_row, long long pitch_img, int B, int H, int W,
+                       const unsigned char* rgb, int channels, long long rgb_pitch_row, long long rgb_pitch_img,
+                       float fx, float fy, float cx, float cy, int u0, int v0, const float* T_host, float trunc,
+                       float max_weight, float max_depth, void* stream);
+int dca_tsdf_count_surface(const float* volume, int planes, int nx, int ny, int nz, float min_weight,
+                           long long* workspace, long long* count, void* stream);
+int dca_tsdf_extract_surface(const float* volume, int planes, int nx, int ny, int nz, float ox, float oy, float oz,
+                             float voxel_size, float min_weight, const long long* workspace, long long capacity,
+                             float* xyz, float* normal, unsigned char* rgb, void* stream);
+
 /* layout + parameter preparation ---------------------------------------------------------------- */
 int dca_planes_from_ncdhw(const float* x, void* y, int planes, int B, int C, int Cp, int D, int H, int W,
                           void* stream);
