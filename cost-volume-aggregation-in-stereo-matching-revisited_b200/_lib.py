@@ -94,6 +94,9 @@ SIGNATURES = {
                           + [_vp, _c_int, _ll, _ll] + [_f] * 4 + [_c_int] * 2 + [_vp] + [_f] * 3 + [_vp],
     "dca_tsdf_count_surface": [_vp] + [_c_int] * 4 + [_f, _vp, _vp, _vp],
     "dca_tsdf_extract_surface": [_vp] + [_c_int] * 4 + [_f] * 5 + [_vp, _ll, _vp, _vp, _vp, _vp],
+    "dca_tsdf_raycast": [_vp] + [_c_int] * 4 + [_f] * 10 + [_c_int] * 4 + [_vp, _f, _f] + [_vp, _ll] * 4 + [_vp],
+    "dca_icp_track": [_vp, _vp, _ll, _c_int, _c_int] + [_f] * 4 + [_c_int] * 2 + [_f, _vp, _ll, _vp, _ll, _vp, _c_int]
+                     + [_vp] * 3 + [_c_int] + [_vp] * 5,
 }
 _RESTYPES = {"dca_pack_weights_tc_bytes": ctypes.c_longlong, "dca_pack_weights_tc2d_bytes": ctypes.c_longlong,
              "dca_pack_weights_tc_march_bytes": ctypes.c_longlong}

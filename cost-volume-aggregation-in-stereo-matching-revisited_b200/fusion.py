@@ -6,8 +6,10 @@ volume (include/dca_b200.h section 12).
                      dca_tsdf_integrate per 16 frames (one launch, no host sync) on the voxel box that can see them;
                      .extract() -> SurfacePoints(xyz, normal, rgb): the zero crossings of the tsdf between neighbouring
                      voxels, in voxel order (count, one sync to read the total, then the ordered scatter)
+                     .raycast(cam_to_world, calib, shape, window=) -> Rendered(depth, vertex, normal, rgb): the fused
+                     surface seen from any pose (dca_tsdf_raycast, one launch, no host sync)
   read_kitti_poses   KITTI odometry poses.txt -> camera-to-world [N, 4, 4] float64 (camera 0, or with the sequence's
-                     calib.txt the rectified left colour camera the depth maps live in)
+                     calib.txt the rectified left colour camera the depth maps live in); save_kitti_poses writes them back
   fuse_files         stereo pairs on disk + poses -> one fused volume: ReprojectPipeline with the forward, reproject and
                      integrate on the compute stream, pair after pair in input order
 """
@@ -53,6 +55,28 @@ def _integrate_kernel(vol, box, depth, weight, rgb, intrinsics, u0, v0, T, max_d
               depth.data_ptr(), 0 if weight is None else weight.data_ptr(), pitch_row, pitch_img, B, H, W,
               0 if rgb is None else rgb.data_ptr(), C, c_row, c_img, *intrinsics, u0, v0, t.ctypes.data, vol.trunc,
               vol.max_weight, max_depth, torch.cuda.current_stream(vol.state.device).cuda_stream)
+
+
+class Rendered(NamedTuple):
+    """Device maps of one raycast, [h, w] of the window: depth fp32 (camera Z, 0 = no hit, as PointCloud.depth), vertex
+    fp32 [h,w,3] in the camera frame (NaN = no hit), normal fp32 [h,w,3] unit vectors in the camera frame pointing
+    towards the camera (NaN = no hit), rgb uint8 [h,w,3] or None (a volume without colour)."""
+    depth: torch.Tensor
+    vertex: torch.Tensor
+    normal: torch.Tensor
+    rgb: torch.Tensor
+
+
+def _raycast_kernel(vol, intrinsics, u0, v0, M, min_weight, min_depth, max_depth, out):
+    """One dca_tsdf_raycast into the Rendered `out` (contiguous maps of one window); M float32 [12] camera-to-world."""
+    engine._require_cuda(vol.state, *out)
+    h, w = out.depth.shape
+    nx, ny, nz = vol.dims
+    m = np.ascontiguousarray(M, np.float32)
+    _lib.call("dca_tsdf_raycast", vol.state.data_ptr(), vol.planes, nx, ny, nz, *vol.origin, vol.voxel_size, vol.trunc,
+              float(min_weight), *intrinsics, u0, v0, h, w, m.ctypes.data, float(min_depth), float(max_depth),
+              out.depth.data_ptr(), w, out.vertex.data_ptr(), 3 * w, out.normal.data_ptr(), 3 * w,
+              0 if out.rgb is None else out.rgb.data_ptr(), 3 * w, torch.cuda.current_stream(vol.state.device).cuda_stream)
 
 
 def _extract_kernel(vol, min_weight, normals, colours):
@@ -210,12 +234,7 @@ class TSDFVolume:
                                  f"{tuple(rgb.shape)} on {rgb.device}")
             if rgb.stride(3) != 1 or rgb.stride(2) != rgb.shape[3]:
                 rgb = rgb.contiguous()
-        u0 = v0 = 0
-        if window is not None:
-            _, x0, wh, ww, v_origin = (int(v) for v in window)
-            if (wh, ww) != (h, w):
-                raise ValueError(f"window {tuple(window)}: its size is not the {h}x{w} of the depth map")
-            u0, v0 = x0, v_origin
+        u0, v0 = _window_origin(window, h, w)
         if max_depth is not None and not max_depth > 0:
             raise ValueError(f"max_depth must be > 0 (inf = no limit) or None, got {max_depth!r}")
         c2w = _poses(cam_to_world, B)
@@ -239,6 +258,39 @@ class TSDFVolume:
                               None if rgb is None else rgb[s:e], intr, u0, v0, T[s:e], md)
         return self
 
+    def raycast(self, cam_to_world, calib, shape, window=None, min_weight=0.5, min_depth=0.0, max_depth=40.0):
+        """Render the fused surface from one pose, without a host sync -> Rendered on the volume's device.
+
+        cam_to_world  [4,4] or [3,4] float64 on the host, stored float32
+        calib         the StereoCalib of the rendered camera (fx, fy, cx, cy)
+        shape         (h, w) of the window
+        window        the (y0, x0, h, w, v_origin) of reproject: rendered pixel (x, y) is image pixel (x0 + x,
+                      v_origin + y); None = (0, 0, h, w, 0)
+        min_weight    a march sample whose 8 voxels do not all reach it is unknown (skipped, never a hit)
+        min_depth, max_depth   the march along camera Z; max_depth must be finite, the ray marches to it
+        The first crossing from positive to negative tsdf is the hit (include/dca_b200.h section 13).
+        save_depth_png writes Rendered.depth."""
+        h, w = (int(v) for v in shape)
+        if h <= 0 or w <= 0:
+            raise ValueError(f"shape {tuple(shape)}: two sizes > 0 expected")
+        u0, v0 = _window_origin(window, h, w)
+        if not min_weight == min_weight:
+            raise ValueError("min_weight is NaN")
+        if not (math.isfinite(max_depth) and 0 <= min_depth <= max_depth):
+            raise ValueError(f"min_depth {min_depth!r}, max_depth {max_depth!r}: 0 <= min_depth <= max_depth, finite")
+        M = _poses(cam_to_world, 1)[0, :3].reshape(12).astype(np.float32)
+        out = self._maps(h, w)
+        _raycast_kernel(self, (calib.fx, calib.fy, calib.cx, calib.cy), u0, v0, M, min_weight, min_depth, max_depth,
+                        out)
+        return out
+
+    def _maps(self, h, w):
+        dev = self.state.device
+        return Rendered(torch.empty((h, w), dtype=torch.float32, device=dev),
+                        torch.empty((h, w, 3), dtype=torch.float32, device=dev),
+                        torch.empty((h, w, 3), dtype=torch.float32, device=dev),
+                        torch.empty((h, w, 3), dtype=torch.uint8, device=dev) if self.colour else None)
+
     def extract(self, min_weight=0.5, normals=True, colours=None):
         """The surface points: crossings of the tsdf's sign between neighbouring voxels whose weights are both
         >= min_weight, ordered by voxel then axis -> SurfacePoints on the volume's device.  colours None = when the
@@ -256,6 +308,16 @@ class TSDFVolume:
         xyz, nrm, rgb = s.numpy()
         save_ply(path, xyz, rgb, normal=nrm)
         return s
+
+
+def _window_origin(window, h, w):
+    """reproject's window (y0, x0, h, w, v_origin) of an h x w map -> (u0, v0), the image pixel of map pixel (0, 0)."""
+    if window is None:
+        return 0, 0
+    _, x0, wh, ww, v_origin = (int(v) for v in window)
+    if (wh, ww) != (h, w):
+        raise ValueError(f"window {tuple(window)}: its size is not the {h}x{w} of the depth map")
+    return x0, v_origin
 
 
 def _bhw(t, what, dtype):
@@ -286,15 +348,33 @@ def read_kitti_poses(poses_txt, calib_path=None):
     if rows:
         out[:, :3] = np.stack(rows).reshape(-1, 3, 4)
     if calib_path is not None:
-        kv = _read_kv(calib_path, ":")
-        key = "P2" if "P2" in kv else "P_rect_02"
-        if key not in kv:
-            raise ValueError(f"{calib_path}: no P2 (or P_rect_02) projection matrix")
-        P2 = _floats(kv[key]).reshape(3, 4)
-        shift = np.eye(4)
-        shift[:3, 3] = (-P2[0, 3] / P2[0, 0], -P2[1, 3] / P2[1, 1], 0.0)
-        out = out @ shift
+        out = out @ _camera2_shift(calib_path)
     return out
+
+
+def _camera2_shift(calib_path):
+    """[4,4] pose of camera 2 in camera 0 from a KITTI calib.txt: the translation (-P2[0,3] / fx, -P2[1,3] / fy, 0)."""
+    kv = _read_kv(calib_path, ":")
+    key = "P2" if "P2" in kv else "P_rect_02"
+    if key not in kv:
+        raise ValueError(f"{calib_path}: no P2 (or P_rect_02) projection matrix")
+    P2 = _floats(kv[key]).reshape(3, 4)
+    shift = np.eye(4)
+    shift[:3, 3] = (-P2[0, 3] / P2[0, 0], -P2[1, 3] / P2[1, 1], 0.0)
+    return shift
+
+
+def save_kitti_poses(path, cam_to_world, calib_path=None):
+    """The inverse of read_kitti_poses: camera-to-world [N,4,4] or [N,3,4] float64 -> a KITTI odometry poses.txt (12
+    numbers per line, %.17g, so read_kitti_poses gives the poses back exactly).  With the sequence's calib.txt the poses
+    are of camera 2 (those of read_kitti_poses with that file, of TSDFVolume.integrate and of track_files) and camera 2's
+    offset is removed again, so the file holds camera 0 as the KITTI odometry devkit expects."""
+    m = _poses(cam_to_world)
+    if calib_path is not None:
+        m = m @ np.linalg.inv(_camera2_shift(calib_path))
+    with open(path, "w") as f:
+        for p in m:
+            f.write(" ".join("%.17g" % v for v in p[:3].ravel()) + "\n")
 
 
 # ---- files in, one fused volume out ---------------------------------------------------------------------------------
@@ -338,7 +418,8 @@ class FusePipeline(ReprojectPipeline):
                 else self.rgb_host[slot]
         np.copyto(self.rgb_host[slot].numpy(), rgb)
 
-    def _fuse(self, slot, calib, window, pose):
+    def _observe(self, slot, calib, window):
+        """The forward and reproject of the pair in `slot` -> (depth, weight map or None, colours, window)."""
         if self.rectifier is not None:
             from .rectify import rectify
             raw = self.raw.dev[slot]
@@ -366,8 +447,20 @@ class FusePipeline(ReprojectPipeline):
         if self.weight == "peak":
             y0, x0, h, w, _ = window
             wmap = out[2].peak[:, 0, y0:y0 + h, x0:x0 + w]
-        self.volume.integrate(pc.depth, calib, pose, weight=wmap, rgb=rgb if self.volume.colour else None,
+        return pc.depth, wmap, rgb, window
+
+    def _integrate(self, obs, calib, pose):
+        depth, wmap, rgb, window = obs
+        self.volume.integrate(depth, calib, pose, weight=wmap, rgb=rgb if self.volume.colour else None,
                               window=window, max_depth=self.fuse_max_depth)
+
+    def _fuse(self, slot, calib, window, pose):
+        """The device work of one pair, on the compute stream; returns what _finish needs (None here)."""
+        self._integrate(self._observe(slot, calib, window), calib, pose)
+
+    def _finish(self, pending):
+        """The host step of a pair whose _fuse returned `pending`, run after the next pair's copy is queued (nothing
+        here)."""
 
     def run(self, items, poses):
         """items: (left, right) file pairs; poses: camera-to-world [N,4,4] or [N,3,4] aligned with them.  Returns the
@@ -387,9 +480,13 @@ class FusePipeline(ReprojectPipeline):
             with ThreadPoolExecutor(self.workers) as pool, torch.no_grad():
                 load = self.raw.load if raw else self._load_item
                 futs = [pool.submit(load, it[0], it[1]) for it in items]
+                pending = None                                   # (slot, what _fuse returned) of the previous pair
                 for i, fut in enumerate(futs):
                     got = fut.result()
                     slot = i % self.depth
+                    if pending is not None and pending[0] == slot:
+                        self._close(pending)                     # one slot: the pair in it is finished first
+                        pending = None
                     if self.cuda and i >= self.depth:
                         self.free[slot].synchronize()            # the slot's previous pair is fused: its buffers are free
                     window = None
@@ -410,18 +507,32 @@ class FusePipeline(ReprojectPipeline):
                                 self.in_dev[slot].copy_(self.in_host[slot], non_blocking=True)
                                 self.rgb_dev[slot].copy_(self.rgb_host[slot], non_blocking=True)
                             self.h2d[slot].record(self.copy_stream)
+                        if pending is not None:
+                            self._close(pending)                 # after pair i's copy is queued
                         with torch.cuda.stream(self.compute_stream):
                             self.compute_stream.wait_event(self.h2d[slot])
-                            self._fuse(slot, calibs[i], window, poses[i])
-                            self.free[slot].record(self.compute_stream)
+                            pending = (slot, self._fuse(slot, calibs[i], window, poses[i]))
                     else:
-                        self._fuse(slot, calibs[i], window, poses[i])
+                        if pending is not None:
+                            self._close(pending)
+                        pending = (slot, self._fuse(slot, calibs[i], window, poses[i]))
+                if pending is not None:
+                    self._close(pending)
             if self.cuda:
                 torch.cuda.current_stream(self.dev).wait_stream(self.compute_stream)
         finally:
             if was_training and hasattr(self.model, "train"):
                 self.model.train()
         return self.volume
+
+    def _close(self, pending):
+        slot, state = pending
+        if self.cuda:
+            with torch.cuda.stream(self.compute_stream):
+                self._finish(state)
+                self.free[slot].record(self.compute_stream)
+        else:
+            self._finish(state)
 
 
 def fuse_files(model, items, poses, volume, calib=None, rectifier=None, mode="fit", crop=(384, 1248),

@@ -557,6 +557,118 @@ int dca_tsdf_extract_surface(const float* volume, int planes, int nx, int ny, in
                              float voxel_size, float min_weight, const long long* workspace, long long capacity,
                              float* xyz, float* normal, unsigned char* rgb, void* stream);
 
+/* (13) camera tracking against the fused volume: raycast model maps and projective point-to-plane ICP ------------ */
+/* The tracking half of KinectFusion (Newcombe et al., ISMAR 2011) with the linearised point-to-plane system of Low (2004).
+ * fp32 steps use the notation of section 12 ((+) (-) (x) (/) correctly rounded, no contraction, matrix rows applied as
+ * ((m0 a (+) m1 b) (+) m2 c) (+) m3); fp64 steps are __dadd_rn / __dmul_rn / __ddiv_rn / __dsqrt_rn, a - b as
+ * a + (-b).  Window pixel (x, y) is image pixel (x + u0, y + v0), as in dca_reproject and dca_tsdf_integrate.
+ *
+ * dca_tsdf_raycast.  Renders a volume in the state layout of section 12 through an H x W pinhole window.  M = T_host, the
+ * camera-to-world 3x4 (row-major, a HOST pointer that travels as launch parameters).  Per pixel:
+ *   xn = ((fp32(x) (+) fp32(u0)) (-) cx) (/) fx,  yn = ((fp32(y) (+) fp32(v0)) (-) cy) (/) fy
+ *   L = sqrt((xn (x) xn (+) yn (x) yn) (+) 1)           (ray length per metre of camera Z)
+ *   the sample at camera Z = z: c = (xn (x) z, yn (x) z, z), p = M c, g = ((p_a (-) o_a) (/) vs) per axis (grid units,
+ *       voxel centres at integers); it is UNKNOWN when a corner of its cell (floorf(g), floorf(g) + 1 per axis) lies
+ *       outside the grid or has weight < min_weight, else T = trilinear tsdf:
+ *       lerp(a, b, t) = a (+) t (x) (b (-) a) along x (fraction g_x (-) floorf(g_x)), then y, then z
+ *   march: z = min_depth, no previous sample; while z <= max_depth:
+ *       known T:  if the previous sample is known with Tp >= 0 and T < 0: hit, zh = zp (+) (z (-) zp) (x) (Tp (/) (Tp (-) T)),
+ *                 stop;  if the previous sample is known with Tp < 0 and T >= 0 (the back of a surface): stop, no hit;
+ *                 else s = max(vs (x) 0.5, |T| (x) trunc)
+ *       unknown:  s = trunc, and the next sample has no known previous sample (unknown samples never end the march)
+ *       z' = z (+) (s (/) L); stop (no hit) unless z' > z;  z = z'
+ *   Every step is at most trunc of ray length (|T| <= 1), so a known band of trunc on each side of a surface, crossed by
+ *   the ray over at least trunc of its length per band, holds a sample on each side: the ray cannot step over it.
+ *   With a hit at zh > 0, at h = the sample point of zh (c, p and g as above):
+ *     gradient  G_a = C(g (+) e_a) (-) C(g (-) e_a) per axis, C = the clamped trilinear tsdf: each coordinate clamped
+ *               into [0, n - 1], cell corner min(floorf, n - 2), weights ignored; len = sqrt((Gx Gx (+) Gy Gy) (+) Gz Gz);
+ *               len = 0 is no hit.  n_world = G (/) len (pointing from behind the surface towards the camera)
+ *     outputs   depth = zh (camera Z, the convention of dca_reproject's depth map);  vertex = (xn (x) zh, yn (x) zh, zh)
+ *               in the camera frame;  normal_k = ((M0k nwx (+) M1k nwy) (+) M2k nwz) (M^T n_world: camera frame);
+ *               rgb_c = clamp(rint(C_c(g)), 0, 255) (round half to even) with C_c the clamped trilinear colour plane
+ *   No hit: depth 0, vertex and normal NaN, rgb (0, 0, 0).
+ * Outputs fp32 depth [H][depth_pitch], vertex [H][vertex_pitch] (x, y, z per pixel), normal [H][normal_pitch], uint8
+ * rgb [H][rgb_pitch] (NULL = not written; planes = 5 only); pitches in elements (bytes for rgb).  One launch, no host
+ * sync, no allocation.  DCA_ERR_ARG for NULL volume / T_host / depth / vertex / normal, planes other than 2 or 5, nx, ny
+ * or nz < 2, non-finite origin, voxel_size not > 0, trunc not finite and > 0, a NaN min_weight, non-finite or zero
+ * fx / fy, non-finite cx / cy, min_depth not >= 0, max_depth not finite or < min_depth, a non-finite T_host, H, W <= 0,
+ * depth_pitch < W, vertex_pitch or normal_pitch < 3 W, rgb with planes = 2 or rgb_pitch < 3 W; DCA_ERR_UNSUPPORTED for
+ * N >= 2^31, H W >= 2^31, H, W, nx, ny or nz >= 2^24 and |u0| or |v0| >= 2^24.
+ *
+ * dca_icp_track.  All ICP iterations of one frame.  The source is a depth map (weight optional) of the window, element
+ * (y, x) at y pitch + x; the model is the vertex and normal maps of dca_tsdf_raycast with the same intrinsics and window,
+ * in the model camera's frame (pitches in elements).  A = T(model camera <- current camera), fp64 3x4, starts at A0_host
+ * (a HOST pointer that travels as launch parameters).  Levels l = 0..num_levels-1 run level_iters[l] iterations each
+ * with pixel stride s = level_stride[l] and distance gate G = level_gate[l] (fp32).  Per iteration, with Af = fp32(A)
+ * (rounded once), for each source pixel (x, y) with x % s = y % s = 0:
+ *   z = depth;  keep only z finite and 0 < z <= max_depth
+ *   w = 1 without weight, else the weight clamped to [0, 1], 0 where NaN;  keep only w > 0
+ *   p = ((((fp32(x) (+) fp32(u0)) (-) cx) (x) z) (/) fx, (((fp32(y) (+) fp32(v0)) (-) cy) (x) z) (/) fy, z)
+ *   q = Af p;  keep only 0 < q_z <= Q, |q_x| <= Q, |q_y| <= Q with Q = 2 (x) max_depth
+ *   xm = floorf((((fx (x) q_x) (/) q_z) (+) cx) (-) fp32(u0) (+) 0.5), ym likewise; keep only 0 <= xm < W, 0 <= ym < H
+ *   m, n = model vertex and normal at (xm, ym);  keep only (n.n) <= DCA_ICP_MAX_NORMAL2 (false for NaN: no model hit)
+ *   d = q (-) m;  keep only (dx dx (+) dy dy) (+) dz dz <= G (x) G (false for NaN)
+ *   r = (nx dx (+) ny dy) (+) nz dz;  J = (q x n, n) with (q x n) = (qy nz (-) qz ny, qz nx (-) qx nz, qx ny (-) qy nx):
+ *       the Jacobian of r for the left-multiplied update (omega, t)
+ *   sums, each term rounded to an integer (round half to even) after an exact scaling by a power of two:
+ *       H_ij (i <= j, row-major upper triangle) += rint(((w (x) J_i) (x) J_j) * DCA_ICP_SCALE_H)
+ *       g_i += rint(((w (x) J_i) (x) r) * DCA_ICP_SCALE_G);  e += rint(((w (x) r) (x) r) * DCA_ICP_SCALE_E)
+ *       sw += rint(w * DCA_ICP_SCALE_W);  count += 1
+ *   Integer sums are exact and order-free: each CTA of DCA_ICP_TILE pixels of the stride grid writes its int64 row to
+ *   the workspace, and one CTA adds the rows.  No sum overflows while max_depth <= DCA_ICP_MAX_DEPTH, G <=
+ *   DCA_ICP_MAX_GATE and H W <= DCA_ICP_MAX_PIXELS: |J_i| <= |q||n| <= 2 sqrt(3) max_depth 1.031 < 4 max_depth <= 2^10,
+ *   |r| <= 1.031 G (1 + 2^-20) <= 2^4 1.04, so a term is below 2^38 (1.09) of its unit and H W of them below 2^63.  There is
+ *   no normal-compatibility test on the source side: stereo normals from forward differences are much noisier than the
+ *   raycast normals, and the gate, the confidence weight and the left-right filter already applied by dca_reproject
+ *   reject the outliers such a test would.
+ *   solve (fp64, one thread): H, g, e, sw = the int64 sums converted to fp64 (correctly rounded) times the inverse
+ *       scales;  fail with DCA_ICP_FEW_INLIERS when count < min_inliers;  Cholesky H = L L^T, column j = 0..5:
+ *       s = H_jj - L_j0 L_j0 - ... - L_j,j-1 L_j,j-1 (left to right); fail with DCA_ICP_DEGENERATE unless
+ *       s > DCA_ICP_PIVOT_REL (x) max_i H_ii;  L_jj = sqrt(s);  L_ij = (H_ij - L_i0 L_j0 - ... ) / L_jj for i > j;
+ *       forward  y_i = (-g_i - L_i0 y_0 - ... - L_i,i-1 y_i-1) / L_ii;  backward xi_i = (y_i - L_i+1,i xi_i+1 - ... -
+ *       L_5i xi_5) / L_ii  (k ascending);  (omega, t) = xi
+ *   update: (hx, hy, hz) = omega (x) 0.5, nq = sqrt(((1 + hx hx) + hy hy) + hz hz), (w, x, y, z) = (1, hx, hy, hz) / nq;
+ *       R = [[1 - 2 (yy + zz), 2 (xy - wz), 2 (xz + wy)], [2 (xy + wz), 1 - 2 (xx + zz), 2 (yz - wx)],
+ *            [2 (xz - wy), 2 (yz + wx), 1 - 2 (xx + yy)]] (each product and sum rounded as written);
+ *       A <- [R | t] A: A'_ij = ((R_i0 A_0j + R_i1 A_1j) + R_i2 A_2j) (+ t_i for j = 3).  A failed iteration leaves A.
+ * Outputs (device): pose fp64 [12] = the final A; stats fp64 [total iterations][4] = (count, sw, e, flag) per
+ * iteration, flag 0 or DCA_ICP_FEW_INLIERS or DCA_ICP_DEGENERATE; ok int32 = 1 when no iteration failed, else 0.
+ * workspace = DCA_ICP_WORKSPACE_BYTES(H, W) bytes.  Fixed iteration counts (no early exit): 2 launches per iteration,
+ * no host sync, no allocation: capturable in a CUDA graph.  DCA_ERR_ARG for NULL depth / model maps / A0_host / level
+ * arrays / workspace / pose / stats / ok, H, W <= 0, pitch < W, vertex_pitch or normal_pitch < 3 W, non-finite or zero
+ * fx / fy, non-finite cx / cy, max_depth not finite and > 0, min_inliers < 1, num_levels outside
+ * 1..DCA_ICP_MAX_LEVELS, a stride < 1, iterations outside 1..DCA_ICP_MAX_ITERS, a gate not finite and > 0 and a
+ * non-finite A0; DCA_ERR_UNSUPPORTED for max_depth > DCA_ICP_MAX_DEPTH, a gate > DCA_ICP_MAX_GATE, H W >
+ * DCA_ICP_MAX_PIXELS and |u0| or |v0| >= 2^24. */
+#define DCA_ICP_TILE 1024
+#define DCA_ICP_WORKSPACE_ROW 32
+#define DCA_ICP_WORKSPACE_BYTES(H, W)                                                                                 \
+  (8ull * DCA_ICP_WORKSPACE_ROW *                                                                                     \
+   (((unsigned long long)(H) * (unsigned long long)(W) + DCA_ICP_TILE - 1) / DCA_ICP_TILE))
+#define DCA_ICP_MAX_LEVELS 4
+#define DCA_ICP_MAX_ITERS 64
+#define DCA_ICP_MAX_DEPTH 256.0f
+#define DCA_ICP_MAX_GATE 16.0f
+#define DCA_ICP_MAX_PIXELS (1ll << 24)
+#define DCA_ICP_MAX_NORMAL2 1.0625f
+#define DCA_ICP_SCALE_H 262144.0f      /* 2^18 */
+#define DCA_ICP_SCALE_G 16777216.0f    /* 2^24 */
+#define DCA_ICP_SCALE_E 1073741824.0f  /* 2^30 */
+#define DCA_ICP_SCALE_W 1073741824.0f  /* 2^30 */
+#define DCA_ICP_PIVOT_REL 5e-5        /* DESIGN.md, "Tracking": between a ground plane (<= 1.3e-5) and the full scene (>= 3e-4) */
+#define DCA_ICP_FEW_INLIERS 1
+#define DCA_ICP_DEGENERATE 2
+int dca_tsdf_raycast(const float* volume, int planes, int nx, int ny, int nz, float ox, float oy, float oz,
+                     float voxel_size, float trunc, float min_weight, float fx, float fy, float cx, float cy, int u0,
+                     int v0, int H, int W, const float* T_host, float min_depth, float max_depth, float* depth,
+                     long long depth_pitch, float* vertex, long long vertex_pitch, float* normal,
+                     long long normal_pitch, unsigned char* rgb, long long rgb_pitch, void* stream);
+int dca_icp_track(const float* depth, const float* weight, long long pitch, int H, int W, float fx, float fy, float cx,
+                  float cy, int u0, int v0, float max_depth, const float* model_vertex, long long vertex_pitch,
+                  const float* model_normal, long long normal_pitch, const double* A0_host, int num_levels,
+                  const int* level_stride, const int* level_iters, const float* level_gate, int min_inliers,
+                  void* workspace, double* pose, double* stats, int* ok, void* stream);
+
 /* layout + parameter preparation ---------------------------------------------------------------- */
 int dca_planes_from_ncdhw(const float* x, void* y, int planes, int B, int C, int Cp, int D, int H, int W,
                           void* stream);
