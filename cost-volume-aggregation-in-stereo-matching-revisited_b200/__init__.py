@@ -1,5 +1,6 @@
 """B200-native DCANet cost-volume hot path (feature maps -> disparity) behind the reference's module API."""
-from . import _lib, engine, evaluation, frontend, fusion, geometry, gwcnet, hshard, kitti_io, pipeline, tracking, wls
+from . import (_lib, engine, evaluation, frontend, fusion, geometry, guide, gwcnet, hshard, kitti_io, pipeline, tracking,
+               wls)
 from . import gwcnet_dca0_g, gwcnet_dca1_g, gwcnet_dca2_g, gwcnet_dca4_g
 from .cva import Multi_Aggregation, cva
 from .engine import LR_CONSISTENT, LR_MISMATCH, LR_OCCLUDED, LR_OUT_OF_VIEW, Confidence, LRCheck
@@ -7,6 +8,7 @@ from .evaluation import DisparityMeter, evaluate_files, read_kitti_disparity, re
 from .fusion import Rendered, SurfacePoints, TSDFVolume, fuse_files, read_kitti_poses, save_kitti_poses
 from .geometry import (PointCloud, StereoCalib, read_kitti_calib, read_middlebury_calib, reproject,
                        reproject_files, save_depth_png, save_ply)
+from .guide import lidar_hints, read_velodyne
 from .gwcnet_dca_g import GwcNet, feature_extraction, hourglass
 from .pipeline import HotPathPipeline
 from .rectify import (RectifyPipeline, Rectified, StereoRectifier, read_kitti_raw_rectifier, rectify,
@@ -35,4 +37,4 @@ __all__ = ["GwcNet", "feature_extraction", "hourglass", "cva", "Multi_Aggregatio
            "save_ply", "save_depth_png", "StereoRectifier", "read_kitti_raw_rectifier", "rectify", "Rectified",
            "RectifyPipeline", "rectify_files", "wls", "wls_filter", "Refined", "fusion", "TSDFVolume", "SurfacePoints",
            "fuse_files", "read_kitti_poses", "Rendered", "save_kitti_poses", "tracking", "Tracker", "TrackResult",
-           "Trajectory", "track_files"]
+           "Trajectory", "track_files", "guide", "lidar_hints", "read_velodyne"]

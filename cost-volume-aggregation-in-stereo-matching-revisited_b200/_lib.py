@@ -19,6 +19,7 @@ SIGNATURES = {
     "dca_version": [],
     "dca_plane_format": [],
     "dca_volume_gwc_concat": [_vp, _vp, _vp, _vp, _vp] + [_c_int] * 9 + [_vp],
+    "dca_volume_gwc_concat_guided": [_vp, _vp, _vp, _vp, _vp] + [_c_int] * 9 + [_vp, _f, _f, _vp],
     "dca_build_gwc_volume_f32": [_vp, _vp, _vp] + [_c_int] * 6 + [_vp],
     "dca_build_concat_volume_f32": [_vp, _vp, _vp] + [_c_int] * 5 + [_vp],
     "dca_conv3d_direct": [_c_int, _vp, _c_int, _vp, _vp, _vp, _vp, _vp, _c_int, _vp, _c_int, _c_int, _c_int]
@@ -97,6 +98,9 @@ SIGNATURES = {
     "dca_tsdf_raycast": [_vp] + [_c_int] * 4 + [_f] * 10 + [_c_int] * 4 + [_vp, _f, _f] + [_vp, _ll] * 4 + [_vp],
     "dca_icp_track": [_vp, _vp, _ll, _c_int, _c_int] + [_f] * 4 + [_c_int] * 2 + [_f, _vp, _ll, _vp, _ll, _vp, _c_int]
                      + [_vp] * 3 + [_c_int] + [_vp] * 5,
+    "dca_lidar_hints": [_vp, _c_int, _vp, _c_int, _c_int, _vp] + [_f] * 6 + [_c_int] * 6 + [_f] * 2
+                       + [_vp, _vp, _c_int, _c_int, _vp],
+    "dca_guide_quarter": [_vp] + [_c_int] * 3 + [_f, _vp, _vp],
 }
 _RESTYPES = {"dca_pack_weights_tc_bytes": ctypes.c_longlong, "dca_pack_weights_tc2d_bytes": ctypes.c_longlong,
              "dca_pack_weights_tc_march_bytes": ctypes.c_longlong}

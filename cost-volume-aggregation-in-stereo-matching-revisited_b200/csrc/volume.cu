@@ -36,14 +36,26 @@ __device__ __forceinline__ void cp_async4(float* dst, const float* src, bool val
 
 __device__ __forceinline__ void vol_split2(float a, float b, uint32_t& hi, uint32_t& lo) { split_pair(a, b, hi, lo); }
 
+// LiDAR guidance of the guided instantiations (include/dca_b200.h section 14): every channel of volume plane d at a
+// 1/4-res pixel with hq > 0 is multiplied by k * expf(-(t * t) * s), t = d - hq, before the hi/lo split.  The unguided
+// instantiations never read it.
+struct VolGuide { const float* hq; float k, s; };
+__device__ __forceinline__ float guide_factor(const VolGuide& g, float hv, int d) {
+  const float t = (float)d - hv;
+  return g.k * expf(-(t * t) * g.s);
+}
+
 // CVT = compile-time channel pitch of the volume (64 for DCANet's 40 groups + 2x12 concat); 0 = runtime Cv.
 // GT / CPGT = compile-time group count / channels per group (40 / 8 for DCANet); 0 = runtime.  With them fixed
 // every shared-memory offset of the inner product loop is an immediate and the channel loop unrolls fully.
-template <int PLANES, int CVT, int GT, int CPGT>
+// GUIDED: lane (j, i) = (lane / 4, lane % 4) of a warp tile computes the factor of (d0+dt+j, w0+wt+i) once; the store
+// fetches it by shuffle.
+template <int PLANES, int CVT, int GT, int CPGT, bool GUIDED = false>
 __global__ void __launch_bounds__(VOL_THREADS, 2)
 volume_fused_kernel(const float* __restrict__ gl, const float* __restrict__ gr,
                     const float* __restrict__ cl, const float* __restrict__ cr,
-                    __nv_bfloat16* __restrict__ vol, int B, int C, int G_rt, int Cc, int D, int H, int W, int Cv_rt) {
+                    __nv_bfloat16* __restrict__ vol, int B, int C, int G_rt, int Cc, int D, int H, int W, int Cv_rt,
+                    const VolGuide guide) {
   extern __shared__ float smem[];
   const int Cv = CVT ? CVT : Cv_rt;
   const int G = GT ? GT : G_rt;
@@ -109,6 +121,12 @@ volume_fused_kernel(const float* __restrict__ gl, const float* __restrict__ gr,
     const int dt = (t / n_wt) * 8;            // local disparity of the 8-deep tile
     // window index of (w = w0+wt+i, d = d0+dt+j):  ul = wt + i - dt - j + (VOL_DC-1)
     const int ubase = wt - dt + (VOL_DC - 1) - 7;   // ul = ubase + (i - j + 7), i-j+7 in [0,10]
+    float gf = 1.f;
+    if (GUIDED) {
+      const int w = w0 + wt + (lane & 3);
+      const float hv = w < W ? guide.hq[((size_t)b * H + h) * W + w] : 0.f;
+      if (hv > 0.f) gf = guide_factor(guide, hv, d0 + dt + (lane >> 2));
+    }
     for (int pass = 0; pass < 2; ++pass) {
       const int slot = lane + 32 * pass;
       if (32 * pass >= Cv) break;
@@ -165,7 +183,12 @@ volume_fused_kernel(const float* __restrict__ gl, const float* __restrict__ gr,
           const float mine_a = acc[j][ip], mine_b = acc[j][ip + 1];
           const float got = __shfl_xor_sync(0xffffffffu, odd ? mine_a : mine_b, 1);
           // even lane: voxel a, channels (slot, slot+1) = (mine_a, got); odd lane: voxel b, (slot-1, slot) = (got, mine_b)
-          const float lo_ch = odd ? got : mine_a, hi_ch = odd ? mine_b : got;
+          float lo_ch = odd ? got : mine_a, hi_ch = odd ? mine_b : got;
+          if (GUIDED) {
+            const float f = __shfl_sync(0xffffffffu, gf, j * 4 + ip + odd);
+            lo_ch *= f;
+            hi_ch *= f;
+          }
           if (d_ok && ch_ok && (w0 + wt + ip + odd) < W) {
             uint32_t hw, lw;
             vol_split2(lo_ch, hi_ch, hw, lw);
@@ -249,16 +272,19 @@ struct Vol3Cfg {
   static constexpr int R_BYTES = RQ * 16, L_BYTES = LQ * 16, CR_BYTES = CC * V2_UW * 4, CL_BYTES = CC * V2_TW * 4;
   static constexpr int BUF_BYTES = R_BYTES + L_BYTES + CR_BYTES + CL_BYTES;
   static constexpr int SMEM_BYTES = 2 * BUF_BYTES + 128 + 1024;      // + barriers/counters + alignment slack
+  static constexpr int GUIDE_BYTES = V3_WARPS * 32 * 4;              // guided: one factor per (j, i) of a warp's tile
 };
 
 // KS (1, 2 or 4) lanes share one group pair, each summing CPG / KS of its channels (xor-butterfly at the end).  8 groups
 // (40 channels each) run with KS = 4: 4 x 4 + 12 = 28 busy lanes instead of 16, 328 -> 191 us at KITTI size.  20 groups
 // stay at KS = 1 (measured: KS = 2 is 8 % SLOWER, 152 vs 141 us -- the kernel is bound by its 32-bit store instructions,
 // one 2 x CV-byte row per warp instruction, not by the lanes' FMA work).
-template <int PLANES, int G, int CPG, int CC, int CV, int KS = 1>
+// GUIDED: lane (j, i) = (lane / 4, lane % 4) computes the factor of (d0+dt+j, w0+wt+i) into its warp's 32 floats after
+// the barriers; hq = 0 stores factor 1, and v * 1 = v.
+template <int PLANES, int G, int CPG, int CC, int CV, int KS = 1, bool GUIDED = false>
 __global__ void __launch_bounds__(V3_THREADS, 1)
 volume_fused3_kernel(const __grid_constant__ VolMaps maps, __nv_bfloat16* __restrict__ vol, int B, int D, int H, int W,
-                     int dbg) {
+                     int dbg, const VolGuide guide) {
   using Cfg = Vol3Cfg<G, CPG, CC>;
   constexpr int HG = Cfg::HG, LW4 = Cfg::LW4, UW4 = Cfg::UW4, LW8 = Cfg::LW8, UW8 = Cfg::UW8;
   constexpr int HGK = HG * KS, CPK = CPG / KS;      // lanes doing correlation work, channels per such lane
@@ -411,6 +437,12 @@ volume_fused3_kernel(const __grid_constant__ VolMaps maps, __nv_bfloat16* __rest
             for (int i = 0; i < 4; ++i) acc[q][j][i] = l[i] * r[i - j + 8];
         }
       }
+      float* gfw = reinterpret_cast<float*>(base + 2 * Cfg::BUF_BYTES + 128) + warp * 32;
+      if (GUIDED) {
+        const float hv = guide.hq[((size_t)b * H + h) * W + w0 + wt + (lane & 3)];     // W % 8 == 0: in the row
+        gfw[lane] = hv > 0.f ? guide_factor(guide, hv, d0 + dt + (lane >> 2)) : 1.f;
+        __syncwarp();
+      }
       if (2 * gl < CV && ks == 0) {
         __nv_bfloat16* rowp = vol + ((((size_t)b * D + d0 + dt) * H + h) * W + (w0 + wt)) * CV + 2 * gl;
         // the 32 lanes own 2 * NVL channels; zero-pad channels beyond that (KS > 1 uses lanes up) fall to the last lane
@@ -425,7 +457,12 @@ volume_fused3_kernel(const __grid_constant__ VolMaps maps, __nv_bfloat16* __rest
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
               uint32_t hw, lw;
-              vol_split2b(acc[0][j][i] * lane_scale, acc[1][j][i] * lane_scale, hw, lw);
+              if (GUIDED) {
+                const float f = gfw[j * 4 + i];
+                vol_split2b(acc[0][j][i] * lane_scale * f, acc[1][j][i] * lane_scale * f, hw, lw);
+              } else {
+                vol_split2b(acc[0][j][i] * lane_scale, acc[1][j][i] * lane_scale, hw, lw);
+              }
               *reinterpret_cast<uint32_t*>(rowp + i * CV) = hw;
               if (PLANES == 2) *reinterpret_cast<uint32_t*>(rowp + plane_stride + i * CV) = lw;
               if (pads) {
@@ -503,9 +540,9 @@ static bool vol_concat_map(CUtensorMap* m, const float* p, int B, int CC, int H,
 
 static int g_vol_sms = 0;
 static int g_volume_v2 = 1;   // bit0: use the TMA-staged kernel; bits 1..2: timing probes (skip compute / skip staging)
-template <int G, int CPG, int CC, int CV, int KS = 1>
+template <int G, int CPG, int CC, int CV, int KS, bool GUIDED>
 static int launch_volume3(const float* gl, const float* gr, const float* cl, const float* cr, void* vol, int B, int D,
-                          int H, int W, int planes, cudaStream_t st) {
+                          int H, int W, int planes, cudaStream_t st, const VolGuide& guide) {
   using Cfg = Vol3Cfg<G, CPG, CC>;
   static_assert(G % 2 == 0 && (G / 2) * KS + CC <= 32 && CV >= G + 2 * CC && CV <= 64 && Cfg::SMEM_BYTES <= 227 * 1024 &&
                 Cfg::R_BYTES % 128 == 0 && Cfg::L_BYTES % 128 == 0 && Cfg::CR_BYTES % 128 == 0 && Cfg::CL_BYTES % 128 == 0,
@@ -519,14 +556,16 @@ static int launch_volume3(const float* gl, const float* gr, const float* cl, con
   const long long items = (long long)wtiles * dchunks * H * B;
   if (items * V3_SLOTS >= (1ll << 31)) return DCA_ERR_UNSUPPORTED;
   const int grid = (int)(items < g_vol_sms ? items : g_vol_sms);
+  const int smem = Cfg::SMEM_BYTES + (GUIDED ? Cfg::GUIDE_BYTES : 0);
+  static_assert(Cfg::SMEM_BYTES + Cfg::GUIDE_BYTES <= 227 * 1024, "guided shared memory");
   if (planes == 2) {
-    auto kern = volume_fused3_kernel<2, G, CPG, CC, CV, KS>;
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
-    dca_launch(kern, grid, V3_THREADS, Cfg::SMEM_BYTES, st, maps, (__nv_bfloat16*)vol, B, D, H, W, g_volume_v2 >> 1);
+    auto kern = volume_fused3_kernel<2, G, CPG, CC, CV, KS, GUIDED>;
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    dca_launch(kern, grid, V3_THREADS, smem, st, maps, (__nv_bfloat16*)vol, B, D, H, W, g_volume_v2 >> 1, guide);
   } else {
-    auto kern = volume_fused3_kernel<1, G, CPG, CC, CV, KS>;
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
-    dca_launch(kern, grid, V3_THREADS, Cfg::SMEM_BYTES, st, maps, (__nv_bfloat16*)vol, B, D, H, W, g_volume_v2 >> 1);
+    auto kern = volume_fused3_kernel<1, G, CPG, CC, CV, KS, GUIDED>;
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    dca_launch(kern, grid, V3_THREADS, smem, st, maps, (__nv_bfloat16*)vol, B, D, H, W, g_volume_v2 >> 1, guide);
   }
   DCA_RETURN_IF_LAUNCH_FAILED();
   return DCA_OK;
@@ -594,30 +633,33 @@ using namespace dca;
 // 1 (default) = 16-byte-staged pair kernel for the DCANet shapes, 0 = generic kernel everywhere (A/B timing, tests)
 extern "C" int dca_volume_set_v2(int on) { g_volume_v2 = on; return DCA_OK; }
 
-extern "C" int dca_volume_gwc_concat(const float* gwc_l, const float* gwc_r, const float* cat_l, const float* cat_r,
-                                     void* vol, int B, int C, int G, int Cc, int D, int H, int W, int Cv, int planes,
-                                     void* stream) {
+namespace dca {
+template <bool GUIDED>
+static int volume_gwc_concat(const float* gwc_l, const float* gwc_r, const float* cat_l, const float* cat_r, void* vol,
+                             int B, int C, int G, int Cc, int D, int H, int W, int Cv, int planes, void* stream,
+                             const VolGuide& guide) {
   if (!gwc_l || !gwc_r || !vol || B <= 0 || C <= 0 || G <= 0 || D <= 0 || H <= 0 || W <= 0) return DCA_ERR_ARG;
   if (C % G != 0 || (Cc > 0 && (!cat_l || !cat_r)) || Cc < 0) return DCA_ERR_ARG;
   if (Cv < G + 2 * Cc || Cv > 64 || (Cv % 8) != 0 || (planes != 1 && planes != 2)) return DCA_ERR_ARG;
   const int cpg = C / G, gp = G + 1, UW = VOL_TW + VOL_DC - 1;
+  cudaStream_t st = (cudaStream_t)stream;
   if ((W % 8) == 0 && Cc == 12 && C == 320 && (g_volume_v2 & 1)) {      // DCANet's shape (40 groups) and the 20- and 8-group points of config 4's sweep
-    if (G == 40 && Cv == 64) return launch_volume3<40, 8, 12, 64>(gwc_l, gwc_r, cat_l, cat_r, vol, B, D, H, W, planes, (cudaStream_t)stream);
-    if (G == 20 && Cv == 64) return launch_volume3<20, 16, 12, 64>(gwc_l, gwc_r, cat_l, cat_r, vol, B, D, H, W, planes, (cudaStream_t)stream);
-    if (G == 20 && Cv == 48) return launch_volume3<20, 16, 12, 48>(gwc_l, gwc_r, cat_l, cat_r, vol, B, D, H, W, planes, (cudaStream_t)stream);
-    if (G == 8 && Cv == 32) return launch_volume3<8, 40, 12, 32, 4>(gwc_l, gwc_r, cat_l, cat_r, vol, B, D, H, W, planes, (cudaStream_t)stream);
-    if (G == 8 && Cv == 64) return launch_volume3<8, 40, 12, 64, 4>(gwc_l, gwc_r, cat_l, cat_r, vol, B, D, H, W, planes, (cudaStream_t)stream);
+    if (G == 40 && Cv == 64) return launch_volume3<40, 8, 12, 64, 1, GUIDED>(gwc_l, gwc_r, cat_l, cat_r, vol, B, D, H, W, planes, st, guide);
+    if (G == 20 && Cv == 64) return launch_volume3<20, 16, 12, 64, 1, GUIDED>(gwc_l, gwc_r, cat_l, cat_r, vol, B, D, H, W, planes, st, guide);
+    if (G == 20 && Cv == 48) return launch_volume3<20, 16, 12, 48, 1, GUIDED>(gwc_l, gwc_r, cat_l, cat_r, vol, B, D, H, W, planes, st, guide);
+    if (G == 8 && Cv == 32) return launch_volume3<8, 40, 12, 32, 4, GUIDED>(gwc_l, gwc_r, cat_l, cat_r, vol, B, D, H, W, planes, st, guide);
+    if (G == 8 && Cv == 64) return launch_volume3<8, 40, 12, 64, 4, GUIDED>(gwc_l, gwc_r, cat_l, cat_r, vol, B, D, H, W, planes, st, guide);
   }
   size_t smem = ((size_t)cpg * (VOL_TW + UW) * gp + (size_t)Cc * (VOL_TW + UW)) * sizeof(float);
   if (smem > 220 * 1024) return DCA_ERR_UNSUPPORTED;
   const int wtiles = (W + VOL_TW - 1) / VOL_TW, dchunks = (D + VOL_DC - 1) / VOL_DC;
   dim3 grid(wtiles * dchunks, H, B);
-  cudaStream_t st = (cudaStream_t)stream;
 #define DCA_VOL_LAUNCH(P, CVT)                                                                                   \
   do {                                                                                                           \
-    auto kern = volume_fused_kernel<P, CVT, GT_, CPG_>;                                                          \
+    auto kern = volume_fused_kernel<P, CVT, GT_, CPG_, GUIDED>;                                                  \
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                          \
-    kern<<<grid, VOL_THREADS, smem, st>>>(gwc_l, gwc_r, cat_l, cat_r, (__nv_bfloat16*)vol, B, C, G, Cc, D, H, W, Cv); \
+    kern<<<grid, VOL_THREADS, smem, st>>>(gwc_l, gwc_r, cat_l, cat_r, (__nv_bfloat16*)vol, B, C, G, Cc, D, H, W, Cv, \
+                                          guide);                                                                \
   } while (0)
   const bool dcanet_shape = (Cv == 64 && G == 40 && cpg == 8);
 #define GT_ 40
@@ -633,6 +675,22 @@ extern "C" int dca_volume_gwc_concat(const float* gwc_l, const float* gwc_r, con
 #undef DCA_VOL_LAUNCH
   DCA_RETURN_IF_LAUNCH_FAILED();
   return DCA_OK;
+}
+}  // namespace dca
+
+extern "C" int dca_volume_gwc_concat(const float* gwc_l, const float* gwc_r, const float* cat_l, const float* cat_r,
+                                     void* vol, int B, int C, int G, int Cc, int D, int H, int W, int Cv, int planes,
+                                     void* stream) {
+  return volume_gwc_concat<false>(gwc_l, gwc_r, cat_l, cat_r, vol, B, C, G, Cc, D, H, W, Cv, planes, stream,
+                                  VolGuide{nullptr, 0.f, 0.f});
+}
+
+extern "C" int dca_volume_gwc_concat_guided(const float* gwc_l, const float* gwc_r, const float* cat_l,
+                                            const float* cat_r, void* vol, int B, int C, int G, int Cc, int D, int H,
+                                            int W, int Cv, int planes, const float* hq, float k, float s, void* stream) {
+  if (!hq || !(k > 0.f) || !isfinite(k) || !(s >= 0.f) || !isfinite(s)) return DCA_ERR_ARG;
+  return volume_gwc_concat<true>(gwc_l, gwc_r, cat_l, cat_r, vol, B, C, G, Cc, D, H, W, Cv, planes, stream,
+                                 VolGuide{hq, k, s});
 }
 
 extern "C" int dca_build_gwc_volume_f32(const float* l, const float* r, float* vol, int B, int C, int G, int D, int H,

@@ -589,15 +589,33 @@ def lr_consistency(disp_left, disp_right, tau=1.0, mirrored=False, want_right=Fa
     return label, filled, right
 
 
-def fused_volume(gwc_l, gwc_r, cat_l, cat_r, D, G, planes, Cv=None):
+def fused_volume(gwc_l, gwc_r, cat_l, cat_r, D, G, planes, Cv=None, guide=None):
+    """guide = (hq fp32 [B,H,W] contiguous, k, s): the guided volume of include/dca_b200.h section 14."""
     _require_cuda(gwc_l, gwc_r, cat_l, cat_r)
     B, C, H, W = gwc_l.shape
     Cc = 0 if cat_l is None else cat_l.shape[1]
     Cv = Cv or ((G + 2 * Cc + 7) // 8 * 8)
     vol = Planes(B, D, H, W, Cv, planes, gwc_l.device)
-    _lib.call("dca_volume_gwc_concat", gwc_l.data_ptr(), gwc_r.data_ptr(), _ptr(cat_l), _ptr(cat_r), vol.ptr, B, C, G,
-              Cc, D, H, W, Cv, planes, _stream())
+    args = (gwc_l.data_ptr(), gwc_r.data_ptr(), _ptr(cat_l), _ptr(cat_r), vol.ptr, B, C, G, Cc, D, H, W, Cv, planes)
+    if guide is None:
+        _lib.call("dca_volume_gwc_concat", *args, _stream())
+    else:
+        hq, k, s = guide
+        _require_cuda(hq)
+        if tuple(hq.shape) != (B, H, W) or hq.dtype != torch.float32 or not hq.is_contiguous():
+            raise _lib.DcaError(f"hq: expected contiguous float32 [{B}, {H}, {W}], got {hq.dtype} {tuple(hq.shape)}")
+        _lib.call("dca_volume_gwc_concat_guided", *args, hq.data_ptr(), float(k), float(s), _stream())
     return vol
+
+
+def guide_quarter(hints, maxdisp):
+    """Full-res hint map fp32 [B,H,W] (contiguous, H and W multiples of 4) -> hq [B,H/4,W/4]: the largest valid hint
+    (finite, 0 < h < maxdisp) of each 4x4 block divided by 4, 0 where there is none (dca_guide_quarter)."""
+    _require_cuda(hints)
+    B, H, W = hints.shape
+    hq = torch.empty((B, H // 4, W // 4), dtype=torch.float32, device=hints.device)
+    _lib.call("dca_guide_quarter", hints.data_ptr(), B, H, W, float(maxdisp), hq.data_ptr(), _stream())
+    return hq
 
 
 def _f32c(t):
@@ -943,31 +961,45 @@ def check_feature_shapes(pk, gwc_l, gwc_r, cat_l, cat_r, g):
                             "multiple of 8 (the reference's callers pad to 16, main_dca.py:153-166)")
 
 
-def hot_path_forward(pk: PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g, keep=None, confidence=False):
+def hot_path_forward(pk: PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g, keep=None, confidence=False, guide=None):
     """Feature maps -> (pred4 [B,1,H,W], prob_volume2 logits [B,D8,H8,W8]), plus a third item Confidence(peak, std)
     (fp32 [B,1,H,W] each) when `confidence`.  Mirrors GwcNet.forward (eval) of the reference,
     models/gwcnet_dca_g.py:216-240,282; the confidence is this library's addition (one more launch after the upsampling,
-    pred4 and prob_volume2 unchanged bit for bit)."""
+    pred4 and prob_volume2 unchanged bit for bit).  guide = (hints fp32 [B, 4 H/4, 4 W/4] contiguous, k, s) runs the
+    LiDAR-guided volume (include/dca_b200.h section 14)."""
     _require_cuda(gwc_l, gwc_r, cat_l, cat_r, g)
     check_feature_shapes(pk, gwc_l, gwc_r, cat_l, cat_r, g)
+    if guide is not None:
+        B, _, H4, W4 = gwc_l.shape
+        hints = guide[0]
+        _require_cuda(hints)
+        if tuple(hints.shape) != (B, 4 * H4, 4 * W4) or hints.dtype != torch.float32 or not hints.is_contiguous():
+            raise _lib.DcaError(f"hints: expected contiguous float32 [{B}, {4 * H4}, {4 * W4}], got {hints.dtype} "
+                                f"{tuple(hints.shape)}")
     tc0 = Options.use_tc
     try:
-        return _result(hot_path_steps(pk, gwc_l, gwc_r, cat_l, cat_r, g, keep, confidence))
+        return _result(hot_path_steps(pk, gwc_l, gwc_r, cat_l, cat_r, g, keep, confidence, guide=guide))
     finally:
         Options.use_tc = tc0          # fp32_stages (diagnostics) toggles it per stage; never leak that into later calls
 
 
-def hot_path_steps(pk: PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g, keep=None, confidence=False, sharded=False):
+def hot_path_steps(pk: PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g, keep=None, confidence=False, sharded=False,
+                   guide=None):
     """The launches of `hot_path_forward`, as a generator returning its result through StopIteration.  Sharded, the
     feature maps are one rank's row slab with H4_HALO refreshed halo rows per side (hshard.py), a `Rows` request follows
     every layer whose halo rows need a refresh and a `Sum` request the per-class sums S[b,k]; the results keep their
-    halo rows.  Unsharded, nothing is yielded."""
+    halo rows.  Unsharded, nothing is yielded.  guide = (full-res hints [B,H,W], k, s): dca_guide_quarter, then the
+    guided volume (unsharded only)."""
     P = pk.planes
     D4 = pk.maxdisp // 4
     g = _f32c(g)
+    if guide is not None and sharded:
+        raise _lib.DcaError("LiDAR guidance is not available in the H-sharded forward")
+    hq = guide_quarter(guide[0], pk.maxdisp) if guide is not None else None
     side_job = _prop_mask_start(pk, g, P) if Options.prop_side_stream and not sharded else None
     vol = fused_volume(_f32c(gwc_l), _f32c(gwc_r), _f32c(cat_l) if cat_l is not None else None,
-                       _f32c(cat_r) if cat_r is not None else None, D4, pk.num_groups, P)
+                       _f32c(cat_r) if cat_r is not None else None, D4, pk.num_groups, P,
+                       guide=(hq, guide[1], guide[2]) if guide is not None else None)
     tc0 = Options.use_tc
     Options.use_tc = tc0 and "dres" not in Options.fp32_stages
     c = conv(vol, pk.dres0_0, K3S1, ACT_RELU)
@@ -1022,6 +1054,8 @@ def hot_path_steps(pk: PackedHotPath, gwc_l, gwc_r, cat_l, cat_r, g, keep=None, 
         keep.update({f"cva{i + 1}": k for i, k in enumerate(kept)})
         if confidence:
             keep.update(peak_quarter=peak_q, std_quarter=std_q)
+        if hq is not None:
+            keep.update(hint_quarter=hq)
     pv = logits if not pk.cva else logits2     # no cva stage (gwcnet_dca0_g.py:190): the head's own logits
     return (pred4, pv, conf) if confidence else (pred4, pv)
 
@@ -1038,7 +1072,8 @@ class GraphedHotPath:
     tensors (new contents) replays; other tensors capture another graph (a small LRU of them, all sharing one memory
     pool -- their replays are ordered on the calling stream, so they may reuse each other's activations).  Results are
     returned as copies, so they survive the next replay.  `confidence` is part of the graph key: the forward with the
-    confidence maps is a graph of its own.  Weights are baked in as well: `GwcNet` drops its graphs
+    confidence maps is a graph of its own.  So are the LiDAR hint map's address and shape, k and s: the hint map is read
+    in place like the other inputs.  Weights are baked in as well: `GwcNet` drops its graphs
     whenever it drops its packed parameters."""
     MAX_GRAPHS = 8
 
@@ -1052,35 +1087,38 @@ class GraphedHotPath:
     def _key(tensors):
         return tuple((0, ()) if t is None else (t.data_ptr(), tuple(t.shape)) for t in tensors)
 
-    def _capture(self, ins, confidence=False):
+    def _capture(self, ins, confidence=False, guide=None):
         s = torch.cuda.Stream(device=ins[0].device)
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s):                 # warm-up outside the capture: lazy module loads, persistent side buffers
             for _ in range(2):
-                hot_path_forward(self.pk, *ins, confidence=confidence)
+                hot_path_forward(self.pk, *ins, confidence=confidence, guide=guide)
         torch.cuda.current_stream().wait_stream(s)
         torch.cuda.synchronize(ins[0].device)
         g = torch.cuda.CUDAGraph()
         if self.pool is None:
             self.pool = torch.cuda.graph_pool_handle()
         with torch.cuda.graph(g, pool=self.pool):
-            out = hot_path_forward(self.pk, *ins, confidence=confidence)
+            out = hot_path_forward(self.pk, *ins, confidence=confidence, guide=guide)
         return g, out
 
-    def __call__(self, gwc_l, gwc_r, cat_l, cat_r, g, confidence=False):
+    def __call__(self, gwc_l, gwc_r, cat_l, cat_r, g, confidence=False, guide=None):
         ins = (gwc_l, gwc_r, cat_l, cat_r, g)
         _require_cuda(*ins)
-        for t in ins:
+        for t in ins + ((guide[0],) if guide is not None else ()):
             if t is not None and (t.dtype != torch.float32 or not t.is_contiguous()):
                 raise _lib.DcaError("the graphed forward reads its inputs in place: contiguous fp32 tensors only")
         confidence = bool(confidence)
         key = self._key(ins) + (confidence,)
+        if guide is not None:
+            guide = (guide[0], float(guide[1]), float(guide[2]))
+            key += self._key(guide[:1]) + guide[1:]
         hit = self.graphs.pop(key, None)
         if hit is None:
             if len(self.graphs) >= self.MAX_GRAPHS:
                 self.graphs.pop(next(iter(self.graphs)))
-            graph, out = self._capture(ins, confidence)
-            hit = (graph, out, ins)
+            graph, out = self._capture(ins, confidence) if guide is None else self._capture(ins, confidence, guide)
+            hit = (graph, out, ins + (guide,))
         self.graphs[key] = hit                     # most recently used last
         hit[0].replay()
         self.replays += 1

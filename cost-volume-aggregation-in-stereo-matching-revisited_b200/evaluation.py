@@ -10,7 +10,8 @@
                                    errors of dca_depth_metrics (abs rel, sq rel, RMSE, RMSE log, delta < 1.25^k)
   evaluate_files                   the `mytest` loop as a streaming pipeline (ImagePipeline plus a GT slot per pair);
                                    with lr_check=True also the metrics of the left-right consistent pixels and of the
-                                   background-filled disparity, with wls= those of the refined disparity (wls.py)
+                                   background-filled disparity, with wls= those of the refined disparity (wls.py), with
+                                   hints= the LiDAR-guided forward (guide.py) and the metrics of the unhinted pixels
 
 Per-rank meters of a distributed run combine by concatenating their `rows()` (and summing `confusion()` and the
 `sparsification_histograms()`) before `summarize`.  There is no CPU path: the kernels need CUDA tensors.
@@ -25,6 +26,11 @@ from . import _lib
 from .engine import _require_cuda
 from .kitti_io import ImagePipeline, crop_prediction, fit_gt_to_crop, pad_gt_to_multiple, save_disparity_png
 from .wls import wls_filter
+
+
+def _lidar_hints(points, calib, shape, window, view):
+    from .guide import lidar_hints
+    return lidar_hints(points, calib, shape, window=window, view=view)
 
 # column order of the counter rows (DCA_METRIC_* of include/dca_b200.h)
 VALID, SUM_ABS, GT1, GT2, GT3, D1, PRED_NONFINITE = range(7)
@@ -394,7 +400,7 @@ class EvalPipeline(ImagePipeline):
     the GT of the window."""
 
     def __init__(self, model, meter, mode="fit", crop_height=384, crop_width=1248, depth=3, workers=2, confidence=False,
-                 lr_check=False, lr_threshold=1.0, calib=None, wls=None):
+                 lr_check=False, lr_threshold=1.0, calib=None, wls=None, hints=None, hint_k=10.0, hint_c=1.0):
         if mode not in ("fit", "pad16"):
             raise ValueError(f"mode must be 'fit' or 'pad16', got {mode!r}")
         super().__init__(model, crop_height, crop_width, depth, workers)
@@ -415,6 +421,13 @@ class EvalPipeline(ImagePipeline):
         self.rgb_host = [None] * self.depth
         self.rgb_dev = [None] * self.depth
         self._pair_window = None
+        # with hints: one hint file per pair (velodyne .bin, or a sparse-depth PNG framed like the GT), the guided forward,
+        # and `unhinted_meter` scoring pred on the GT pixels without a valid hint
+        self.hints, self.hint_k, self.hint_c = hints, hint_k, hint_c
+        self.unhinted_meter = DisparityMeter(meter.maxdisp, meter.max_valid, meter.device) if hints is not None else None
+        self.hint_host = [None] * self.depth
+        self.hint_dev = [None] * self.depth
+        self._pair_hint = None          # (hints, hints_right or None) on the device, for the forward of the current pair
 
     def _host(self, *shape):
         t = torch.empty(shape, dtype=torch.float32)
@@ -452,6 +465,58 @@ class EvalPipeline(ImagePipeline):
             return fitted, fit_gt_to_crop(gt, self.ch, self.cw), h, w, 0, rgb, window
         return fitted, pad_gt_to_multiple(gt, 16)[0], h, w, window[0], rgb, window
 
+    def _load_hint(self, path, calib, h, w, fitted_shape):
+        """A pair's hint file -> ("bin", float32 [N, 4] points) or ("png", the disparity map fB / depth - doffs framed like
+        the GT, float32 [Hn, Wn])."""
+        from .guide import read_velodyne
+        if str(path).lower().endswith(".bin"):
+            return "bin", read_velodyne(path)
+        depth = read_kitti_disparity(path)          # KITTI depth PNGs share the disparity format: uint16, x 256, 0 = none
+        if depth.shape != (h, w):
+            raise ValueError(f"{path}: sparse depth {depth.shape} does not match the images ({h}, {w})")
+        with np.errstate(divide="ignore"):
+            disp = np.where(depth > 0, np.float32(calib.focal_baseline) / depth - np.float32(calib.doffs),
+                            np.float32(0)).astype(np.float32)
+        framed = fit_gt_to_crop(disp, self.ch, self.cw) if self.mode == "fit" else pad_gt_to_multiple(disp, 16)[0]
+        assert framed.shape == fitted_shape
+        return "png", framed
+
+    def _load_eval_hinted(self, left, right, gt_path, hint_path, calib):
+        out = self._load_eval(left, right, gt_path)
+        fitted, _, h, w = out[0], out[1], out[2], out[3]
+        return out + (self._load_hint(hint_path, calib, h, w, fitted.shape[1:]),)
+
+    def _hint_slot(self, slot, shape):
+        if self.hint_host[slot] is None or tuple(self.hint_host[slot].shape) != shape:
+            self.hint_host[slot] = self._host(*shape)
+            self.hint_dev[slot] = torch.empty(shape, dtype=torch.float32, device=self.dev) if self.cuda \
+                else self.hint_host[slot]
+        return self.hint_host[slot], self.hint_dev[slot]
+
+    def _prepare_hints(self, slot, hint, calib, window):
+        """On the compute stream: the pair's hint maps [1,1,Hn,Wn] (the right view's too for a .bin with lr_check)."""
+        kind, data = hint
+        shape = tuple(self.in_dev[slot].shape[1:])
+        if kind == "png":
+            self._pair_hint = (self.hint_dev[slot][None, None], None)
+            return
+        right = _lidar_hints(data, calib, shape, window, "right") if self.lr_check else None
+        self._pair_hint = (_lidar_hints(data, calib, shape, window, "left"), right)
+
+    def _hint_kw(self):
+        if self._pair_hint is None:
+            return {}
+        kw = dict(hints=self._pair_hint[0], hint_k=self.hint_k, hint_c=self.hint_c)
+        if self._pair_hint[1] is not None:
+            kw["hints_right"] = self._pair_hint[1]
+        return kw
+
+    def _unhinted_update(self, pred, gt):
+        """Score pred on the GT pixels without a valid hint (finite, 0 < h < maxdisp): zero GT = no GT."""
+        h = self._pair_hint[0].reshape(gt.shape)
+        hinted = torch.isfinite(h) & (h > 0) & (h < self.meter.maxdisp)
+        self.unhinted_meter.update(pred, torch.where(hinted, 0.0, gt))
+
     def _wls_update(self, slot, pred, peak, lr):
         y0, x0, h, w, _ = self._pair_window
         src, label = (lr.filled, lr.label) if lr is not None else (pred, None)
@@ -460,11 +525,18 @@ class EvalPipeline(ImagePipeline):
         self.wls_meter.update(ref.disp, self.gt_dev[slot][None, y0:y0 + h, x0:x0 + w])
 
     def _forward_eval(self, slot):
+        pred = self._forward_scored(slot)
+        if self.unhinted_meter is not None:
+            self._unhinted_update(pred[None], self.gt_dev[slot][None])
+        return pred
+
+    def _forward_scored(self, slot):
         x = self.in_dev[slot]
+        hkw = self._hint_kw()
         if self.lr_check:            # (pred, prob_volume, [Confidence,] LRCheck), checked in the network frame
             gt = self.gt_dev[slot][None]
             out = self.model(x[None, 0:3], x[None, 3:6], confidence=self.confidence, lr_check=True,
-                             lr_threshold=self.lr_threshold)
+                             lr_threshold=self.lr_threshold, **hkw)
             pred, pv, lr = out[0], out[1], out[-1]
             self.meter.update(pred, gt, pv if torch.is_tensor(pv) else None, out[2].peak if self.confidence else None,
                               calib=self._pair_calib)
@@ -475,13 +547,13 @@ class EvalPipeline(ImagePipeline):
                 self._wls_update(slot, pred, out[2].peak if self.confidence else None, lr)
             return pred.reshape(x.shape[1], x.shape[2])
         if self.confidence:          # (pred, prob_volume, Confidence(peak, std)): the peak map ranks the pixels
-            pred, pv, conf = self.model(x[None, 0:3], x[None, 3:6], confidence=True)
+            pred, pv, conf = self.model(x[None, 0:3], x[None, 3:6], confidence=True, **hkw)
             self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None, conf.peak,
                               calib=self._pair_calib)
             if self.wls is not None:
                 self._wls_update(slot, pred, conf.peak, None)
             return pred.reshape(x.shape[1], x.shape[2])
-        out = self.model(x[None, 0:3], x[None, 3:6])
+        out = self.model(x[None, 0:3], x[None, 3:6], **hkw)
         pred, pv = (out[0], out[1]) if isinstance(out, (tuple, list)) else (out, None)
         self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None, calib=self._pair_calib)
         if self.wls is not None:
@@ -503,6 +575,8 @@ class EvalPipeline(ImagePipeline):
         calibs = self.calib if isinstance(self.calib, (list, tuple)) else [self.calib] * len(quads)
         if len(calibs) != len(quads):
             raise ValueError(f"{len(calibs)} calibrations for {len(quads)} pairs")
+        if self.hints is not None and len(self.hints) != len(quads):
+            raise ValueError(f"{len(self.hints)} hint files for {len(quads)} pairs")
         slot_sem = threading.Semaphore(self.depth)          # a slot is reusable once the writer is done with it
         q = queue.Queue()
         err = []
@@ -530,14 +604,22 @@ class EvalPipeline(ImagePipeline):
             self.model.eval()
         try:
             with ThreadPoolExecutor(self.workers) as pool, torch.no_grad():
-                futs = [pool.submit(self._load_eval, l, r, g) for l, r, g, _ in quads]
+                if self.hints is None:
+                    futs = [pool.submit(self._load_eval, l, r, g) for l, r, g, _ in quads]
+                else:
+                    futs = [pool.submit(self._load_eval_hinted, l, r, g, hp, c)
+                            for (l, r, g, _), hp, c in zip(quads, self.hints, calibs)]
                 for i, (fut, quad) in enumerate(zip(futs, quads)):
-                    fitted, gt, h, w, top, rgb, window = fut.result()
+                    fitted, gt, h, w, top, rgb, window, *hint = fut.result()
+                    hint = hint[0] if hint else None
                     slot_sem.acquire()
                     slot = i % self.depth
                     self._ensure(slot, fitted.shape[1], fitted.shape[2])
                     np.copyto(self.in_host[slot].numpy(), fitted)
                     np.copyto(self.gt_host[slot].numpy(), gt)
+                    if hint is not None and hint[0] == "png":
+                        hint_h, hint_d = self._hint_slot(slot, hint[1].shape)
+                        np.copyto(hint_h.numpy(), hint[1])
                     if self.wls is not None:
                         rgb_h, rgb_d = self._rgb_slot(slot, rgb.shape[0], rgb.shape[1])
                         np.copyto(rgb_h.numpy(), rgb)
@@ -552,15 +634,21 @@ class EvalPipeline(ImagePipeline):
                             self.gt_dev[slot].copy_(self.gt_host[slot], non_blocking=True)
                             if self.wls is not None:
                                 rgb_d.copy_(rgb_h, non_blocking=True)
+                            if hint is not None and hint[0] == "png":
+                                hint_d.copy_(hint_h, non_blocking=True)
                             self.h2d[slot].record(self.copy_stream)
                         with torch.cuda.stream(self.compute_stream):
                             self.compute_stream.wait_event(self.h2d[slot])
+                            if hint is not None:
+                                self._prepare_hints(slot, hint, calibs[i], window)
                             pred = self._forward_eval(slot)
                             self.free[slot].record(self.compute_stream)
                             if savename is not None:
                                 self.out_host[slot].copy_(pred, non_blocking=True)
                             self.done[slot].record(self.compute_stream)
                     else:
+                        if hint is not None:
+                            self._prepare_hints(slot, hint, calibs[i], window)
                         pred = self._forward_eval(slot)
                         if savename is not None:
                             self.out_host[slot].copy_(pred)
@@ -579,7 +667,7 @@ WLS_KEYS = ("lam", "sigma", "num_iter", "min_support")
 
 def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=2, maxdisp=None, max_valid=None,
                    confidence=False, lr_check=False, lr_threshold=1.0, calib=None, min_depth=1e-3, max_depth=80.0,
-                   wls=None):
+                   wls=None, hints=None, hint_k=10.0, hint_c=1.0):
     """main_dca.py `mytest` over files: quads = (left, right, gt_path, savename or None); GT is a KITTI PNG or a PFM
     (by extension).  maxdisp defaults to model.maxdisp, max_valid as in DisparityMeter.  Returns (summary dict,
     per-image counter rows [N, METRIC_COUNT] in input order); synchronises once, at the end.  confidence=True runs
@@ -597,7 +685,16 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
 
     wls=True (the defaults of wls.wls_filter) or a dict of its lam / sigma / num_iter / min_support adds `wls`:
     summarize() of the refined disparity of the image window against the GT of the window.  The refinement uses the
-    left image, Confidence.peak when confidence=True, and LRCheck.filled with LRCheck.label when lr_check=True."""
+    left image, Confidence.peak when confidence=True, and LRCheck.filled with LRCheck.label when lr_check=True.
+
+    hints (a list aligned with quads; needs calib=) runs the LiDAR-guided forward, model(..., hints=, hint_k=, hint_c=)
+    (guide.py).  Each entry is a velodyne .bin, projected on the compute stream with the pair's calib into the network
+    frame (and into the right view as hints_right when lr_check=True), or a sparse-depth PNG (KITTI depth completion
+    velodyne_raw: uint16 depth x 256, 0 = none; left view only) converted to fB / depth - doffs and framed like the GT.
+    The summary adds
+      hint_density    the fraction of the valid GT pixels that carry a valid hint
+      unhinted        summarize() of pred against the GT of the pixels without a hint: KITTI's GT is itself LiDAR-derived,
+                      so the hinted pixels score the hint as much as the network"""
     if wls is not None and wls is not False:
         wls = {} if wls is True else dict(wls)
         bad = set(wls) - set(WLS_KEYS)
@@ -605,6 +702,12 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
             raise ValueError(f"wls: unknown keys {sorted(bad)}, expected a subset of {WLS_KEYS}")
     else:
         wls = None
+    if hints is not None:
+        if calib is None:
+            raise ValueError("evaluate_files(hints=) needs calib= (the projection of the scans / the depth conversion)")
+        from .guide import modulation_scale
+        modulation_scale(hint_k, hint_c)
+        hints = list(hints)
     if maxdisp is None:
         maxdisp = getattr(model, "maxdisp", 192)
     try:
@@ -613,7 +716,7 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
         dev = torch.device("cpu")
     meter = DisparityMeter(maxdisp, max_valid, dev, min_depth=min_depth, max_depth=max_depth)
     pipe = EvalPipeline(model, meter, mode, crop[0], crop[1], depth, workers, confidence, lr_check, lr_threshold,
-                        calib, wls)
+                        calib, wls, hints, hint_k, hint_c)
     pipe.run(quads)
     rows = meter.rows()
     h = meter.sparsification_histograms()
@@ -626,4 +729,8 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
         summary["lr_density"] = summary["lr_consistent"]["n_valid"] / n if n else float("nan")
     if wls is not None:
         summary["wls"] = summarize(pipe.wls_meter.rows())
+    if hints is not None:
+        summary["unhinted"] = summarize(pipe.unhinted_meter.rows())
+        n = summary["n_valid"]
+        summary["hint_density"] = 1.0 - summary["unhinted"]["n_valid"] / n if n else float("nan")
     return summary, rows

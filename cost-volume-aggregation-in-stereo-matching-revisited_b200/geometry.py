@@ -3,7 +3,7 @@
   StereoCalib              focal lengths, principal point, baseline (metres) and doffs of a rectified pair; .Q() is the
                            4x4 reprojection matrix of OpenCV's reprojectImageTo3D convention
   read_kitti_calib         KITTI object / odometry calib files (P2, P3, R0_rect, Tr_velo_to_cam) and the stereo-2015 /
-                           raw calib_cam_to_cam.txt (P_rect_02, P_rect_03)
+                           raw calib_cam_to_cam.txt (P_rect_02, P_rect_03; R_rect_00 with calib_velo_to_cam.txt)
   read_middlebury_calib    Middlebury calib.txt (cam0, doffs, baseline in mm)
   reproject                disparity (+ confidence / left-right labels as filters) -> PointCloud(xyz, index, count,
                            depth) on the device: one dca_reproject (two launches), no host sync
@@ -27,14 +27,16 @@ REPROJECT_TILE = 1024          # DCA_REPROJECT_TILE: pixels per tile of the work
 class StereoCalib:
     """A rectified stereo pair: fx, fy, cx, cy in px, baseline in metres, doffs = the x-difference of the principal
     points (px; Middlebury), rect_to_velo = an optional 3x4 float32 transform from the rectified camera frame to
-    another frame (KITTI's velodyne frame, see read_kitti_calib)."""
+    another frame (KITTI's velodyne frame, see read_kitti_calib), velo_to_rect = the optional 3x4 float32 transform the
+    other way (LiDAR points into the rectified camera frame: guide.lidar_hints)."""
 
-    def __init__(self, fx, fy, cx, cy, baseline, doffs=0.0, rect_to_velo=None):
+    def __init__(self, fx, fy, cx, cy, baseline, doffs=0.0, rect_to_velo=None, velo_to_rect=None):
         self.fx, self.fy, self.cx, self.cy = float(fx), float(fy), float(cx), float(cy)
         self.baseline, self.doffs = float(baseline), float(doffs)
         if not (self.fx > 0 and self.fy > 0 and self.baseline > 0):
             raise ValueError(f"fx, fy and the baseline must be positive, got {fx}, {fy}, {baseline}")
         self.rect_to_velo = None if rect_to_velo is None else np.asarray(rect_to_velo, np.float32).reshape(3, 4)
+        self.velo_to_rect = None if velo_to_rect is None else np.asarray(velo_to_rect, np.float32).reshape(3, 4)
 
     def Q(self):
         """float32 [4,4]: (X', Y', Z', W') = Q (u, v, d, 1) gives Z = fx B / (d + doffs), X = (u - cx) Z / fx,
@@ -52,7 +54,8 @@ class StereoCalib:
 
     def __repr__(self):
         return (f"StereoCalib(fx={self.fx}, fy={self.fy}, cx={self.cx}, cy={self.cy}, baseline={self.baseline}, "
-                f"doffs={self.doffs}, rect_to_velo={'set' if self.rect_to_velo is not None else None})")
+                f"doffs={self.doffs}, rect_to_velo={'set' if self.rect_to_velo is not None else None}, "
+                f"velo_to_rect={'set' if self.velo_to_rect is not None else None})")
 
 
 def _read_kv(path, sep):
@@ -69,14 +72,27 @@ def _floats(text):
     return np.array([float(v) for v in text.replace("[", " ").replace("]", " ").replace(";", " ").split()])
 
 
-def read_kitti_calib(path):
+def _h(m):
+    """3x4 or 3x3 -> 4x4 homogeneous (float64)."""
+    out = np.eye(4)
+    m = np.asarray(m, np.float64)
+    out[:3, :m.shape[1]] = m
+    return out
+
+
+def read_kitti_calib(path, velo_to_cam=None):
     """KITTI calibration -> StereoCalib of the colour pair (camera 2 = left, camera 3 = right).
 
     Object / odometry files: P2, P3 and, when present, R0_rect and Tr_velo_to_cam (odometry: Tr, already rectified).
     Stereo-2015 / raw calib_cam_to_cam.txt: P_rect_02, P_rect_03.  B = (P2[0,3] - P3[0,3]) / P2[0,0].  With a
     velodyne transform, rect_to_velo is the pseudo-LiDAR convention: the rectified cam-2 point shifted by camera 2's
     offset (-P2[0,3] / fx, -P2[1,3] / fy, 0), rotated by inv(R0_rect), then the inverse rigid transform of
-    Tr_velo_to_cam; composed in float64, stored as float32."""
+    Tr_velo_to_cam; composed in float64, stored as float32.  velo_to_rect is its float64 inverse, Tr_velo_to_cam, then
+    R0_rect, then the shift back: a velodyne point in the rectified cam-2 frame, where u = fx X / Z + cx.
+
+    velo_to_cam = the path of a raw drive's calib_velo_to_cam.txt (R, T): with a raw calib_cam_to_cam.txt, the velodyne
+    transform is [R | T] and the rectifying rotation R_rect_00 (the devkit's P_rect_02 R_rect_00 [R | T]), and both
+    rect_to_velo and velo_to_rect are set."""
     kv = _read_kv(path, ":")
     k2, k3 = ("P2", "P3") if "P2" in kv else ("P_rect_02", "P_rect_03")
     if k2 not in kv or k3 not in kv:
@@ -84,20 +100,34 @@ def read_kitti_calib(path):
     P2, P3 = _floats(kv[k2]).reshape(3, 4), _floats(kv[k3]).reshape(3, 4)
     fx, fy, cx, cy = P2[0, 0], P2[1, 1], P2[0, 2], P2[1, 2]
     baseline = (P2[0, 3] - P3[0, 3]) / fx
-    tr = kv.get("Tr_velo_to_cam", kv.get("Tr"))
-    rect_to_velo = None
-    if tr is not None and ("R0_rect" in kv or "Tr_velo_to_cam" not in kv):
-        V2C = _floats(tr).reshape(3, 4)
-        R0 = _floats(kv["R0_rect"]).reshape(3, 3) if "R0_rect" in kv else np.eye(3)
+    V2C = R0 = None
+    if velo_to_cam is not None:
+        vk = _read_kv(velo_to_cam, ":")
+        if "R" not in vk or "T" not in vk:
+            raise ValueError(f"{velo_to_cam}: no R / T (a KITTI raw calib_velo_to_cam.txt)")
+        V2C = np.hstack([_floats(vk["R"]).reshape(3, 3), _floats(vk["T"]).reshape(3, 1)])
+        r0 = kv.get("R0_rect", kv.get("R_rect_00"))
+        if r0 is None:
+            raise ValueError(f"{path}: velo_to_cam needs the rectifying rotation (R_rect_00 or R0_rect)")
+        R0 = _floats(r0).reshape(3, 3)
+    else:
+        tr = kv.get("Tr_velo_to_cam", kv.get("Tr"))
+        if tr is not None and ("R0_rect" in kv or "Tr_velo_to_cam" not in kv):
+            V2C = _floats(tr).reshape(3, 4)
+            R0 = _floats(kv["R0_rect"]).reshape(3, 3) if "R0_rect" in kv else np.eye(3)
+    rect_to_velo = velo_to_rect = None
+    if V2C is not None:
         C2V = np.eye(4)
         C2V[:3, :3] = V2C[:, :3].T
         C2V[:3, 3] = -V2C[:, :3].T @ V2C[:, 3]
         R0inv = np.eye(4)
         R0inv[:3, :3] = np.linalg.inv(R0)
-        shift = np.eye(4)
+        shift, unshift = np.eye(4), np.eye(4)
         shift[:3, 3] = (-P2[0, 3] / fx, -P2[1, 3] / fy, 0.0)
+        unshift[:3, 3] = (P2[0, 3] / fx, P2[1, 3] / fy, 0.0)
         rect_to_velo = (C2V @ R0inv @ shift)[:3]
-    return StereoCalib(fx, fy, cx, cy, baseline, 0.0, rect_to_velo)
+        velo_to_rect = (unshift @ _h(R0) @ _h(V2C))[:3]
+    return StereoCalib(fx, fy, cx, cy, baseline, 0.0, rect_to_velo, velo_to_rect)
 
 
 def read_middlebury_calib(path):

@@ -10,9 +10,11 @@ class GwcNet(_GwcNet3):
     PV_STAGE = 4
     SQUEEZE_PRED = False
 
-    def forward(self, left, right, disp_true=None, *, confidence=False, lr_check=False, lr_threshold=1.0):
+    def forward(self, left, right, disp_true=None, *, confidence=False, lr_check=False, lr_threshold=1.0, hints=None,
+                hints_right=None, hint_k=10.0, hint_c=1.0):
         # reference signature: forward(left, right)
-        return super().forward(left, right, confidence=confidence, lr_check=lr_check, lr_threshold=lr_threshold)
+        return super().forward(left, right, confidence=confidence, lr_check=lr_check, lr_threshold=lr_threshold,
+                               hints=hints, hints_right=hints_right, hint_k=hint_k, hint_c=hint_c)
 
 
 def GwcNet_G(d):

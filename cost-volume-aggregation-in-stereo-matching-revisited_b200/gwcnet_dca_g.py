@@ -179,18 +179,34 @@ class GwcNet(nn.Module):
         return super().load_state_dict(state_dict, strict=strict, **kw)
 
     # ---- forward -------------------------------------------------------------------------
-    def hot_path(self, gwc_l, gwc_r, cat_l, cat_r, g, keep=None, confidence=False):
+    def _guide(self, gwc_l, hints, hint_k, hint_c):
+        """(hints as contiguous fp32 [B, 4 H/4, 4 W/4], k, s) for the engine, or None without hints."""
+        if hints is None:
+            return None
+        from . import guide
+        s = guide.modulation_scale(hint_k, hint_c)
+        B, _, H4, W4 = gwc_l.shape
+        return guide.hint_map(hints, B, 4 * H4, 4 * W4), float(hint_k), s
+
+    def hot_path(self, gwc_l, gwc_r, cat_l, cat_r, g, keep=None, confidence=False, hints=None, hint_k=10.0,
+                 hint_c=1.0):
         """feature maps -> (pred4 [B,1,H,W], prob_volume2 [B,D8,H8,W8]); the graded path.  confidence=True adds a third
         item, `Confidence(peak, std)` (fp32 [B,1,H,W] each, include/dca_b200.h section 4); pred4 and prob_volume2 stay
-        bit-identical."""
-        return engine.hot_path_forward(self.packed(), gwc_l, gwc_r, cat_l, cat_r, g, keep, confidence)
+        bit-identical.  hints = a LiDAR hint map fp32 [B,1,4 H/4,4 W/4] (or [B,4 H/4,4 W/4]) in full-res px, 0 = none:
+        the cost volume of every hinted pixel is multiplied by hint_k exp(-(d - h/4)^2 / (2 hint_c^2)) over its planes d
+        (include/dca_b200.h section 14, Poggi et al. CVPR 2019); items without a valid hint run as without hints, bit for
+        bit."""
+        guide = self._guide(gwc_l, hints, hint_k, hint_c)
+        return engine.hot_path_forward(self.packed(), gwc_l, gwc_r, cat_l, cat_r, g, keep, confidence, guide=guide)
 
-    def hot_path_graphed(self, gwc_l, gwc_r, cat_l, cat_r, g, confidence=False):
+    def hot_path_graphed(self, gwc_l, gwc_r, cat_l, cat_r, g, confidence=False, hints=None, hint_k=10.0, hint_c=1.0):
         """`hot_path` as one CUDA graph per set of input buffers (captured on first use, replayed afterwards; the inputs
         are read in place, results are returned as copies).  Same kernels, same results, one launch.  Graphs (and their
         shared activation pool) are kept per CALLING stream, so forwards replayed concurrently on several streams do not
-        share buffers.  With and without `confidence` are two graphs."""
-        return self.graphed()(gwc_l, gwc_r, cat_l, cat_r, g, confidence)
+        share buffers.  With and without `confidence` are two graphs.  A hint map (contiguous fp32) is read in place too;
+        its address and shape, hint_k and hint_c select the graph."""
+        guide = self._guide(gwc_l, hints, hint_k, hint_c)
+        return self.graphed()(gwc_l, gwc_r, cat_l, cat_r, g, confidence, guide=guide)
 
     def graphed(self):
         """The `engine.GraphedHotPath` of the current stream (created on first use; dropped with the packed parameters)."""
@@ -211,18 +227,37 @@ class GwcNet(nn.Module):
         return hshard.hot_path_forward_hsharded(self.packed(), gwc_l, gwc_r, cat_l, cat_r, g, rank, world, group,
                                                 transport)
 
-    def forward(self, left, right, disp_true=None, *, confidence=False, lr_check=False, lr_threshold=1.0):
+    def forward(self, left, right, disp_true=None, *, confidence=False, lr_check=False, lr_threshold=1.0, hints=None,
+                hints_right=None, hint_k=10.0, hint_c=1.0):
         """(pred, prob_volume) as the reference's eval forward; confidence=True adds `Confidence(peak, std)`, shaped like
         pred (squeezed with it in the 0/1/2-stage variants).  lr_check=True appends, last, `LRCheck(disp_right, label,
         filled)` of the left-right consistency check with threshold `lr_threshold` px (include/dca_b200.h section 8),
         each shaped like pred: the right view runs in the same forward as the mirrored pair (flip(R), flip(L)), at twice
-        the batch, and pred / prob_volume / Confidence are those of the forward without the flag."""
+        the batch, and pred / prob_volume / Confidence are those of the forward without the flag.
+
+        hints = LiDAR disparity hints of the left view, fp32 [B,1,H,W] (or [B,H,W]) shaped like `left`, full-res px,
+        0 = none (guide.lidar_hints): the guided forward of `hot_path`.  With lr_check, hints_right (the right view's
+        hints, in its own image frame) guide the mirrored half; without it that half runs unguided."""
         if self.training:
             raise NotImplementedError("dcanet_b200 is an inference engine: call .eval() (training-mode heads "
                                       "classif0-2 exist only so checkpoints load)")
+        if hints_right is not None and not lr_check:
+            raise ValueError("hints_right guides the right view of the left-right check: it needs lr_check=True")
         from . import frontend
         B = left.shape[0]
         nb = 2 * B if lr_check else B       # pairs through the hot path
+        guide_map = None
+        if hints is not None or hints_right is not None:
+            from . import guide
+            H, W = left.shape[-2:]
+            maps = [guide.hint_map(h, B, H, W, what) if h is not None else None
+                    for h, what in ((hints, "hints"), (hints_right, "hints_right"))]
+            if lr_check:
+                z = torch.zeros((B, H, W), dtype=torch.float32, device=left.device)
+                guide_map = torch.cat((maps[0] if maps[0] is not None else z,
+                                       maps[1].flip(-1) if maps[1] is not None else z))
+            else:
+                guide_map = maps[0]
         with frontend._no_tf32():          # whatever part of the front end runs on cuDNN runs in true fp32
             if lr_check:                   # left references (L, flip(R)), right images (R, flip(L)): one 4B front end
                 imgs = torch.cat((left, right.flip(-1), right, left.flip(-1)), dim=0)
@@ -233,7 +268,7 @@ class GwcNet(nn.Module):
                 g = self.guidance(left)["g"]
         gwc, cat = f["gwc_feature"], f.get("concat_feature")
         out = self.hot_path(gwc[:nb], gwc[nb:], None if cat is None else cat[:nb], None if cat is None else cat[nb:], g,
-                            confidence=confidence)
+                            confidence=confidence, hints=guide_map, hint_k=hint_k, hint_c=hint_c)
         sq = (lambda t: t.squeeze(1)) if self.SQUEEZE_PRED else (lambda t: t)
         left_view = (lambda t: t[:B]) if lr_check else (lambda t: t)
         pred, pv = out[0], out[1]

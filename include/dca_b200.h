@@ -669,6 +669,52 @@ int dca_icp_track(const float* depth, const float* weight, long long pitch, int 
                   const int* level_stride, const int* level_iters, const float* level_gate, int min_inliers,
                   void* workspace, double* pose, double* stats, int* ok, void* stream);
 
+/* (14) LiDAR guidance of the cost volume ------------------------------------------------------------------------------ */
+/* Guided Stereo Matching (Poggi, Pallotti, Tosi, Mattoccia, CVPR 2019): sparse, metric disparities ("hints") from a LiDAR
+ * scan scale the cost volume around the hinted disparity before aggregation.  fp32 steps use the notation of section 12
+ * ((+) (-) (x) (/) correctly rounded, no contraction); fmaf is the fused multiply-add.
+ *
+ * Hint map: fp32 [B][H][W] (contiguous) in the network frame, full-resolution px.  A hint is valid when it is finite and
+ * 0 < h < maxdisp; anything else, 0 included, is no hint (the "0 = none" convention of the GT maps).
+ *
+ * dca_lidar_hints.  Points fp32 [N][stride] (stride 3: x, y, z; 4: x, y, z, reflectance, a KITTI .bin scan); image b owns
+ * rows offsets[b] .. offsets[b+1] (device int32 [B+1], clamped to [0, N]).  M = velo_to_rect_host (a HOST pointer to 12
+ * floats, row-major 3x4, travelling as launch parameters).  Per point p = (x, y, z) of image b:
+ *   X_i = fmaf(M_i2, z, fmaf(M_i1, y, fmaf(M_i0, x, M_i3)))  for rows i = 0, 1, 2 -> (X, Y, Z), the rectified camera-2 frame
+ *   kept when min_depth <= Z <= max_depth (false for NaN)
+ *   u = ((fx (x) X) (/) Z) (+) cx,  v = ((fy (x) Y) (/) Z) (+) cy,  disp = (fB (/) Z) (-) doffs;  view 1 (right): u = u (-) disp
+ *   pixel (floorf(u (+) 0.5), floorf(v (+) 0.5)) = (cu, cv); kept when x0 <= cu < x0 + w and v_origin <= cv < v_origin + h
+ *   it lands at map row y0 + cv - v_origin, column cu: the exact inverse of dca_reproject's window, which reads window
+ *   pixel (y, x) = map pixel (y0 + y, x0 + x) as image pixel (x0 + x, v_origin + y)
+ *   zbuf[b][row][col] = min(zbuf, (bits(Z) << 32) | p)   (64-bit atomicMin: the smallest Z wins, ties the smallest p)
+ * out[b][y][x] = (fB (/) Z_winner) (-) doffs, or 0 where no point landed (every pixel outside the window is 0).  zbuf =
+ * uint64 [B][H][W] workspace.  Three launches (fill, scatter, finalise), no host sync, no allocation: capturable in a CUDA
+ * graph; the result does not depend on the order of the atomics.  DCA_ERR_ARG for NULL offsets / M / zbuf / out (points
+ * with N > 0), stride not 3 or 4, B, H, W <= 0, N < 0, view not 0 or 1, a window outside the map, non-finite or zero fx /
+ * fy, non-finite cx, cy, doffs or M, fB not finite and > 0, min_depth not > 0 or max_depth not finite and >= min_depth;
+ * DCA_ERR_UNSUPPORTED for H, W, |v_origin| or |v_origin + h| >= 2^24.
+ *
+ * dca_guide_quarter.  hints [B][H][W] -> hq [B][H/4][W/4]: hq = (the largest valid hint of rows 4i..4i+3, columns 4j..4j+3)
+ * (x) 0.25 (exact), 0 when the block has none.  The largest is the nearest surface: LiDAR points behind a foreground edge,
+ * seen by the scanner but hidden from the camera, are dropped.  One launch.  DCA_ERR_ARG for NULL pointers, B, H, W <= 0,
+ * H or W not a multiple of 4 and maxdisp not > 0.
+ *
+ * dca_volume_gwc_concat_guided.  dca_volume_gwc_concat with hq fp32 [B][H][W] at the volume's resolution: every channel
+ * (group correlations and both concat copies; the zero pad stays 0) of plane d at a pixel with hq > 0 is multiplied, in
+ * fp32 and before the hi/lo split, by f = k (x) expf(-(t (x) t) (x) s), t = fp32(d) (-) hq; the caller passes
+ * s = fp32(1 / (2 c^2)) with c in volume planes (4 full-res px).  Pixels with hq <= 0 (or NaN) are stored exactly as by
+ * dca_volume_gwc_concat.  expf is CUDA's (max 2 ulp).  Nothing is clamped: k |volume| must stay inside the plane
+ * format's range (fp16: 65504).  Same kernels and dispatch as dca_volume_gwc_concat, in a guided instantiation; DCA_ERR_ARG
+ * as there, and for NULL hq, k not finite and > 0 and s not finite and >= 0. */
+int dca_lidar_hints(const float* points, int stride, const int* offsets, int B, int N, const float* velo_to_rect_host,
+                    float fx, float fy, float cx, float cy, float fB, float doffs, int view, int y0, int x0, int h,
+                    int w, int v_origin, float min_depth, float max_depth, unsigned long long* zbuf, float* out, int H,
+                    int W, void* stream);
+int dca_guide_quarter(const float* hints, int B, int H, int W, float maxdisp, float* hq, void* stream);
+int dca_volume_gwc_concat_guided(const float* gwc_l, const float* gwc_r, const float* cat_l, const float* cat_r,
+                                 void* vol, int B, int C, int G, int Cc, int D, int H, int W, int Cv, int planes,
+                                 const float* hq, float k, float s, void* stream);
+
 /* layout + parameter preparation ---------------------------------------------------------------- */
 int dca_planes_from_ncdhw(const float* x, void* y, int planes, int B, int C, int Cp, int D, int H, int W,
                           void* stream);
