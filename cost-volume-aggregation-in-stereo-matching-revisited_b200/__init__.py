@@ -1,6 +1,6 @@
 """B200-native DCANet cost-volume hot path (feature maps -> disparity) behind the reference's module API."""
-from . import (_lib, engine, evaluation, frontend, fusion, geometry, guide, gwcnet, hshard, kitti_io, pipeline, tracking,
-               wls)
+from . import (_lib, engine, evaluation, frontend, fusion, geometry, guide, gwcnet, hshard, kitti_io, pipeline, stixel,
+               tracking, wls)
 from . import gwcnet_dca0_g, gwcnet_dca1_g, gwcnet_dca2_g, gwcnet_dca4_g
 from .cva import Multi_Aggregation, cva
 from .engine import LR_CONSISTENT, LR_MISMATCH, LR_OCCLUDED, LR_OUT_OF_VIEW, Confidence, LRCheck
@@ -14,6 +14,7 @@ from .pipeline import HotPathPipeline
 from .rectify import (RectifyPipeline, Rectified, StereoRectifier, read_kitti_raw_rectifier, rectify,
                       rectify_files)
 from .self_attention import SelfAttentionBlock
+from .stixel import GroundProfile, StixelMetric, Stixels, ground_profile, stixels
 from .semantic_level import SemanticLevelContext
 from .tracking import TrackResult, Tracker, Trajectory, track_files
 from .wls import Refined, wls_filter
@@ -37,4 +38,5 @@ __all__ = ["GwcNet", "feature_extraction", "hourglass", "cva", "Multi_Aggregatio
            "save_ply", "save_depth_png", "StereoRectifier", "read_kitti_raw_rectifier", "rectify", "Rectified",
            "RectifyPipeline", "rectify_files", "wls", "wls_filter", "Refined", "fusion", "TSDFVolume", "SurfacePoints",
            "fuse_files", "read_kitti_poses", "Rendered", "save_kitti_poses", "tracking", "Tracker", "TrackResult",
-           "Trajectory", "track_files", "guide", "lidar_hints", "read_velodyne"]
+           "Trajectory", "track_files", "guide", "lidar_hints", "read_velodyne", "stixel", "ground_profile", "stixels",
+           "GroundProfile", "Stixels", "StixelMetric"]

@@ -25,6 +25,7 @@ import torch
 from . import _lib
 from .engine import _require_cuda
 from .kitti_io import ImagePipeline, crop_prediction, fit_gt_to_crop, pad_gt_to_multiple, save_disparity_png
+from .stixel import ground_profile, stixels
 from .wls import wls_filter
 
 
@@ -400,7 +401,8 @@ class EvalPipeline(ImagePipeline):
     the GT of the window."""
 
     def __init__(self, model, meter, mode="fit", crop_height=384, crop_width=1248, depth=3, workers=2, confidence=False,
-                 lr_check=False, lr_threshold=1.0, calib=None, wls=None, hints=None, hint_k=10.0, hint_c=1.0):
+                 lr_check=False, lr_threshold=1.0, calib=None, wls=None, hints=None, hint_k=10.0, hint_c=1.0,
+                 stixels=None):
         if mode not in ("fit", "pad16"):
             raise ValueError(f"mode must be 'fit' or 'pad16', got {mode!r}")
         super().__init__(model, crop_height, crop_width, depth, workers)
@@ -428,6 +430,12 @@ class EvalPipeline(ImagePipeline):
         self.hint_host = [None] * self.depth
         self.hint_dev = [None] * self.depth
         self._pair_hint = None          # (hints, hints_right or None) on the device, for the forward of the current pair
+        # with stixels: `stixel_meter` scores the rendered stixel map of the window, and the segment counts add up on the
+        # device
+        self.stixels = stixels
+        self.stixel_meter = DisparityMeter(meter.maxdisp, meter.max_valid, meter.device) if stixels is not None else None
+        self.stixel_segments = None
+        self.stixel_images = 0
 
     def _host(self, *shape):
         t = torch.empty(shape, dtype=torch.float32)
@@ -524,6 +532,26 @@ class EvalPipeline(ImagePipeline):
         ref = wls_filter(src, rgb, confidence=peak, label=label, window=self._pair_window, **self.wls)
         self.wls_meter.update(ref.disp, self.gt_dev[slot][None, y0:y0 + h, x0:x0 + w])
 
+    def _stixel_update(self, slot, pred, peak, lr):
+        y0, x0, h, w, _ = self._pair_window
+        src, label = (lr.filled, lr.label) if lr is not None else (pred, None)
+        kw = dict(self.stixels)
+        kw.setdefault("max_disp", self.meter.maxdisp)
+        gkw = {k: kw.pop(k) for k in ("min_inliers",) if k in kw}
+        gkw.update({k: kw[k] for k in ("min_confidence", "max_disp") if k in kw})
+        ground = ground_profile(src, confidence=peak, label=label, window=self._pair_window, **gkw)
+        st = stixels(src, ground, confidence=peak, label=label, window=self._pair_window, **kw)
+        self.stixel_meter.update(st.render(ground)[0][:, None], self.gt_dev[slot][None, y0:y0 + h, x0:x0 + w])
+        n = st.count.sum(dtype=torch.int64)
+        self.stixel_segments = n if self.stixel_segments is None else self.stixel_segments + n
+        self.stixel_images += 1
+
+    def _post(self, slot, pred, peak, lr):
+        if self.wls is not None:
+            self._wls_update(slot, pred, peak, lr)
+        if self.stixels is not None:
+            self._stixel_update(slot, pred, peak, lr)
+
     def _forward_eval(self, slot):
         pred = self._forward_scored(slot)
         if self.unhinted_meter is not None:
@@ -543,21 +571,18 @@ class EvalPipeline(ImagePipeline):
             # zero GT = no GT: the inconsistent pixels leave this meter without a change to the metrics kernel
             self.lr_meters["lr_consistent"].update(pred, torch.where(lr.label.reshape(gt.shape) == 0, gt, 0.0))
             self.lr_meters["lr_filled"].update(lr.filled, gt)
-            if self.wls is not None:
-                self._wls_update(slot, pred, out[2].peak if self.confidence else None, lr)
+            self._post(slot, pred, out[2].peak if self.confidence else None, lr)
             return pred.reshape(x.shape[1], x.shape[2])
         if self.confidence:          # (pred, prob_volume, Confidence(peak, std)): the peak map ranks the pixels
             pred, pv, conf = self.model(x[None, 0:3], x[None, 3:6], confidence=True, **hkw)
             self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None, conf.peak,
                               calib=self._pair_calib)
-            if self.wls is not None:
-                self._wls_update(slot, pred, conf.peak, None)
+            self._post(slot, pred, conf.peak, None)
             return pred.reshape(x.shape[1], x.shape[2])
         out = self.model(x[None, 0:3], x[None, 3:6], **hkw)
         pred, pv = (out[0], out[1]) if isinstance(out, (tuple, list)) else (out, None)
         self.meter.update(pred, self.gt_dev[slot][None], pv if torch.is_tensor(pv) else None, calib=self._pair_calib)
-        if self.wls is not None:
-            self._wls_update(slot, pred, None, None)
+        self._post(slot, pred, None, None)
         return pred.reshape(x.shape[1], x.shape[2])
 
     def _crop_back(self, disp, h, w, top):
@@ -623,6 +648,7 @@ class EvalPipeline(ImagePipeline):
                     if self.wls is not None:
                         rgb_h, rgb_d = self._rgb_slot(slot, rgb.shape[0], rgb.shape[1])
                         np.copyto(rgb_h.numpy(), rgb)
+                    if self.wls is not None or self.stixels is not None:
                         self._pair_window = window
                     savename = quad[3]
                     self._pair_calib = calibs[i]
@@ -663,11 +689,13 @@ class EvalPipeline(ImagePipeline):
 
 
 WLS_KEYS = ("lam", "sigma", "num_iter", "min_support")
+STIXEL_KEYS = ("min_confidence", "width", "max_disp", "sigma_ground", "sigma_object", "sigma_sky", "tau", "p_seg",
+               "p_gravity", "p_order", "eps_gravity", "eps_order", "min_inliers")
 
 
 def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=2, maxdisp=None, max_valid=None,
                    confidence=False, lr_check=False, lr_threshold=1.0, calib=None, min_depth=1e-3, max_depth=80.0,
-                   wls=None, hints=None, hint_k=10.0, hint_c=1.0):
+                   wls=None, hints=None, hint_k=10.0, hint_c=1.0, stixels=None):
     """main_dca.py `mytest` over files: quads = (left, right, gt_path, savename or None); GT is a KITTI PNG or a PFM
     (by extension).  maxdisp defaults to model.maxdisp, max_valid as in DisparityMeter.  Returns (summary dict,
     per-image counter rows [N, METRIC_COUNT] in input order); synchronises once, at the end.  confidence=True runs
@@ -694,7 +722,15 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
     The summary adds
       hint_density    the fraction of the valid GT pixels that carry a valid hint
       unhinted        summarize() of pred against the GT of the pixels without a hint: KITTI's GT is itself LiDAR-derived,
-                      so the hinted pixels score the hint as much as the network"""
+                      so the hinted pixels score the hint as much as the network
+
+    stixels=True (the defaults of stixel.stixels) or a dict of its keyword arguments (and ground_profile's min_inliers)
+    computes, after the forward, the ground profile and the stixels of the image window of pred (of LRCheck.filled, with
+    LRCheck.label, when lr_check is set; with Confidence.peak when confidence is set; max_disp defaults to maxdisp) and
+    adds
+      stixels            summarize() of the rendered stixel disparity against the GT of the window (the "disparity
+                         accuracy" of Cordts et al. 2017)
+      stixels_per_image  the mean number of segments per image"""
     if wls is not None and wls is not False:
         wls = {} if wls is True else dict(wls)
         bad = set(wls) - set(WLS_KEYS)
@@ -702,6 +738,13 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
             raise ValueError(f"wls: unknown keys {sorted(bad)}, expected a subset of {WLS_KEYS}")
     else:
         wls = None
+    if stixels is not None and stixels is not False:
+        stixels = {} if stixels is True else dict(stixels)
+        bad = set(stixels) - set(STIXEL_KEYS)
+        if bad:
+            raise ValueError(f"stixels: unknown keys {sorted(bad)}, expected a subset of {STIXEL_KEYS}")
+    else:
+        stixels = None
     if hints is not None:
         if calib is None:
             raise ValueError("evaluate_files(hints=) needs calib= (the projection of the scans / the depth conversion)")
@@ -716,7 +759,7 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
         dev = torch.device("cpu")
     meter = DisparityMeter(maxdisp, max_valid, dev, min_depth=min_depth, max_depth=max_depth)
     pipe = EvalPipeline(model, meter, mode, crop[0], crop[1], depth, workers, confidence, lr_check, lr_threshold,
-                        calib, wls, hints, hint_k, hint_c)
+                        calib, wls, hints, hint_k, hint_c, stixels)
     pipe.run(quads)
     rows = meter.rows()
     h = meter.sparsification_histograms()
@@ -729,6 +772,10 @@ def evaluate_files(model, quads, mode="fit", crop=(384, 1248), depth=3, workers=
         summary["lr_density"] = summary["lr_consistent"]["n_valid"] / n if n else float("nan")
     if wls is not None:
         summary["wls"] = summarize(pipe.wls_meter.rows())
+    if stixels is not None:
+        summary["stixels"] = summarize(pipe.stixel_meter.rows())
+        summary["stixels_per_image"] = (int(pipe.stixel_segments) / pipe.stixel_images if pipe.stixel_images
+                                        else float("nan"))
     if hints is not None:
         summary["unhinted"] = summarize(pipe.unhinted_meter.rows())
         n = summary["n_valid"]

@@ -183,11 +183,37 @@ def _reproject_kernel(disp, peak, label, u0, v0, Q, T, min_peak, min_depth, max_
 
 
 def _bhw(t, what, dtype):
+    if not torch.is_tensor(t):
+        raise ValueError(f"{what}: expected a torch tensor, got {type(t).__name__}")
     if t.dim() == 4 and t.shape[1] == 1:
         t = t[:, 0]
     if t.dim() != 3 or t.dtype != dtype:
         raise ValueError(f"{what}: expected {dtype} [B,H,W] or [B,1,H,W], got {t.dtype} {tuple(t.shape)}")
     return t
+
+
+def _window_maps(disp, confidence, label, window):
+    """The disp / confidence / label maps ([B,H,W] or [B,1,H,W]) as [B,h,w] views of the window that share one layout
+    with a unit column stride (copied only when they do not), and the image pixel (u0, v0) of window pixel (0, 0)."""
+    maps = [_bhw(disp, "disp", torch.float32)]
+    maps.append(None if confidence is None else _bhw(confidence, "confidence", torch.float32))
+    maps.append(None if label is None else _bhw(label, "label", torch.uint8))
+    for m in maps[1:]:
+        if m is not None and (m.shape != maps[0].shape or m.device != maps[0].device):
+            raise ValueError(f"confidence / label {tuple(m.shape)} on {m.device}: expected {tuple(maps[0].shape)} "
+                             f"on {maps[0].device}")
+    u0 = v0 = 0
+    if window is not None:
+        y0, x0, h, w, v_origin = (int(v) for v in window)
+        H, W = maps[0].shape[1:]
+        if not (0 <= y0 and 0 <= x0 and h > 0 and w > 0 and y0 + h <= H and x0 + w <= W):
+            raise ValueError(f"window {tuple(window)} outside the {H}x{W} map")
+        maps = [None if m is None else m[:, y0:y0 + h, x0:x0 + w] for m in maps]
+        u0, v0 = x0, v_origin
+    live = [m for m in maps if m is not None]
+    if any(m.stride() != live[0].stride() or m.stride(2) != 1 for m in live):
+        maps = [None if m is None else m.contiguous() for m in maps]
+    return maps, u0, v0
 
 
 def reproject(disp, calib, *, confidence=None, min_confidence=0.0, label=None, frame="camera", min_depth=0.0,
@@ -211,24 +237,7 @@ def reproject(disp, calib, *, confidence=None, min_confidence=0.0, label=None, f
             raise ValueError("frame='velodyne' needs a calibration with rect_to_velo (read_kitti_calib of an object / "
                              "odometry calib file)")
         T = calib.rect_to_velo
-    maps = [_bhw(disp, "disp", torch.float32)]
-    maps.append(None if confidence is None else _bhw(confidence, "confidence", torch.float32))
-    maps.append(None if label is None else _bhw(label, "label", torch.uint8))
-    for m in maps[1:]:
-        if m is not None and (m.shape != maps[0].shape or m.device != maps[0].device):
-            raise ValueError(f"confidence / label {tuple(m.shape)} on {m.device}: expected {tuple(maps[0].shape)} "
-                             f"on {maps[0].device}")
-    u0 = v0 = 0
-    if window is not None:
-        y0, x0, h, w, v_origin = (int(v) for v in window)
-        H, W = maps[0].shape[1:]
-        if not (0 <= y0 and 0 <= x0 and h > 0 and w > 0 and y0 + h <= H and x0 + w <= W):
-            raise ValueError(f"window {tuple(window)} outside the {H}x{W} map")
-        maps = [None if m is None else m[:, y0:y0 + h, x0:x0 + w] for m in maps]
-        u0, v0 = x0, v_origin
-    live = [m for m in maps if m is not None]
-    if any(m.stride() != live[0].stride() or m.stride(2) != 1 for m in live):
-        maps = [None if m is None else m.contiguous() for m in maps]
+    maps, u0, v0 = _window_maps(disp, confidence, label, window)
     return _reproject_kernel(maps[0], maps[1], maps[2], u0, v0, calib.Q(), T,
                              min_confidence if confidence is not None else 0.0, min_depth, max_depth)
 

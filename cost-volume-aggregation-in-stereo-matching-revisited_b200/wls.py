@@ -14,7 +14,7 @@ from typing import NamedTuple
 import numpy as np
 import torch
 
-from . import _lib, engine
+from . import _lib, engine, geometry
 
 LUT_SIZE = 3 * 255 * 255 + 1        # DCA_WLS_LUT_SIZE: one weight per squared colour distance
 MAX_ITER = 8                        # DCA_WLS_MAX_ITER
@@ -86,16 +86,6 @@ def _wls_kernel(disp, peak, label, guide, lut, lam, num_iter, min_support):
     return refined, support
 
 
-def _bhw(t, what, dtype):
-    if not torch.is_tensor(t):
-        raise ValueError(f"{what}: expected a torch tensor, got {type(t).__name__}")
-    if t.dim() == 4 and t.shape[1] == 1:
-        t = t[:, 0]
-    if t.dim() != 3 or t.dtype != dtype:
-        raise ValueError(f"{what}: expected {dtype} [B,H,W] or [B,1,H,W], got {t.dtype} {tuple(t.shape)}")
-    return t
-
-
 def wls_filter(disp, guide, *, confidence=None, label=None, lam=8000.0, sigma=1.5, num_iter=3, min_support=1e-3,
                window=None):
     """disp fp32 [B,H,W] or [B,1,H,W] (pred4, or LRCheck.filled) -> Refined(disp, support) shaped like the window of
@@ -113,19 +103,7 @@ def wls_filter(disp, guide, *, confidence=None, label=None, lam=8000.0, sigma=1.
                  the maps, so the zero padding of a framed network input is never smoothed into the image
     The pixels that do not pass (low confidence, inconsistent, non-finite) are filled from their neighbours along
     paths that do not cross colour edges."""
-    maps = [_bhw(disp, "disp", torch.float32)]
-    maps.append(None if confidence is None else _bhw(confidence, "confidence", torch.float32))
-    maps.append(None if label is None else _bhw(label, "label", torch.uint8))
-    for m in maps[1:]:
-        if m is not None and (m.shape != maps[0].shape or m.device != maps[0].device):
-            raise ValueError(f"confidence / label {tuple(m.shape)} on {m.device}: expected {tuple(maps[0].shape)} "
-                             f"on {maps[0].device}")
-    if window is not None:
-        y0, x0, h, w, _ = (int(v) for v in window)
-        H, W = maps[0].shape[1:]
-        if not (0 <= y0 and 0 <= x0 and h > 0 and w > 0 and y0 + h <= H and x0 + w <= W):
-            raise ValueError(f"window {tuple(window)} outside the {H}x{W} map")
-        maps = [None if m is None else m[:, y0:y0 + h, x0:x0 + w] for m in maps]
+    maps = geometry._window_maps(disp, confidence, label, window)[0]
     B, h, w = maps[0].shape
     if not torch.is_tensor(guide):
         raise ValueError(f"guide: expected a torch tensor, got {type(guide).__name__}")
@@ -146,9 +124,6 @@ def wls_filter(disp, guide, *, confidence=None, label=None, lam=8000.0, sigma=1.
         raise ValueError(f"min_support must be >= 0, got {min_support!r}")
     if guide.stride(3) != 1 or guide.stride(2) != guide.shape[3]:
         guide = guide.contiguous()
-    live = [m for m in maps if m is not None]
-    if any(m.stride() != live[0].stride() or m.stride(2) != 1 for m in live):
-        maps = [None if m is None else m.contiguous() for m in maps]
     engine._require_cuda(maps[0])
     lut = _device_lut(maps[0].device, sigma)
     refined, support = _wls_kernel(maps[0], maps[1], maps[2], guide, lut, lam, num_iter, min_support)

@@ -715,6 +715,109 @@ int dca_volume_gwc_concat_guided(const float* gwc_l, const float* gwc_r, const f
                                  void* vol, int B, int C, int G, int Cc, int D, int H, int W, int Cv, int planes,
                                  const float* hq, float k, float s, void* stream);
 
+/* (15) Stixels: V-disparity ground profile, per-column segmentation into ground / object / sky ------------------------ */
+/* The Stixel World in the formulation of Pfeiffer & Franke (BMVC 2011), with the per-column dynamic programme and the
+ * object-cost lookup table of Hernandez-Juarez et al. (WACV 2017).  The model is deliberately simplified (one disparity
+ * per object segment, fixed integer object levels in the data cost, a flat-road profile, no height or semantic classes,
+ * no vertical sub-sampling) and is NOT bit-compatible with any published implementation.
+ * disp, peak (fp32, optional) and label (uint8 DCA_LR_*, optional) share one layout, element (b, y, x) at
+ * b pitch_img + y pitch_row + x, as in dca_reproject.  A pixel is VALID when d = disp is finite, 0 <= d < max_disp,
+ * (peak == NULL or peak >= min_peak) and (label == NULL or label == DCA_LR_CONSISTENT).  Window rows y = 0..H-1.
+ *
+ * dca_ground_profile.  Flat-road V-disparity (Labayrade et al., IV 2002): d_g(y) = a (y - y_h) below the horizon y_h.
+ *   histogram  hist[b][y][floor(d)] += 1 (int32 atomics) over the valid pixels
+ *   Hough      candidates a_i = DCA_GROUND_A_MIN + i DCA_GROUND_A_STEP (fp32, exact), i = 0..DCA_GROUND_NA-1, and integer
+ *              horizons j = 0..H-1; score(i, j) = sum over y = j+1..H-1 and delta in {-1, 0, 1} of hist[y][r + delta],
+ *              r = rint(a_i (y - j)) (exact; bins outside 0..max_disp-1 count 0), in int32.  Winner: the largest score,
+ *              ties to the smallest i, then the smallest j
+ *   fit        the inliers are the valid pixels with y > j and floor(d) - rint(a_i (y - j)) in {-1, 0, 1} (the pixels the
+ *              winning score counted); with q = rint(256 d), int64 sums n, Sy, Syy, Sq, Syq (exact, order-free); then in
+ *              fp64 (correctly rounded, no contraction; N, Y, YY, Q, YQ the sums converted):
+ *                den = N YY - Y Y,  alpha = (N YQ - Y Q) / den,  beta = (Q - alpha Y) / N,
+ *                a = alpha / 256,  y_h = -beta / alpha
+ *   ok         n >= min_inliers, den > 0, a >= DCA_GROUND_MIN_SLOPE and y_h finite.  A fronto-parallel surface also
+ *              fills a band of the flattest lines, and the fit of that band follows the band's slope, so a fit flatter
+ *              than DCA_GROUND_MIN_SLOPE (a baseline of 1/16 of the camera height) is not taken for a road
+ *   outputs    profile fp32 [B][H]: fp32(a (y - y_h)) (fp64 operations) for y > y_h, else 0; all 0 when not ok.
+ *              line fp64 [B][2] = (a, y_h), (0, 0) when not ok; inliers int32 [B] = n; ok uint8 [B] = 0 or 1
+ *   workspace = DCA_GROUND_WORKSPACE_BYTES(B, H, max_disp).  Six launches (a memset and five kernels), no host sync, no
+ *   allocation: capturable in a CUDA graph.  DCA_ERR_ARG for NULL required pointers, B, H, W <= 0, B > 65535,
+ *   pitch_row < W, pitch_img < H pitch_row, max_disp outside 1..DCA_STIXEL_MAX_DISP, min_inliers < 1 and a NaN
+ *   min_peak; DCA_ERR_UNSUPPORTED for H W >= 2^31 and H > DCA_GROUND_MAX_ROWS.
+ *
+ * dca_stixels.  All integer once quantised; units of disparity are 1/256 px.
+ *   columns    column k covers window columns k w .. min((k+1) w, W) - 1, k = 0..ncols-1, ncols = ceil(W / w),
+ *              1 <= w <= DCA_STIXEL_MAX_WIDTH.  Rows are processed bottom-up, n = H - 1 - y
+ *   sample     q = rint(256 d) of each valid pixel; the row's sample is the lower median (sorted index (m-1)/2 of the m
+ *              valid values of the row in the column); a row with none is invalid
+ *   profile    fp32 [B][H] (any per-row ground disparity, e.g. dca_ground_profile's); g(y) = rint(256 min(d_g, max_disp))
+ *              where d_g is finite and > 0, else 0.  Ground may only cover rows with g > 0
+ *   data cost  E(r, s) = floor(min(r^2, (tau s)^2) 1024 / s^2) with s = the class's sigma in 1/256 px (integers); a valid
+ *              row costs E(q - g(y), s_ground) as ground, E(q - 256 k, s_object) as an object at level k, E(q, s_sky) as
+ *              sky; an invalid row costs 0 for every class
+ *   object     a segment of rows n_b..n_t with c >= 1 valid rows and S = their sum of q has m = floor((2 S + c) / (2 c))
+ *              and level k = clamp((m + 128) >> 8, 0, max_disp); its data cost is lut[k][n_t+1] - lut[k][n_b], lut the
+ *              prefix sum over n of the object cost at level k.  An object needs c >= 1
+ *   energy     every segment costs p_seg plus its data cost; predecessor (c' below) -> segment (c above):
+ *                sky -> anything: forbidden (sky is always the topmost segment);  ground -> ground: forbidden
+ *                ground -> object: + p_gravity when |m - g(y_b)| > eps_gravity, y_b the object's bottom window row
+ *                object -> object: + p_order when m_upper > m_lower + eps_order (the upper object is nearer)
+ *                object -> ground, ground -> sky, object -> sky: free;  the bottom segment has no predecessor term
+ *   DP         C[n_t][c] = min over n_b <= n_t and c' of C[n_b - 1][c'] + prior + data + p_seg (no C term for n_b = 0),
+ *              in int32.  The disparity-dependent priors read m_lower = the m of the best path's last segment stored at
+ *              (n_b - 1, object) (the approximation of Pfeiffer and Hernandez-Juarez: exact when p_order = p_gravity = 0).
+ *              Ties: the smallest n_b, then c' in the order none (n_b = 0) < ground < object < sky; at the top row the
+ *              class order ground < object < sky.  Backtrack from the top row
+ *   outputs    count int32 [B][ncols]; bottom, top int16 [B][ncols][H] (window rows, bottom >= top), cls uint8
+ *              [B][ncols][H] (DCA_STIXEL_*), disp fp32 [B][ncols][H] (m / 256 for objects, 0 otherwise): segment i =
+ *              0..count-1 from the bottom up, entries past count not written; free_space int32 [B][ncols] = the top row of
+ *              the ground segment that touches the bottom edge, H when the bottom segment is not ground
+ *   workspace = DCA_STIXEL_WORKSPACE_BYTES(B, H, W, width, max_disp): the column samples and the object lut
+ *              int32 [B][ncols][max_disp + 1][H + 1].  Three launches (column reduction, lut, one warp per column for the
+ *              DP with its state in shared memory), no host sync, no allocation: capturable in a CUDA graph.
+ *   DCA_ERR_ARG for NULL required pointers, B, H, W <= 0, B > 65535, pitch_row < W, pitch_img < H pitch_row, width
+ *   outside 1..DCA_STIXEL_MAX_WIDTH, max_disp outside 1..DCA_STIXEL_MAX_DISP, a NaN min_peak, sigmas outside
+ *   1..DCA_STIXEL_MAX_SIGMA, tau outside 1..DCA_STIXEL_MAX_TAU and priors or epsilons outside 0..DCA_STIXEL_MAX_PRIOR;
+ *   DCA_ERR_UNSUPPORTED for H > DCA_STIXEL_MAX_ROWS (the DP's shared memory, 52 (H + 1) bytes per column, stays under
+ *   the 48 KB a CTA gets without an opt-in; the sums stay inside int32) and H W >= 2^31.
+ *
+ * dca_stixel_render.  One thread per pixel (b, y, x) of the H x W window: the segment of column x / width that holds y
+ * gives out_disp = profile[b][y] (ground, the fp32 value as given), disp (object) or 0 (sky), and out_cls = its class.
+ * One launch.  DCA_ERR_ARG for NULL pointers, B, H, W <= 0, B > 65535, width outside 1..DCA_STIXEL_MAX_WIDTH and
+ * ncols != ceil(W / width); DCA_ERR_UNSUPPORTED for H > DCA_STIXEL_MAX_ROWS and H W >= 2^31. */
+#define DCA_STIXEL_GROUND 0
+#define DCA_STIXEL_OBJECT 1
+#define DCA_STIXEL_SKY 2
+#define DCA_STIXEL_MAX_WIDTH 16
+#define DCA_STIXEL_MAX_ROWS 768
+#define DCA_STIXEL_MAX_DISP 1024
+#define DCA_STIXEL_MAX_SIGMA 16384      /* 64 px in 1/256 px */
+#define DCA_STIXEL_MAX_TAU 8
+#define DCA_STIXEL_MAX_PRIOR (1 << 20)
+#define DCA_GROUND_A_MIN 0.015625f      /* 1/64 px per row */
+#define DCA_GROUND_A_STEP 0.00390625f   /* 1/256 px per row */
+#define DCA_GROUND_NA 253               /* a in [1/64, 1]: baselines of 5 cm to 1 m per 1 m of camera height */
+#define DCA_GROUND_MIN_SLOPE 0.0625     /* 1/16 px per row */
+#define DCA_GROUND_MAX_ROWS 4096
+#define DCA_STIXEL_COLS(W, width) (((W) + (width) - 1) / (width))
+#define DCA_GROUND_WORKSPACE_BYTES(B, H, max_disp)                                                                    \
+  (4ull * (unsigned long long)(B) * (unsigned long long)(H) * ((unsigned long long)(max_disp) + DCA_GROUND_NA) +      \
+   48ull * (unsigned long long)(B))
+#define DCA_STIXEL_WORKSPACE_BYTES(B, H, W, width, max_disp)                                                          \
+  (4ull * (unsigned long long)(B) * (unsigned long long)DCA_STIXEL_COLS(W, width) *                                   \
+   ((unsigned long long)(H) + ((unsigned long long)(max_disp) + 1ull) * ((unsigned long long)(H) + 1ull)))
+int dca_ground_profile(const float* disp, const float* peak, const unsigned char* label, long long pitch_row,
+                       long long pitch_img, int B, int H, int W, float min_peak, int max_disp, int min_inliers,
+                       float* profile, double* line, int* inliers, unsigned char* ok, void* workspace, void* stream);
+int dca_stixels(const float* disp, const float* peak, const unsigned char* label, long long pitch_row,
+                long long pitch_img, int B, int H, int W, float min_peak, const float* profile, int width, int max_disp,
+                int s_ground, int s_object, int s_sky, int tau, int p_seg, int p_gravity, int p_order, int eps_gravity,
+                int eps_order, int* count, short* bottom, short* top, unsigned char* cls, float* sdisp, int* free_space,
+                void* workspace, void* stream);
+int dca_stixel_render(const int* count, const short* bottom, const short* top, const unsigned char* cls,
+                      const float* sdisp, const float* profile, int B, int H, int W, int width, int ncols,
+                      float* out_disp, unsigned char* out_cls, void* stream);
+
 /* layout + parameter preparation ---------------------------------------------------------------- */
 int dca_planes_from_ncdhw(const float* x, void* y, int planes, int B, int C, int Cp, int D, int H, int W,
                           void* stream);
