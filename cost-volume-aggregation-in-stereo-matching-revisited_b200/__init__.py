@@ -9,6 +9,7 @@ from .fusion import Rendered, SurfacePoints, TSDFVolume, fuse_files, read_kitti_
 from .geometry import (PointCloud, StereoCalib, read_kitti_calib, read_middlebury_calib, reproject,
                        reproject_files, save_depth_png, save_ply)
 from .guide import lidar_hints, read_velodyne
+from .motion import Motion, MovingObjects, motion           # the function: the module is <package>.motion in sys.modules
 from .gwcnet_dca_g import GwcNet, feature_extraction, hourglass
 from .pipeline import HotPathPipeline
 from .rectify import (RectifyPipeline, Rectified, StereoRectifier, read_kitti_raw_rectifier, rectify,
@@ -39,4 +40,4 @@ __all__ = ["GwcNet", "feature_extraction", "hourglass", "cva", "Multi_Aggregatio
            "RectifyPipeline", "rectify_files", "wls", "wls_filter", "Refined", "fusion", "TSDFVolume", "SurfacePoints",
            "fuse_files", "read_kitti_poses", "Rendered", "save_kitti_poses", "tracking", "Tracker", "TrackResult",
            "Trajectory", "track_files", "guide", "lidar_hints", "read_velodyne", "stixel", "ground_profile", "stixels",
-           "GroundProfile", "Stixels", "StixelMetric"]
+           "GroundProfile", "Stixels", "StixelMetric", "motion", "Motion", "MovingObjects"]

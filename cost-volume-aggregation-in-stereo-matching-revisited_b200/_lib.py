@@ -104,6 +104,10 @@ SIGNATURES = {
     "dca_ground_profile": [_vp, _vp, _vp, _ll, _ll] + [_c_int] * 3 + [_f, _c_int, _c_int] + [_vp] * 6,
     "dca_stixels": [_vp, _vp, _vp, _ll, _ll] + [_c_int] * 3 + [_f, _vp] + [_c_int] * 11 + [_vp] * 8,
     "dca_stixel_render": [_vp] * 6 + [_c_int] * 5 + [_vp] * 3,
+    "dca_motion_labels": [_vp, _vp, _ll, _ll] + [_c_int] * 3 + [_f] * 4 + [_c_int] * 2 + [_f] * 2
+                         + [_vp, _f, _f, _c_int, _vp, _vp, _vp],
+    "dca_motion_components": [_vp, _ll, _ll, _vp, _vp] + [_c_int] * 3 + [_f] * 4 + [_c_int] * 2 + [_f] * 3
+                             + [_c_int] + [_vp] * 8,
 }
 _RESTYPES = {"dca_pack_weights_tc_bytes": ctypes.c_longlong, "dca_pack_weights_tc2d_bytes": ctypes.c_longlong,
              "dca_pack_weights_tc_march_bytes": ctypes.c_longlong}

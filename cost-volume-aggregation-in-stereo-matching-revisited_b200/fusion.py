@@ -387,9 +387,12 @@ class FusePipeline(ReprojectPipeline):
 
     def __init__(self, model, calibs, volume, mode="fit", crop_height=384, crop_width=1248, min_confidence=None,
                  lr_check=False, lr_threshold=1.0, min_depth=0.0, max_depth=None, weight="peak", depth=3, workers=2,
-                 rectifier=None):
+                 rectifier=None, motion=None):
         if weight not in ("peak", None):
             raise ValueError(f"weight must be 'peak' or None, got {weight!r}")
+        from .motion import _options
+        self.motion = _options(motion)
+        self._reference = None                                   # (depth, calib values, window, pose) last integrated
         # the rectifier is set up here rather than by ReprojectPipeline, whose per-slot point-cloud and colour
         # read-back buffers fusion does not use
         super().__init__(model, calibs, mode, crop_height, crop_width, min_confidence, lr_check, lr_threshold,
@@ -451,8 +454,24 @@ class FusePipeline(ReprojectPipeline):
 
     def _integrate(self, obs, calib, pose):
         depth, wmap, rgb, window = obs
+        if self.motion is not None:
+            wmap = self._mask_moving(depth, wmap, calib, window, pose)
         self.volume.integrate(depth, calib, pose, weight=wmap, rgb=rgb if self.volume.colour else None,
                               window=window, max_depth=self.fuse_max_depth)
+
+    def _mask_moving(self, depth, wmap, calib, window, pose):
+        """With motion= set: the weight map of a frame with its moving objects' pixels at 0, tested against the last
+        frame integrated (motion.motion with T(previous <- current) from the two integration poses).  A frame without
+        such a reference (the first, or one whose window or calibration differs) keeps its weights."""
+        from .motion import motion as moving
+        key = (calib.fx, calib.fy, calib.cx, calib.cy, calib.baseline, calib.doffs)
+        win = None if window is None else tuple(int(v) for v in window)
+        ref, self._reference = self._reference, (depth, key, win, pose)
+        if ref is None or ref[0].shape != depth.shape or ref[1] != key or ref[2] != win:
+            return wmap
+        m = moving(depth, ref[0], calib, np.linalg.solve(ref[3], pose), window=window, **self.motion)
+        still = m.instance == 0
+        return still.to(torch.float32) if wmap is None else torch.where(still, wmap, torch.zeros((), device=wmap.device))
 
     def _fuse(self, slot, calib, window, pose):
         """The device work of one pair, on the compute stream; returns what _finish needs (None here)."""
@@ -537,7 +556,7 @@ class FusePipeline(ReprojectPipeline):
 
 def fuse_files(model, items, poses, volume, calib=None, rectifier=None, mode="fit", crop=(384, 1248),
                min_confidence=None, lr_check=False, max_depth=None, weight="peak", ply=None, min_weight=0.5,
-               lr_threshold=1.0, min_depth=0.0, depth=3, workers=2):
+               lr_threshold=1.0, min_depth=0.0, depth=3, workers=2, motion=None):
     """Stereo pairs on disk and their poses -> the fused TSDFVolume.
 
     items      (left, right) file pairs, fused in this order
@@ -550,11 +569,15 @@ def fuse_files(model, items, poses, volume, calib=None, rectifier=None, mode="fi
     max_depth  depths beyond it are dropped, and integration visits only the voxels the frustum can reach
     weight     "peak" = each depth weighted by Confidence.peak of its pixel; None = unit weights
     ply        a path: the extracted surface (min_weight, with normals and, when the volume has colour, colours)
+    motion     None (default) = every frame fused as it is; True or a dict of motion.motion's options (tau, tau_rel,
+               radius, gate, min_pixels) = each frame is tested against the last frame integrated, at the two
+               integration poses, and the pixels of its moving objects get weight 0.  The first frame has no
+               reference and is fused as it is
     The colours are the left image of the window (the rectified left image with a rectifier)."""
     if calib is None and rectifier is None:
         raise ValueError("fuse_files needs a calibration (calib=) or a rectifier (rectifier=)")
     pipe = FusePipeline(model, calib, volume, mode, crop[0], crop[1], min_confidence, lr_check, lr_threshold,
-                        min_depth, max_depth, weight, depth, workers, rectifier)
+                        min_depth, max_depth, weight, depth, workers, rectifier, motion)
     pipe.run(items, poses)
     if ply is not None:
         volume.save_ply(ply, min_weight)

@@ -245,7 +245,8 @@ class TrackPipeline(FusePipeline):
 
 def track_files(model, items, volume, calib=None, rectifier=None, start=np.eye(4), min_confidence=None,
                 lr_check=False, max_depth=40.0, weight="peak", ply=None, min_weight=0.5, levels=LEVELS,
-                min_inliers=100, mode="fit", crop=(384, 1248), lr_threshold=1.0, min_depth=0.0, depth=3, workers=2):
+                min_inliers=100, mode="fit", crop=(384, 1248), lr_threshold=1.0, min_depth=0.0, depth=3, workers=2,
+                motion=None):
     """Stereo pairs on disk without poses -> Trajectory(poses [N,4,4] float64, ok [N]); the pairs are fused into
     `volume` at their tracked poses.
 
@@ -259,6 +260,8 @@ def track_files(model, items, volume, calib=None, rectifier=None, start=np.eye(4
     weight     "peak" = Confidence.peak weights both ICP and integration; None = unit weights
     ply        a path: the extracted surface (min_weight), as in fuse_files
     levels, min_inliers   of Tracker; min_weight is also the raycast's
+    motion     as in fuse_files: each tracked frame is tested against the last frame integrated, at the tracked poses,
+               and its moving objects get weight 0 in the integration (ICP itself is unchanged)
     One host sync per pair, to read the tracked pose (Tracker.track)."""
     if calib is None and rectifier is None:
         raise ValueError("track_files needs a calibration (calib=) or a rectifier (rectifier=)")
@@ -269,7 +272,7 @@ def track_files(model, items, volume, calib=None, rectifier=None, start=np.eye(4
                          dict(levels=levels, max_depth=max_depth, min_weight=min_weight, min_inliers=min_inliers),
                          mode=mode, crop_height=crop[0], crop_width=crop[1], min_confidence=min_confidence,
                          lr_check=lr_check, lr_threshold=lr_threshold, min_depth=min_depth, max_depth=max_depth,
-                         weight=weight, depth=depth, workers=workers, rectifier=rectifier)
+                         weight=weight, depth=depth, workers=workers, rectifier=rectifier, motion=motion)
     pipe.run(items, np.tile(pipe.start, (len(items), 1, 1)))
     if ply is not None:
         volume.save_ply(ply, min_weight)

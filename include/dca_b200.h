@@ -818,6 +818,82 @@ int dca_stixel_render(const int* count, const short* bottom, const short* top, c
                       const float* sdisp, const float* profile, int B, int H, int W, int width, int ncols,
                       float* out_disp, unsigned char* out_cls, void* stream);
 
+/* (16) moving objects between consecutive depth maps ------------------------------------------------------------------- */
+/* A two-frame test of every depth pixel against the previous frame moved by the ego-motion, and the connected components
+ * of the pixels that fail it.  fp32 steps use the notation of section 12 ((+) (-) (x) (/) correctly rounded, no
+ * contraction, matrix rows applied as ((m0 a (+) m1 b) (+) m2 c) (+) m3).  Window pixel (x, y) is image pixel
+ * (x + u0, y + v0), as in dca_reproject and dca_tsdf_integrate.  Depth maps (current and previous) share one layout:
+ * element (b, y, x) at b pitch_img + y pitch_row + x; a depth is VALID when it is finite and > 0 (0 or NaN = no depth).
+ * Both frames have the same window, intrinsics (fx, fy, cx, cy), fB (= fx baseline) and doffs; the disparity of a depth
+ * z is disp(z) = (fB (/) z) (-) doffs.
+ *
+ * dca_motion_labels.  A_b = A_host[b] (a HOST pointer to B x 12 floats, row-major 3x4, travelling as launch
+ * parameters) = T(previous camera <- current camera) of image b, rounded once from the fp64 poses.  Per window pixel:
+ *   z = depth;  INVALID unless z is valid
+ *   p = ((((fp32(x) (+) fp32(u0)) (-) cx) (x) z) (/) fx, (((fp32(y) (+) fp32(v0)) (-) cy) (x) z) (/) fy, z)  (as in
+ *       dca_icp_track);  q = A_b p;  UNSEEN unless q_z > 0
+ *   xm = floorf(((((fx (x) q_x) (/) q_z) (+) cx) (-) fp32(u0)) (+) 0.5), ym likewise;  UNSEEN unless 0 <= xm < W and
+ *       0 <= ym < H (in float, so NaN is UNSEEN)
+ *   e = disp(q_z), the disparity the previous frame should hold there;  tol = max(tau, tau_rel (x) e)
+ *   for each previous pixel (ym + dy, xm + dx) inside the window with a valid depth, dy = -r..r, dx = -r..r in raster
+ *   order:  d = disp(z_prev), s = d (-) e
+ *   STATIC    some |s| <= tol
+ *   APPEARED  every s < -tol: each neighbour lies farther from the camera than q, so the previous camera saw through the
+ *             point: something moved into empty space
+ *   BEHIND    otherwise: the point was hidden at t-1, or the surface moved away (a receding object, or one followed at
+ *             the ego speed)
+ *   UNSEEN    no neighbour has a valid depth (also for q_z <= 0 and a projection outside the window, above)
+ *   residual = s of the neighbour with the smallest |s| (ties to the first in raster order), NaN when there is none.
+ * Outputs label uint8 [B][H][W] (DCA_MOTION_*) and residual fp32 [B][H][W] (contiguous).  One launch, no host sync, no
+ * allocation: capturable in a CUDA graph.  DCA_ERR_ARG for NULL depth / prev / A_host / label / residual, B outside
+ * 1..DCA_MOTION_MAX_FRAMES, H, W <= 0, pitch_row < W, pitch_img < H pitch_row, non-finite or zero fx / fy, non-finite
+ * cx / cy / doffs, fB not finite and > 0, a non-finite A, tau or tau_rel not finite and >= 0 and r outside
+ * 0..DCA_MOTION_MAX_RADIUS; DCA_ERR_UNSUPPORTED for H or W >= 2^24, H W >= 2^31 and |u0| or |v0| >= 2^24.
+ *
+ * dca_motion_components.  Moving instances: 4-connected components of the pixels labelled APPEARED or BEHIND (MOVING
+ * pixels), with an edge between neighbours a, b only where |disp(z_a) (-) disp(z_b)| <= gate (current depths).
+ *   union-find  every MOVING pixel starts as its own root; each edge joins the two roots, the larger hooked under the
+ *               smaller by atomicMin (Playne & Hawick, IEEE TPDS 2018), so a component's root is its smallest raster
+ *               index y W + x whatever order the unions run in
+ *   numbering   components with at least min_pixels pixels, in raster order of their roots, get ids 1..K per image
+ *               (an exclusive scan over tiles of DCA_MOTION_TILE pixels); K = min(kept, DCA_MOTION_MAX_OBJECTS) and
+ *               dropped = kept - K
+ *   instance    int32 [B][H][W]: the id of the pixel's component, 0 for every other pixel
+ *   objects     for id k (row k - 1 of image b), over its pixels:  ints int32 [B][DCA_MOTION_MAX_OBJECTS][8] =
+ *               (pixels, APPEARED pixels, BEHIND pixels, x_min, y_min, x_max, y_max, 0) in window pixels;  extent fp32
+ *               [B][DCA_MOTION_MAX_OBJECTS][6] = (min X, max X, min Y, max Y, min Z, max Z) of p (as in
+ *               dca_motion_labels) in the current camera frame, by atomics on order-preserving integer keys;
+ *               res_sum int64 [B][DCA_MOTION_MAX_OBJECTS] = the sum of rint(256 residual) (round half to even).
+ *               Rows k >= K: ints and res_sum 0, extent NaN
+ *   count int32 [B] = K and dropped int32 [B] stay on the device.  Every sum, min and max is an integer atomic, so the
+ *   outputs do not depend on thread order.  label, residual and depth are the outputs and the input of
+ *   dca_motion_labels (residual and label contiguous, depth in its layout).  workspace =
+ *   DCA_MOTION_WORKSPACE_BYTES(B, H, W).  Eight launches, no host sync, no allocation: capturable in a CUDA graph.
+ *   DCA_ERR_ARG for NULL pointers, B, H, W <= 0, B > 65535, pitch_row < W, pitch_img < H pitch_row, non-finite or zero
+ *   fx / fy, non-finite cx / cy / doffs, fB not finite and > 0, gate not finite and >= 0 and min_pixels < 1;
+ *   DCA_ERR_UNSUPPORTED for H or W >= 2^24, H W >= 2^31 and |u0| or |v0| >= 2^24. */
+#define DCA_MOTION_STATIC 0
+#define DCA_MOTION_APPEARED 1
+#define DCA_MOTION_BEHIND 2
+#define DCA_MOTION_UNSEEN 3
+#define DCA_MOTION_INVALID 4
+#define DCA_MOTION_MAX_FRAMES 16
+#define DCA_MOTION_MAX_RADIUS 4
+#define DCA_MOTION_MAX_OBJECTS 256
+#define DCA_MOTION_TILE 1024
+#define DCA_MOTION_WORKSPACE_BYTES(B, H, W)                                                                           \
+  (8ull * (unsigned long long)(B) * (unsigned long long)(H) * (unsigned long long)(W) +                               \
+   4ull * (unsigned long long)(B) *                                                                                   \
+       (((unsigned long long)(H) * (unsigned long long)(W) + DCA_MOTION_TILE - 1) / DCA_MOTION_TILE))
+int dca_motion_labels(const float* depth, const float* prev, long long pitch_row, long long pitch_img, int B, int H,
+                      int W, float fx, float fy, float cx, float cy, int u0, int v0, float fB, float doffs,
+                      const float* A_host, float tau, float tau_rel, int radius, unsigned char* label, float* residual,
+                      void* stream);
+int dca_motion_components(const float* depth, long long pitch_row, long long pitch_img, const unsigned char* label,
+                          const float* residual, int B, int H, int W, float fx, float fy, float cx, float cy, int u0,
+                          int v0, float fB, float doffs, float gate, int min_pixels, int* instance, int* count,
+                          int* dropped, int* ints, float* extent, long long* res_sum, void* workspace, void* stream);
+
 /* layout + parameter preparation ---------------------------------------------------------------- */
 int dca_planes_from_ncdhw(const float* x, void* y, int planes, int B, int C, int Cp, int D, int H, int W,
                           void* stream);
