@@ -1,6 +1,6 @@
 """B200-native DCANet cost-volume hot path (feature maps -> disparity) behind the reference's module API."""
-from . import (_lib, engine, evaluation, frontend, fusion, geometry, guide, gwcnet, hshard, kitti_io, pipeline, stixel,
-               tracking, wls)
+from . import (_lib, engine, evaluation, frontend, fusion, geometry, guide, gwcnet, hshard, kitti_io, occupancy,
+               pipeline, stixel, tracking, wls)
 from . import gwcnet_dca0_g, gwcnet_dca1_g, gwcnet_dca2_g, gwcnet_dca4_g
 from .cva import Multi_Aggregation, cva
 from .engine import LR_CONSISTENT, LR_MISMATCH, LR_OCCLUDED, LR_OUT_OF_VIEW, Confidence, LRCheck
@@ -10,6 +10,7 @@ from .geometry import (PointCloud, StereoCalib, read_kitti_calib, read_middlebur
                        reproject_files, save_depth_png, save_ply)
 from .guide import lidar_hints, read_velodyne
 from .motion import Motion, MovingObjects, motion           # the function: the module is <package>.motion in sys.modules
+from .occupancy import FREE, OCCUPIED, UNKNOWN, Agreement, OccupancyGrid
 from .gwcnet_dca_g import GwcNet, feature_extraction, hourglass
 from .pipeline import HotPathPipeline
 from .rectify import (RectifyPipeline, Rectified, StereoRectifier, read_kitti_raw_rectifier, rectify,
@@ -40,4 +41,5 @@ __all__ = ["GwcNet", "feature_extraction", "hourglass", "cva", "Multi_Aggregatio
            "RectifyPipeline", "rectify_files", "wls", "wls_filter", "Refined", "fusion", "TSDFVolume", "SurfacePoints",
            "fuse_files", "read_kitti_poses", "Rendered", "save_kitti_poses", "tracking", "Tracker", "TrackResult",
            "Trajectory", "track_files", "guide", "lidar_hints", "read_velodyne", "stixel", "ground_profile", "stixels",
-           "GroundProfile", "Stixels", "StixelMetric", "motion", "Motion", "MovingObjects"]
+           "GroundProfile", "Stixels", "StixelMetric", "motion", "Motion", "MovingObjects", "occupancy",
+           "OccupancyGrid", "Agreement", "FREE", "OCCUPIED", "UNKNOWN"]

@@ -108,6 +108,9 @@ SIGNATURES = {
                          + [_vp, _f, _f, _c_int, _vp, _vp, _vp],
     "dca_motion_components": [_vp, _ll, _ll, _vp, _vp] + [_c_int] * 3 + [_f] * 4 + [_c_int] * 2 + [_f] * 3
                              + [_c_int] + [_vp] * 8,
+    "dca_occupancy_integrate": [_vp, _vp] + [_c_int] * 2 + [_f] * 3 + [_c_int] * 4 + [_vp, _vp, _ll, _ll]
+                               + [_c_int] * 3 + [_f] * 4 + [_c_int] * 2 + [_vp, _vp] + [_f] * 3 + [_c_int] + [_f] * 2
+                               + [_c_int] + [_f] * 4 + [_vp, _vp],
 }
 _RESTYPES = {"dca_pack_weights_tc_bytes": ctypes.c_longlong, "dca_pack_weights_tc2d_bytes": ctypes.c_longlong,
              "dca_pack_weights_tc_march_bytes": ctypes.c_longlong}

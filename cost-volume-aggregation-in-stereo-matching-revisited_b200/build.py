@@ -12,7 +12,7 @@ CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libdca_b200.so")
 SOURCES = ["volume.cu", "conv_direct.cu", "conv_tc.cu", "dca_ops.cu", "halo_p2p.cu", "abi_composites.cu", "metrics.cu",
            "confidence.cu", "lr_check.cu", "reproject.cu", "rectify.cu", "wls.cu", "tsdf.cu", "track.cu",
-           "guide.cu", "stixel.cu", "motion.cu"]
+           "guide.cu", "stixel.cu", "motion.cu", "occupancy.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "--use_fast_math=false"]

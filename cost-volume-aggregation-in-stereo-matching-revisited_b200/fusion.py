@@ -557,18 +557,20 @@ class FusePipeline(ReprojectPipeline):
 def fuse_files(model, items, poses, volume, calib=None, rectifier=None, mode="fit", crop=(384, 1248),
                min_confidence=None, lr_check=False, max_depth=None, weight="peak", ply=None, min_weight=0.5,
                lr_threshold=1.0, min_depth=0.0, depth=3, workers=2, motion=None):
-    """Stereo pairs on disk and their poses -> the fused TSDFVolume.
+    """Stereo pairs on disk and their poses -> the fused TSDFVolume (or the filled OccupancyGrid).
 
     items      (left, right) file pairs, fused in this order
     poses      camera-to-world [N,4,4] or [N,3,4] float64 of the rectified left camera (read_kitti_poses with the
                sequence's calib.txt for KITTI odometry)
-    volume     a TSDFVolume on the model's device (fused into, not reset)
+    volume     a TSDFVolume, or an occupancy.OccupancyGrid, on the model's device (fused into, not reset); a grid takes
+               no colours, and max_depth may not exceed the grid's
     calib      one StereoCalib or a list aligned with items; with a rectifier (rectify.StereoRectifier) the items are
                RAW pairs, rectified on the device, and calib defaults to rectifier.calib
     min_confidence, lr_check   the filters of reproject (the forward runs with confidence / the left-right check)
     max_depth  depths beyond it are dropped, and integration visits only the voxels the frustum can reach
     weight     "peak" = each depth weighted by Confidence.peak of its pixel; None = unit weights
-    ply        a path: the extracted surface (min_weight, with normals and, when the volume has colour, colours)
+    ply        a path: the extracted surface (min_weight, with normals and, when the volume has colour, colours); a
+               TSDFVolume only (an OccupancyGrid writes its map with save_map)
     motion     None (default) = every frame fused as it is; True or a dict of motion.motion's options (tau, tau_rel,
                radius, gate, min_pixels) = each frame is tested against the last frame integrated, at the two
                integration poses, and the pixels of its moving objects get weight 0.  The first frame has no
@@ -576,6 +578,8 @@ def fuse_files(model, items, poses, volume, calib=None, rectifier=None, mode="fi
     The colours are the left image of the window (the rectified left image with a rectifier)."""
     if calib is None and rectifier is None:
         raise ValueError("fuse_files needs a calibration (calib=) or a rectifier (rectifier=)")
+    if ply is not None and not isinstance(volume, TSDFVolume):
+        raise ValueError("ply= writes the surface of a TSDFVolume; an OccupancyGrid writes its map with save_map")
     pipe = FusePipeline(model, calib, volume, mode, crop[0], crop[1], min_confidence, lr_check, lr_threshold,
                         min_depth, max_depth, weight, depth, workers, rectifier, motion)
     pipe.run(items, poses)

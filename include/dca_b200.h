@@ -894,6 +894,72 @@ int dca_motion_components(const float* depth, long long pitch_row, long long pit
                           int v0, float fB, float doffs, float gate, int min_pixels, int* instance, int* count,
                           int* dropped, int* ints, float* extent, long long* res_sum, void* workspace, void* stream);
 
+/* (17) 2-D occupancy grid: obstacle hits and polar free space from posed depth maps, in log-odds ------------------- */
+/* The occupancy grid of Moravec & Elfes (ICRA 1985) and Elfes (IEEE Computer 1989) with clamped log-odds updates
+ * (Hornung et al., OctoMap, 2013) and the polar free-space model of Badino, Franke & Mester (2007): along each image
+ * column the space in front of the first obstacle is free.  fp32 steps use the notation of section 12 ((+) (-) (x) (/)
+ * correctly rounded, no contraction, matrix rows applied as ((m0 a (+) m1 b) (+) m2 c) (+) m3).  Window pixel (x, y)
+ * is image pixel (x + u0, y + v0), as in dca_reproject and dca_tsdf_integrate.
+ * Grid: nx x ny cells of size cs in a plane of the grid frame (x, y horizontal, z up); cell (i, j) has linear index
+ * j nx + i and centre (ox (+) cs (x) fp32(i), oy (+) cs (x) fp32(j)).  State: log_odds fp32 [ny][nx] and updates int32
+ * [ny][nx] (the caller initialises them, normally to 0).
+ * Frames b = 0..B-1: depth (and weight, optional) fp32, element (b, y, x) at b pitch_img + y pitch_row + x.
+ * M_b = M_host[b], grid <- camera, and Minv_b = Minv_host[b], camera <- grid (3x4 row-major; HOST pointers that travel
+ * as launch parameters).  Road level r_b = M_b[11] (-) camera_height (the camera centre's grid z minus its height).
+ * Range bins: nbins = DCA_OCC_BINS = floorf(max_depth (/) range_res) + 1.  Columns: ncols = ceil(W / col_width).
+ * thr = 256 min_hits.
+ *
+ *   pixels   per pixel (b, y, x) of the window:
+ *              z = depth;  skip unless z is finite and 0 < z <= max_depth
+ *              w = 1 without a weight map, else the map clamped to [0, 1], 0 where it holds NaN;  skip unless w > 0
+ *              p = ((((fp32(x) (+) fp32(u0)) (-) cx) (x) z) (/) fx, (((fp32(y) (+) fp32(v0)) (-) cy) (x) z) (/) fy, z)
+ *                  (as in dca_icp_track);  g = M_b p;  h = g_z (-) r_b
+ *              skip unless h <= h_hi (overhangs; NaN skips);  OBSTACLE when h >= h_lo, else GROUND
+ *              q = rint(256 (x) w) (round half to even, exact scaling);  c = x / col_width;  k = floorf(z (/) range_res)
+ *              OBSTACLE: i = floorf(((g_x (-) ox) (/) cs) (+) 0.5), j likewise with g_y, oy; when (i, j) lies in the
+ *                        box, hits[b][cell] += q;  and occ[b][c][k] += q
+ *              every pixel not skipped: near[b][c] = min(near, k), far[b][c] = max(far, k)
+ *   columns  first[b][c] = the smallest k with occ[b][c][k] >= thr, or nbins when there is none
+ *   cells    per cell of the box, frames b = 0..B-1 applied in order with the state in registers (so one call with B
+ *            frames equals B calls of one frame, bit for bit); L = log_odds, n = updates:
+ *              OCCUPIED  when hits[b][cell] >= thr:  L = min(L (+) l_hit, l_max), n += 1
+ *              else the sample s = (centre x, centre y, r_b);  (Xc, Yc, Zc) = Minv_b s;  no update unless Zc > 0
+ *                x = ((fx (x) Xc) (/) Zc) (+) cx (-) fp32(u0),  y = ((fy (x) Yc) (/) Zc) (+) cy (-) fp32(v0)
+ *                xf = floorf(x (+) 0.5), yf = floorf(y (+) 0.5);  no update unless 0 <= xf < W and 0 <= yf < H
+ *                kf = floorf(Zc (/) range_res);  no update unless kf < nbins;  k = kf, c = xf / col_width
+ *              FREE      when column c has a counted pixel, near <= k < first and k <= far:
+ *                        L = max(L (+) l_miss, l_min), n += 1
+ *              any other cell gets no update (occluded, outside the view, under the camera's blind zone, beyond the
+ *              farthest depth of its column)
+ *            A cell that no frame updates is neither read nor written.
+ * Every sum is an integer atomic and each cell's fp32 sequence runs in one thread, so no output depends on thread order.
+ * workspace = DCA_OCC_WORKSPACE_BYTES(B, bi, bj, ncols, nbins): hits int32 [B][bj][bi], occ int32 [B][ncols][nbins],
+ * near / far / first int32 [B][ncols].  Per call one cudaMemsetAsync of the workspace and three kernels (pixels,
+ * columns, cells); no host sync, no allocation: capturable in a CUDA graph.
+ * DCA_ERR_ARG for NULL log_odds / updates / depth / M_host / Minv_host / workspace, nx, ny, H, W <= 0, B outside
+ * 1..DCA_OCC_MAX_FRAMES, pitch_row < W, pitch_img < H pitch_row, a box that is empty or leaves the grid, NaN ox / oy /
+ * camera_height / h_lo / h_hi, non-finite or zero fx / fy, non-finite cx / cy, a non-finite M or Minv, cs or range_res
+ * not > 0 and finite, max_depth not > 0 and finite, h_lo >= h_hi, col_width outside 1..DCA_OCC_MAX_COL_WIDTH,
+ * min_hits outside 1..DCA_OCC_MAX_HITS, l_hit not > 0, l_miss not < 0, and not l_min < 0 < l_max;
+ * DCA_ERR_UNSUPPORTED for nx ny >= 2^31, nx or ny >= 2^24, nbins > DCA_OCC_MAX_BINS, H W >= DCA_OCC_MAX_PIXELS (the int32 sums of q stay
+ * below 2^31), H or W >= 2^24 and |u0| or |v0| >= 2^24. */
+#define DCA_OCC_MAX_FRAMES 16
+#define DCA_OCC_MAX_COL_WIDTH 64
+#define DCA_OCC_MAX_BINS 8192
+#define DCA_OCC_MAX_HITS (1 << 20)
+#define DCA_OCC_MAX_PIXELS (1ll << 23)
+#define DCA_OCC_WORKSPACE_BYTES(B, bi, bj, ncols, nbins)                                                             \
+  (4ull * (unsigned long long)(B) *                                                                                   \
+   ((unsigned long long)(bi) * (unsigned long long)(bj) +                                                             \
+    (unsigned long long)(ncols) * ((unsigned long long)(nbins) + 3ull)))
+int dca_occupancy_integrate(float* log_odds, int* updates, int nx, int ny, float ox, float oy, float cell_size,
+                            int i0, int j0, int bi, int bj, const float* depth, const float* weight,
+                            long long pitch_row, long long pitch_img, int B, int H, int W, float fx, float fy,
+                            float cx, float cy, int u0, int v0, const float* M_host, const float* Minv_host,
+                            float camera_height, float h_lo, float h_hi, int col_width, float range_res,
+                            float max_depth, int min_hits, float l_hit, float l_miss, float l_min, float l_max,
+                            void* workspace, void* stream);
+
 /* layout + parameter preparation ---------------------------------------------------------------- */
 int dca_planes_from_ncdhw(const float* x, void* y, int planes, int B, int C, int Cp, int D, int H, int W,
                           void* stream);
